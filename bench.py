@@ -4,6 +4,7 @@ DDIM-50 flow sampling, Sintel-shaped synthetic 436x1024 frames, batch 8 per GPU.
 
     python bench.py --gpus N --steps K --warmup W            # this implementation (CUDA, sm_100a)
     python bench.py --impl reference --gpus N ...            # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed, as .npy
 
 One "step" = one DDIM-50 sampling pass over one batch of 8 frame pairs = 8 flows.
 Prints ONE JSON line (rank 0).  Multi-GPU: one process per GPU under torchrun, the batch is sharded
@@ -23,6 +24,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True         # the tree may be read-only; the benchmark leaves it as it found it
 
 DDIM_STEPS, TIMESTEPS = 50, 1000
 # --config selects the workload; the default is BASELINE.json configs[1] (the configuration `metric` is quoted on),
@@ -375,6 +377,32 @@ def tiny_config(dev):
     return res
 
 
+# --dump-outputs: an output of at most DUMP_FULL_MAX elements is written whole, a larger one as DUMP_SAMPLE elements at
+# fixed, seeded flat indices.  The sampling outputs (with the hole mask of the samples) come to at most 32 + 3 x 8 MiB of
+# float32.
+DUMP_FULL_MAX = 1 << 23
+DUMP_SAMPLE = 1 << 21
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Write each tensor of `arrays` as <out_dir>/<name>.npy in float32: whole (same shape) when it is small enough, else
+    the 1-D sample flat[idx] with idx = sorted torch.randint(numel, (DUMP_SAMPLE,)) of a CPU generator seeded 0, so two
+    runs or two builds at the same shape sample the same elements.  Every value written is finite: where an output holds
+    NaN or inf (the forward splat leaves NaN holes in the samples), <name>.npy has 0 and <name>_nonfinite.npy has 1."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_FULL_MAX:
+            idx = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        finite = torch.isfinite(t)
+        if not bool(finite.all()):
+            np.save(os.path.join(out_dir, name + "_nonfinite.npy"), (~finite).float().cpu().numpy())
+            t = torch.where(finite, t, torch.zeros_like(t))
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 def run_ours(args, rank: int, world: int, local_rank: int):
     import torch.distributed as dist
@@ -427,14 +455,15 @@ def run_ours(args, rank: int, world: int, local_rank: int):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """Seconds of `steps` calls of fn (slowest rank) and what the last call returned."""
         sync()
         s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         s.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e.record()
         sync()
-        return max_over_ranks(s.elapsed_time(e) * 1e-3, device=dev)
+        return max_over_ranks(s.elapsed_time(e) * 1e-3, device=dev), out
 
     for _ in range(max(args.warmup, 3) if args.warmup >= 0 else 3):
         step_resident()
@@ -442,9 +471,14 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     if rank == 0:
         clocks.start()
     l0 = lib.fd_launch_count() + algo.model.graph_replayed_launches
-    t_res = timed(step_resident, args.steps)
+    t_res, (samples, flows) = timed(step_resident, args.steps)
     launches = int(lib.fd_launch_count() + algo.model.graph_replayed_launches - l0)
-    t_e2e = timed(step_e2e, args.steps)
+    if args.dump_outputs and rank == 0:
+        # what a caller of algo.sample receives: samples (B, 3, H, W) and the flow trajectory (B, 51, 2, H, W), and the
+        # final flow (B, 2, H, W), whole, as the trajectory is only sampled
+        dump_outputs(args.dump_outputs, {"samples": samples, "flows": flows, "flows_last": flows[:, -1]})
+    del samples, flows
+    t_e2e, _ = timed(step_e2e, args.steps)
     clk = clocks.stop() if rank == 0 else None
 
     # roofline pass (not timed above): CUDA events around every tensor-core conv launch of one UNet forward
@@ -721,7 +755,7 @@ def run_train_leg(args, algo_cfg, rank: int, world: int, dev):
 
     for _ in range(3):
         first_loss = step_resident()
-    steps = max(args.steps, 3)
+    steps = args.steps
     l0 = lib.fd_launch_count()
     t_res = timed(step_resident, steps)
     launches = int(lib.fd_launch_count() - l0)
@@ -800,7 +834,14 @@ def main():
     ap.add_argument("--skip-warp", action="store_true", help="omit the warp + photometric/EPE microbench (BASELINE configs[3])")
     ap.add_argument("--skip-train", action="store_true", help="omit the training leg (BASELINE configs[2])")
     ap.add_argument("--skip-sample", action="store_true", help="training leg only (debug; prints a reduced line)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed sampling steps, write what the last one computed as DIR/<name>.npy (float32; "
+                         "an output larger than 2^23 elements as a fixed, seeded sample of 2^21 of them)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.skip_sample):
+        ap.error("--dump-outputs writes the outputs of this implementation's sampling steps (--impl ours, no --skip-sample)")
     # stdout carries exactly ONE JSON line: libraries that chat on file descriptor 1 (NCCL prints its version banner there)
     # are sent to stderr for the duration of the run; _emit() writes the result to the real stdout
     global _REAL_STDOUT

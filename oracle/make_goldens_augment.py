@@ -3,10 +3,12 @@ OWN ``Augmentor`` (algorithms/diffusion_animation/augmentation.py:6-76, imported
 only torch / torchvision / random).  For each seed: ``random.seed(s); torch.manual_seed(s)``, construct the Augmentor (its
 jitter / blur parameters are drawn at construction), call it on a seeded square batch (the reference's resized crop assumes
 square frames, :44-50).  Seeds are chosen so that every branch (jitter, grayscale, blur, h-flip, v-flip, resized crop)
-fires for at least one item.
+fires for at least one item.  The golden stores the SHA-256 of each float32 output (the tests check bit-exactness on it),
+which keeps the file small.
 
 Run in the build container:  python oracle/make_goldens_augment.py  ->  tests/golden/augmentor_ref.npz
 """
+import hashlib
 import os
 import random
 import sys
@@ -40,7 +42,9 @@ def main():
         o_img, o_tgt, o_flow = aug((img.clone(), tgt.clone(), flow.clone()))
         if len(seeds) < 12:
             seeds.append(seed)
-            d[f"img_{seed}"], d[f"tgt_{seed}"], d[f"flow_{seed}"] = o_img.numpy(), o_tgt.numpy(), o_flow.numpy()
+            for name, o in (("img", o_img), ("tgt", o_tgt), ("flow", o_flow)):
+                digest = hashlib.sha256(np.ascontiguousarray(o.numpy(), dtype=np.float32).tobytes()).digest()
+                d[f"sha256_{name}_{seed}"] = np.frombuffer(digest, dtype=np.uint8)
             changed["img"] += int(not torch.equal(o_img, img))
             changed["flip_or_crop"] += int(not torch.equal(o_flow, flow))
     d["seeds"] = np.array(seeds)

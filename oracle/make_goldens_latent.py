@@ -9,6 +9,9 @@ reference-initialised ``Autoencoder`` is written to the local path the reference
 own loading code runs as shipped.  The forward splat is the reference's kernels compiled for the host (oracle/build_ref.py),
 as in oracle/make_goldens_joint.py.
 
+The file keeps only what needs the reference to recompute; oracle/latent_golden.py restores the rest (inputs from their
+seed, ``cond``, the forward latent) bit for bit.
+
 Run in the build container:  python oracle/make_goldens_latent.py  ->  tests/golden/latent_32x48.npz
 """
 import os
@@ -20,12 +23,12 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from oracle import build_ref, ref_stubs  # noqa: E402
+from oracle import build_ref, latent_golden, ref_stubs  # noqa: E402
 from oracle.make_goldens import quiet, weight_checksums  # noqa: E402
 from oracle.make_goldens_flow_learner import HostSplat  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
-AE_SEED, MODEL_SEED = 7, 0
+AE_SEED, MODEL_SEED, INPUT_SEED = 7, 0, 43
 
 
 def main():
@@ -51,10 +54,8 @@ def main():
     assert all(torch.equal(a, b) for a, b in zip(m.ae.state_dict().values(), ae0.state_dict().values()))
     assert not any(p.requires_grad for p in m.ae.parameters())
     sums, asums = weight_checksums(m.unet.state_dict())
-    g = torch.Generator().manual_seed(43)
-    img = torch.rand(B, 3, H, W, generator=g)
-    tgt = torch.rand(B, 3, H, W, generator=g)
-    flow = torch.randn(B, 2, H, W, generator=g) * 3
+    inputs = latent_golden.draw_inputs(INPUT_SEED)
+    img, tgt, flow = (torch.from_numpy(inputs[k]) for k in ("img", "tgt", "flow"))
     t = torch.tensor([710, 64], dtype=torch.long)
     with torch.no_grad():
         latent = m.ae.encode(img)
@@ -62,7 +63,7 @@ def main():
         ae_fwd = quiet(m.ae, img, flow)
         ae_lat = quiet(m.ae, img, flow, return_latent=True)
     first, cond, flow_n = quiet(m.preprocess, (img, tgt, flow), aug=False)
-    noise = torch.randn(first.shape, generator=g)
+    noise = torch.from_numpy(inputs["noise"])
     grabbed = {}
 
     def hook(_m, _i, out):
@@ -76,10 +77,12 @@ def main():
     h.remove()
     torch.autograd.set_detect_anomaly(False)
     fp = grabbed["flow_pred"]
+    assert torch.equal(cond, latent / float(latent_golden.LATENT_MAX))
     out = dict(ae_seed=AE_SEED, seed=MODEL_SEED, ae_w_sums=ae_sums, ae_w_asums=ae_asums, w_sums=sums, w_asums=asums,
-               img=img.numpy(), tgt=tgt.numpy(), flow=flow.numpy(), t=t.numpy(), noise=noise.numpy(),
-               latent=latent.numpy(), decoded=decoded.numpy(), ae_forward=ae_fwd.numpy(), ae_forward_latent=ae_lat.numpy(),
-               first=first.detach().numpy(), cond=cond.numpy(), flow_n=flow_n.numpy(), flow_pred=fp.detach().numpy(),
+               input_seed=INPUT_SEED, input_sums=latent_golden.input_sums(inputs), t=t.numpy(),
+               latent=latent.numpy(), decoded=decoded.numpy(), ae_forward=ae_fwd.numpy(),
+               ae_forward_latent_offset=latent_golden.forward_latent_offset(ae_lat.numpy(), first.detach().numpy()),
+               first=first.detach().numpy(), flow_n=flow_n.numpy(), flow_pred=fp.detach().numpy(),
                grad_flow_pred=fp.grad.numpy(), loss=np.array(float(loss)),
                grad_final_conv_w=m.unet.final_conv.weight.grad.numpy(), grad_final_conv_b=m.unet.final_conv.bias.grad.numpy(),
                grad_init_conv_w=m.unet.init_conv.weight.grad.numpy(), grad_init_conv_b=m.unet.init_conv.bias.grad.numpy())

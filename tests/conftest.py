@@ -32,6 +32,20 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(skip)
 
 
+GOLDEN_THREADS = 8       # intra-op threads the goldens were computed with (oracle/make_goldens.py)
+
+
+@pytest.fixture
+def golden_threads():
+    """Run the test on GOLDEN_THREADS CPU threads.  The CPU convolutions split their sums by thread count, and the oracle
+    tests' fp32 tolerances against the reference's goldens are set at the last bits of that summation order."""
+    import torch
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.fixture(scope="session")
 def golden():
     import numpy as np

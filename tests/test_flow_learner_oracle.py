@@ -4,9 +4,12 @@ host), and the host-side surface of the FlowLearner class here (parameter names,
 import random
 
 import numpy as np
+import pytest
 import torch
 
 from oracle import flowdiff_oracle as O
+
+pytestmark = pytest.mark.usefixtures("golden_threads")
 
 
 def T(a):

@@ -15,6 +15,8 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import latent_golden
+
 pytestmark = pytest.mark.gpu
 
 
@@ -55,7 +57,7 @@ def make_algo(g, tmp_path):
 
 
 def test_autoencoder_encode_decode_vs_reference(golden):
-    g = golden("latent_32x48")
+    g = latent_golden.load(golden("latent_32x48"))
     ae = make_autoencoder(g).cuda()
     img, flow = T(g["img"]).cuda(), T(g["flow"]).cuda()
     lat = ae.encode(img)
@@ -84,7 +86,7 @@ def test_autoencoder_encode_decode_vs_reference(golden):
 
 
 def test_latent_preprocess_and_loss_vs_reference(golden, tmp_path):
-    g = golden("latent_32x48")
+    g = latent_golden.load(golden("latent_32x48"))
     m = make_algo(g, tmp_path)
     first, cond, flow_n = m.preprocess((T(g["img"]).cuda(), T(g["tgt"]).cuda(), T(g["flow"]).cuda()), aug=False)
     assert first.shape == (2, 16, 32, 48) and cond.shape == (2, 16, 32, 48)
@@ -120,7 +122,7 @@ def test_latent_preprocess_and_loss_vs_reference(golden, tmp_path):
 
 
 def test_latent_training_step_sampling_and_validation(golden, tmp_path):
-    g = golden("latent_32x48")
+    g = latent_golden.load(golden("latent_32x48"))
     m = make_algo(g, tmp_path)
     m.model.sampling_timesteps, m.model.is_ddim_sampling = 3, True
     opt = m.configure_optimizers()

@@ -11,6 +11,8 @@ import torch
 
 from oracle import flowdiff_oracle as O
 
+pytestmark = pytest.mark.usefixtures("golden_threads")
+
 
 def T(a):
     return torch.from_numpy(np.asarray(a))

@@ -7,9 +7,12 @@ the rounding level; measured 0).  The map state -> next state is ill-conditioned
 moves splat weight between neighbouring cells), so rounding differences grow ~8x per step: measured max |err| 2e-7, 2e-5,
 7e-5, 5e-4, 6e-3 over the five steps -- asserted: first step 2e-6, whole trajectory 2e-2 max and 1e-4 mean."""
 import numpy as np
+import pytest
 import torch
 
 from oracle import flowdiff_oracle as O
+
+pytestmark = pytest.mark.usefixtures("golden_threads")
 
 
 def T(a):

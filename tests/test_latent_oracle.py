@@ -8,9 +8,13 @@ construction order and initialisers as the reference; the per-tensor checksums i
 Tolerances: fp32 on both sides with different summation orders -> 2e-5 absolute on the [-1, 1] latents / [0, 1] images;
 the level^4-weighted pyramid loss 2e-4 relative end to end, 2e-6 given the reference's own flow prediction."""
 import numpy as np
+import pytest
 import torch
 
 from oracle import flowdiff_oracle as O
+from oracle import latent_golden
+
+pytestmark = pytest.mark.usefixtures("golden_threads")
 
 
 def T(a):
@@ -49,7 +53,7 @@ def same_with_nans(a, b, atol):
 
 
 def test_autoencoder_and_preprocess(golden):
-    g = golden("latent_32x48")
+    g = latent_golden.load(golden("latent_32x48"))
     sd = ae_state(g)
     img, flow = T(g["img"]), T(g["flow"])
     with torch.no_grad():
@@ -71,7 +75,7 @@ def test_autoencoder_and_preprocess(golden):
 
 
 def test_latent_p_losses_target(golden):
-    g = golden("latent_32x48")
+    g = latent_golden.load(golden("latent_32x48"))
     first, cond, flow_n, t, noise = T(g["first"]), T(g["cond"]), T(g["flow_n"]), T(g["t"]), T(g["noise"])
     # given the reference's own flow prediction: value and gradient of the 16-channel pyramid loss
     fp = T(g["flow_pred"]).clone().requires_grad_(True)

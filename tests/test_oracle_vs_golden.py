@@ -6,6 +6,8 @@ import pytest
 import torch
 
 from oracle import flowdiff_oracle as O
+
+pytestmark = pytest.mark.usefixtures("golden_threads")
 from opticalflowdiffusion_b200.unet_params import UnetParams
 
 
