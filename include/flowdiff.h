@@ -136,6 +136,15 @@ FD_API int fd_q_sample(const float* x0, const float* noise, const int64_t* t, co
 FD_API int fd_ddim_step(const float* x, const float* model_out, const float* noise, float* x_next, float* x0_out,
                  long n, float recip, float recipm1, float sqrt_alpha_next, float c, float sigma,
                  int last, void* stream);
+/* DPM-Solver++ multistep step (data prediction, orders 1-3; not in the reference):
+ * D0 = clamp(model_out,-1,1); d_out = D0;
+ * last ? x_next = D0 : x_next = ((cx*x + c0*D0) + c1*d_hist1) + c2*d_hist2, fp32, no FMA, in that order.
+ * A term with a zero coefficient is not evaluated (NaN in unused history does not leak); d_hist1 / d_hist2 may be
+ * NULL when c1 / c2 == 0. Aliasing: x_next == x and d_out == d_hist2 are allowed (each element is read before it
+ * is written), so two rotating history buffers suffice for order 3; no other pair may overlap. */
+FD_API int fd_dpmpp_step(const float* x, const float* model_out, const float* d_hist1, const float* d_hist2,
+                  float* x_next, float* d_out, long n, float cx, float c0, float c1, float c2, int last,
+                  void* stream);
 /* x0 = clamp(model_out,-1,1); x_next = coef1*x0 + coef2*x + (noise ? sigma*noise : 0) */
 FD_API int fd_ddpm_step(const float* x, const float* model_out, const float* noise, float* x_next, float* x0_out,
                  long n, float coef1, float coef2, float sigma, void* stream);

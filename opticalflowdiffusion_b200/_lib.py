@@ -47,6 +47,7 @@ SIGNATURES = {
     "fd_q_sample": (c_int, [_P, _P, _P, _P, _P, _P, _I, _L, _P]),
     "fd_ddim_step": (c_int, [_P, _P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _I, _P]),
     "fd_ddpm_step": (c_int, [_P, _P, _P, _P, _P, _L, _F, _F, _F, _P]),
+    "fd_dpmpp_step": (c_int, [_P, _P, _P, _P, _P, _P, _L, _F, _F, _F, _F, _I, _P]),
     "fd_pack_input": (c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "fd_pack_input_pad": (c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
     "fd_pack_input_wide": (c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),

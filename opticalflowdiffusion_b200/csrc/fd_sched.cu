@@ -2,6 +2,7 @@
 //   q_sample          denoising_diffusion.py:806-812
 //   DDIM update       denoising_diffusion.py:653-656 (clamp), 595-599 (eps from x0), 757-767
 //   DDPM update       denoising_diffusion.py:666-698, 613-623
+//   DPM-Solver++      multistep data-prediction update, orders 1-3 (Lu et al., arXiv:2211.01095); not in the reference
 //   nan_mse/nanmean   warp.py:260-271, denoising_diffusion.py:906-908,973
 // Pure streaming kernels (HBM roofline): 128-bit accesses, one pass, every per-step scalar is a
 // kernel argument computed on the host from the fp32 schedule tables, so the whole update is one
@@ -77,6 +78,64 @@ __global__ void __launch_bounds__(256) ddim_kernel(const float* __restrict__ x, 
       const float r = ddim_one(x[i], __ldg(mo + i), noise ? __ldg(noise + i) : 0.f, noise != nullptr, a, z);
       xn[i] = r;
       if (x0_out) x0_out[i] = z;
+    }
+  }
+}
+
+// DPM-Solver++ multistep (data prediction, deterministic): x_next = cx*x + c0*D0 + c1*D1 + c2*D2 with D0 = clamp(mo).
+// A term whose coefficient is 0 is not evaluated, so a NaN in an unused history slot cannot leak in as 0*NaN.
+struct DpmppArgs {
+  float cx, c0, c1, c2;
+  int last;
+};
+
+__device__ __forceinline__ float dpmpp_one(float x, float mo, float d1, float d2, const DpmppArgs& a, float& d0o) {
+  const float d0 = clamp1(mo);
+  d0o = d0;
+  if (a.last) return d0;
+  float r = __fadd_rn(__fmul_rn(a.cx, x), __fmul_rn(a.c0, d0));
+  if (a.c1 != 0.f) r = __fadd_rn(r, __fmul_rn(a.c1, d1));
+  if (a.c2 != 0.f) r = __fadd_rn(r, __fmul_rn(a.c2, d2));
+  return r;
+}
+
+// x / x_next and d_hist2 / d_out may alias (each element is read, then written, by the same thread): no __restrict__
+// and no read-only-cache loads on those four.
+template <int VEC>
+__global__ void __launch_bounds__(256) dpmpp_kernel(const float* x, const float* __restrict__ mo,
+                                                    const float* __restrict__ d1, const float* d2, float* xn,
+                                                    float* d_out, long n, DpmppArgs a) {
+  const long items = n / VEC;
+  const long stride = (long)gridDim.x * blockDim.x;
+  const long tid = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  for (long i = tid; i < items; i += stride) {
+    if (VEC == 4) {
+      const float4 xv = reinterpret_cast<const float4*>(x)[i];
+      const float4 mv = __ldg(reinterpret_cast<const float4*>(mo) + i);
+      float4 h1 = make_float4(0.f, 0.f, 0.f, 0.f), h2 = h1;
+      if (d1) h1 = __ldg(reinterpret_cast<const float4*>(d1) + i);
+      if (d2) h2 = reinterpret_cast<const float4*>(d2)[i];
+      float4 r, z;
+      r.x = dpmpp_one(xv.x, mv.x, h1.x, h2.x, a, z.x);
+      r.y = dpmpp_one(xv.y, mv.y, h1.y, h2.y, a, z.y);
+      r.z = dpmpp_one(xv.z, mv.z, h1.z, h2.z, a, z.z);
+      r.w = dpmpp_one(xv.w, mv.w, h1.w, h2.w, a, z.w);
+      reinterpret_cast<float4*>(xn)[i] = r;
+      reinterpret_cast<float4*>(d_out)[i] = z;
+    } else {
+      float z;
+      const float r = dpmpp_one(x[i], __ldg(mo + i), d1 ? __ldg(d1 + i) : 0.f, d2 ? d2[i] : 0.f, a, z);
+      xn[i] = r;
+      d_out[i] = z;
+    }
+  }
+  if (VEC == 4) {      // scalar tail: the last n % 4 elements
+    const long i = items * 4 + tid;
+    if (i < n) {
+      float z;
+      const float r = dpmpp_one(x[i], __ldg(mo + i), d1 ? __ldg(d1 + i) : 0.f, d2 ? d2[i] : 0.f, a, z);
+      xn[i] = r;
+      d_out[i] = z;
     }
   }
 }
@@ -220,6 +279,28 @@ int fd_ddim_step(const float* x, const float* model_out, const float* noise, flo
     ddim_kernel<4><<<egrid(n / 4), 256, 0, (cudaStream_t)stream>>>(x, model_out, noise, x_next, x0_out, n, a);
   else
     ddim_kernel<1><<<egrid(n), 256, 0, (cudaStream_t)stream>>>(x, model_out, noise, x_next, x0_out, n, a);
+  FD_LAUNCH_CHECK();
+  return FD_OK;
+}
+
+int fd_dpmpp_step(const float* x, const float* model_out, const float* d_hist1, const float* d_hist2, float* x_next,
+                  float* d_out, long n, float cx, float c0, float c1, float c2, int last, void* stream) {
+  FD_REQUIRE(x && model_out && x_next && d_out && n > 0, "dpmpp_step: bad argument");
+  if (last) c1 = c2 = 0.f;
+  FD_REQUIRE(c1 == 0.f || d_hist1 != nullptr, "dpmpp_step: c1 != 0 needs d_hist1");
+  FD_REQUIRE(c2 == 0.f || d_hist2 != nullptr, "dpmpp_step: c2 != 0 needs d_hist2");
+  if (c1 == 0.f) d_hist1 = nullptr;    // unused history is not read
+  if (c2 == 0.f) d_hist2 = nullptr;
+  FD_REQUIRE(d_out != x_next && d_out != d_hist1 && d_out != x && x_next != d_hist1 && x_next != d_hist2,
+             "dpmpp_step: only x_next == x and d_out == d_hist2 may alias");
+  DpmppArgs a{cx, c0, c1, c2, last};
+  const bool v4 = aligned16(x) && aligned16(model_out) && aligned16(d_hist1) && aligned16(d_hist2) &&
+                  aligned16(x_next) && aligned16(d_out);
+  if (v4)
+    dpmpp_kernel<4><<<egrid(n / 4), 256, 0, (cudaStream_t)stream>>>(x, model_out, d_hist1, d_hist2, x_next, d_out, n,
+                                                                  a);
+  else
+    dpmpp_kernel<1><<<egrid(n), 256, 0, (cudaStream_t)stream>>>(x, model_out, d_hist1, d_hist2, x_next, d_out, n, a);
   FD_LAUNCH_CHECK();
   return FD_OK;
 }

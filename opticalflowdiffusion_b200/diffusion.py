@@ -40,6 +40,47 @@ def ddim_time_pairs(total: int, steps: int) -> List[Tuple[int, int]]:
     return list(zip(times[:-1], times[1:]))
 
 
+def dpmpp_coeffs(alphas_cumprod: Sequence[float], times: Sequence[int], i: int, order: int):
+    """Coefficients of step ``i`` of the multistep DPM-Solver++ (data prediction; Lu et al., arXiv:2211.01095) on the
+    grid ``times`` (descending, ending at -1): ``x_next = cx*x + c0*D0 + c1*D1 + c2*D2`` with D0 the clamped prediction at
+    ``times[i]`` and D1 / D2 those at ``times[i-1]`` / ``times[i-2]``.  float64 from the fp32 ``alphas_cumprod`` table.
+    The step uses order ``min(order, i + 1)``; the final step (to -1) returns D0: ``(0, 1, 0, 0, last=1)``.
+    Order 1 is DDIM with eta = 0: ``cx = sigma_t / sigma_s``, ``c0 = alpha_t - alpha_s * sigma_t / sigma_s``."""
+    s, t = int(times[i]), int(times[i + 1])
+    if t < 0:
+        return 0.0, 1.0, 0.0, 0.0, 1
+    k = min(int(order), i + 1)
+
+    def alpha_sigma_lambda(tt):
+        a = float(alphas_cumprod[tt])
+        al, sg = math.sqrt(a), math.sqrt(1.0 - a)
+        return al, sg, math.log(al) - math.log(sg)
+
+    _, sigma_s, lam_s = alpha_sigma_lambda(s)
+    alpha_t, sigma_t, lam_t = alpha_sigma_lambda(t)
+    h = lam_t - lam_s
+    phi1 = math.expm1(-h)
+    cx, c0, c1, c2 = sigma_t / sigma_s, -alpha_t * phi1, 0.0, 0.0
+    if k >= 2:
+        lam_1 = alpha_sigma_lambda(int(times[i - 1]))[2]
+        r0 = (lam_s - lam_1) / h
+        if k == 2:                                 # - alpha_t*phi1/2 * (D0 - D1)/r0
+            c0 += -0.5 * alpha_t * phi1 / r0
+            c1 = 0.5 * alpha_t * phi1 / r0
+        else:                                      # + alpha_t*phi2*Dd1 - alpha_t*phi3*Dd2
+            lam_2 = alpha_sigma_lambda(int(times[i - 2]))[2]
+            r1 = (lam_1 - lam_2) / h
+            phi2 = phi1 / h + 1.0
+            phi3 = phi2 / h - 0.5
+            f = r0 / (r0 + r1)
+            m = 1.0 / (r0 + r1)
+            # E0 = (D0 - D1)/r0, E1 = (D1 - D2)/r1, Dd1 = E0 + f*(E0 - E1), Dd2 = m*(E0 - E1), expanded in D0, D1, D2
+            c0 += alpha_t * phi2 * (1.0 + f) / r0 - alpha_t * phi3 * m / r0
+            c1 = (alpha_t * phi2 * (-(1.0 + f) / r0 - f / r1) + alpha_t * phi3 * m * (1.0 / r0 + 1.0 / r1))
+            c2 = alpha_t * phi2 * f / r1 - alpha_t * phi3 * m / r1
+    return cx, c0, c1, c2, 0
+
+
 class _SqErrSums(torch.autograd.Function):
     """(sum over non-NaN pairs of (a-b)^2, their count) with the gradient wrt ``a`` (warp.py:260-271 under autograd)."""
 
@@ -80,11 +121,20 @@ class ConditionalDiffusion(nn.Module):
     def __init__(self, model: nn.Module, image_size: Union[int, Sequence[int]], timesteps: int = 1000,
                  sampling_timesteps: Optional[int] = None, objective: str = "pred_x0", beta_schedule: str = "sigmoid",
                  ddim_sampling_eta: float = 0.0, auto_normalize: bool = False, min_snr_loss_weight: bool = True,
-                 min_snr_gamma: float = 5.0, conditioned: bool = True, channels: int = 2, noise_space: str = "image"):
+                 min_snr_gamma: float = 5.0, conditioned: bool = True, channels: int = 2, noise_space: str = "image",
+                 sampler: Optional[str] = None, solver_order: int = 2):
         super().__init__()
         if objective != "pred_x0" or beta_schedule != "sigmoid" or noise_space != "image" or auto_normalize:
             raise NotImplementedError("flow_diffuser uses objective=pred_x0, sigmoid schedule, image noise space, "
                                       "auto_normalize=False (flow_diffuser.py:117-127); nothing else is on the hot path")
+        if sampler not in (None, "dpmpp"):
+            raise ValueError(f"sampler must be null (DDIM / DDPM as the reference) or 'dpmpp', not {sampler!r}")
+        if int(solver_order) not in (1, 2, 3):
+            raise ValueError(f"solver_order must be 1, 2 or 3, not {solver_order}")
+        if sampler == "dpmpp" and float(ddim_sampling_eta) > 0:
+            raise NotImplementedError("sampler='dpmpp' is the deterministic solver: ddim_sampling_eta must be 0")
+        self.sampler = sampler           # None: DDIM when sampling_timesteps < timesteps, else DDPM; "dpmpp": DPM-Solver++
+        self.solver_order = int(solver_order)
         self.model = model
         self.channels = channels
         self.conditioned = conditioned
@@ -92,7 +142,7 @@ class ConditionalDiffusion(nn.Module):
         self.objective = objective
         self.image_size = (image_size, image_size) if isinstance(image_size, int) else tuple(int(v) for v in image_size)
         self.self_condition = False
-        self._graphs = {}          # CUDA graphs of the DDIM loop, keyed by shapes (sample(..., use_cuda_graph=True))
+        self._graphs = {}          # CUDA graphs of the DDIM / DPM-Solver++ loops, keyed by sampler and shapes
         self.graph_replayed_launches = 0   # kernels executed through graph replays (not seen by fd_launch_count)
 
         betas = sigmoid_beta_schedule(timesteps)
@@ -246,12 +296,53 @@ class ConditionalDiffusion(nn.Module):
         return (ret, additionals) if additional_tgt is not None else ret
 
     @torch.no_grad()
-    def _ddim_sample_graphed(self, shape, return_all_timesteps: bool, external_cond: Tensor, x_T: Optional[Tensor]):
-        """The whole eta = 0 DDIM loop (S UNet forwards + S fused updates, ~8k launches at S = 50) as ONE CUDA graph:
-        captured once per (shape, device), replayed with the inputs copied into static buffers.  Deterministic DDIM
-        draws no per-step noise, so only x_T is random and it is drawn outside the graph."""
+    def dpmpp_sample(self, shape, return_all_timesteps: bool = False, external_cond: Optional[Tensor] = None,
+                     additional_tgt: Optional[Tensor] = None, x_T: Optional[Tensor] = None):
+        """Multistep DPM-Solver++ (orders 1-3, ``self.solver_order``) on the DDIM time grid, with the contract and return
+        shapes of ``ddim_sample``.  One fused launch per step (``fd_dpmpp_step``) clamps the prediction, writes it into
+        the history slot the next steps read, and applies the update; two rotating slots hold D_{i-1} and D_{i-2}
+        (order 3 overwrites the older one in the same pass that reads it).  Order 1 is DDIM with eta = 0."""
+        if self.ddim_sampling_eta > 0:
+            raise NotImplementedError("sampler='dpmpp' is the deterministic solver: ddim_sampling_eta must be 0")
+        lib = _lib.load(check_device=True)
         dev = self.device
-        key = (tuple(shape), bool(return_all_timesteps), tuple(external_cond.shape), dev.index)
+        B = shape[0]
+        pairs = ddim_time_pairs(self.num_timesteps, self.sampling_timesteps)
+        times = [p[0] for p in pairs] + [pairs[-1][1]]
+        ac = self._host["alphas_cumprod"].tolist()
+        img = (x_T.to(dev).float().contiguous().clone() if x_T is not None else torch.randn(shape, device=dev))
+        n = img.numel()
+        traj = None
+        if return_all_timesteps:
+            traj = torch.empty((len(pairs) + 1,) + tuple(img.shape), device=dev, dtype=torch.float32)
+            traj[0].copy_(img)
+        hist = (torch.empty_like(img), torch.empty_like(img))
+        additionals = [None]
+        for i, (time, _) in enumerate(pairs):
+            t = torch.full((B,), time, device=dev, dtype=torch.long)
+            out = self.model_with_condition(img, t, None, external_cond, additional_tgt)
+            out, add = self._split_model_out(out, additional_tgt)
+            additionals.append(add)
+            cx, c0, c1, c2, last = dpmpp_coeffs(ac, times, i, self.solver_order)
+            d_out = hist[i % 2]                 # D_{i-2}'s slot: read (order 3) and overwritten with D_i in one pass
+            d1 = hist[(i + 1) % 2] if c1 != 0.0 else None
+            d2 = d_out if c2 != 0.0 else None
+            nxt = traj[i + 1] if traj is not None else img
+            _lib.check(lib.fd_dpmpp_step(_lib.ptr(img), _lib.ptr(out), _lib.ptr(d1), _lib.ptr(d2), _lib.ptr(nxt),
+                                         _lib.ptr(d_out), n, cx, c0, c1, c2, last, _lib.stream()))
+            img = nxt
+        ret = traj.transpose(0, 1) if traj is not None else img
+        return (ret, additionals) if additional_tgt is not None else ret
+
+    @torch.no_grad()
+    def _sample_graphed(self, fn, shape, return_all_timesteps: bool, external_cond: Tensor, x_T: Optional[Tensor]):
+        """A whole deterministic sampling loop -- eta = 0 DDIM or DPM-Solver++, ``fn`` -- (S UNet forwards + S fused
+        updates, ~8k launches at S = 50) as ONE CUDA graph: captured once per (sampler, shape, device), replayed with the
+        inputs copied into static buffers.  Neither sampler draws per-step noise, so only x_T is random and it is drawn
+        outside the graph; the DPM-Solver++ history buffers are allocated inside the capture and live with the graph."""
+        dev = self.device
+        key = (fn.__name__, self.solver_order if fn == self.dpmpp_sample else None,
+               tuple(shape), bool(return_all_timesteps), tuple(external_cond.shape), dev.index)
         if x_T is None:
             x_T = torch.randn(shape, device=dev)
         # The graph holds raw pointers: to the packed bf16 weights and the concatenated time-MLP weights (both rewritten
@@ -270,13 +361,13 @@ class ConditionalDiffusion(nn.Module):
             side = torch.cuda.Stream(device=dev)
             side.wait_stream(torch.cuda.current_stream(dev))
             with torch.cuda.stream(side):        # eager warm-up: lazy one-time initialisation must not be captured
-                self.ddim_sample(shape, return_all_timesteps, s_cond, x_T=s_x)
+                fn(shape, return_all_timesteps, s_cond, x_T=s_x)
             torch.cuda.current_stream(dev).wait_stream(side)
             graph = torch.cuda.CUDAGraph()
             lib = _lib.load()
             n0 = lib.fd_launch_count()
             with torch.cuda.graph(graph):
-                s_out = self.ddim_sample(shape, return_all_timesteps, s_cond, x_T=s_x)
+                s_out = fn(shape, return_all_timesteps, s_cond, x_T=s_x)
             entry = (graph, s_cond, s_x, s_out, int(lib.fd_launch_count() - n0), ptrs)
             self._graphs[key] = entry
         graph, s_cond, s_x, s_out, n_kernels, _ = entry
@@ -298,9 +389,14 @@ class ConditionalDiffusion(nn.Module):
             hw = tuple(image_size) if image_size is not None else self.image_size
         shape = (batch_size, self.channels) + hw
         from .unet import Unet
+        if self.sampler == "dpmpp":
+            if use_cuda_graph and additional_tgt is None and external_cond is not None and isinstance(self.model, Unet):
+                return self._sample_graphed(self.dpmpp_sample, shape, return_all_timesteps, external_cond, kw.get("x_T"))
+            return self.dpmpp_sample(shape, return_all_timesteps=return_all_timesteps, external_cond=external_cond,
+                                     additional_tgt=additional_tgt, **kw)
         if (use_cuda_graph and self.is_ddim_sampling and self.ddim_sampling_eta == 0.0 and additional_tgt is None
                 and external_cond is not None and kw.get("noises") is None and isinstance(self.model, Unet)):
-            return self._ddim_sample_graphed(shape, return_all_timesteps, external_cond, kw.get("x_T"))
+            return self._sample_graphed(self.ddim_sample, shape, return_all_timesteps, external_cond, kw.get("x_T"))
         fn = self.ddim_sample if self.is_ddim_sampling else self.p_sample_loop
         return fn(shape, return_all_timesteps=return_all_timesteps, external_cond=external_cond,
                   additional_tgt=additional_tgt, **kw)

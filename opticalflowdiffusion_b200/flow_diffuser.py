@@ -7,7 +7,8 @@ parameter names (``unet.*``, ``_model.*``, ``model.*`` aliases and the 13 schedu
 experiment runner that drives the reference class (experiments/exp_base.py:120-214) drives this one.
 
 New optional config keys (SURVEY.md section 8b): ``sampling_timesteps`` (DDIM when < ``timesteps``),
-``image_size`` as ``[H, W]``, ``return_all_timesteps`` (default true like the reference).
+``image_size`` as ``[H, W]``, ``return_all_timesteps`` (default true like the reference), ``sampler`` (null: the
+reference's DDIM / DDPM; ``dpmpp``: multistep DPM-Solver++ on the DDIM grid) with ``solver_order`` (1-3).
 
 When ``pytorch_lightning`` is importable the class derives from ``LightningModule``; otherwise from a
 minimal stand-in with the attributes the reference touches (``log_dict``, ``log``, ``global_step``,
@@ -211,7 +212,8 @@ class FlowDiffuser(_Base):
         self.model = ConditionalDiffusion(
             self._model, _cfg_get(cfg, "image_size", 128), objective="pred_x0", channels=channels, auto_normalize=False,
             noise_space="image" if cfg.noiser == "image" else "flow", timesteps=cfg.timesteps,
-            sampling_timesteps=_cfg_get(cfg, "sampling_timesteps"), min_snr_loss_weight=True)
+            sampling_timesteps=_cfg_get(cfg, "sampling_timesteps"), min_snr_loss_weight=True,
+            sampler=_cfg_get(cfg, "sampler"), solver_order=int(_cfg_get(cfg, "solver_order", 2)))
         self.return_all_timesteps = bool(_cfg_get(cfg, "return_all_timesteps", True))
         self.use_cuda_graph = bool(_cfg_get(cfg, "use_cuda_graph", False))
 
