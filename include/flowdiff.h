@@ -282,16 +282,9 @@ FD_API int fd_time_proj(const float* temb, const float* w, const float* bias, fl
  * workspace floats: fd_linattn_workspace_floats(N, HW). */
 FD_API size_t fd_linattn_workspace_floats(int N, int HW);
 FD_API int fd_linattn(const void* qkv, void* out, float* workspace, int N, int HW, void* stream);
-/* the two halves of fd_linattn, exposed for the fused blocks:
- * context: kv rows = [k(128) | v(128)] bf16, row_stride elements apart -> ctx_t bf16 [N][4][32 e][32 d]
- *          (softmax_n(k) v^T / HW, with the 32^-0.5 q scale folded in); workspace as fd_linattn_workspace_floats.
- * apply_fused (C in {64,128}): the whole Residual(PreNorm(LinearAttention)) tail of :81-87,127-135,224-243 in one pass:
- *          out = LayerNorm_g2(W_out (softmax_d(W_q LayerNorm_g1(x)) . ctx) + b_out) + x
- *          x,out bf16 (N,HW,C); wq bf16 [128][C]; wout bf16 [C][128]; g1,g2,bias fp32 [C]. */
+/* the context half of fd_linattn: kv rows = [k(128) | v(128)] bf16, row_stride elements apart -> ctx_t bf16
+ * [N][4][32 e][32 d] (softmax_n(k) v^T / HW, with the 32^-0.5 q scale folded in); workspace as fd_linattn_workspace_floats. */
 FD_API int fd_linattn_context(const void* kv, int row_stride, void* ctx_t, float* workspace, int N, int HW, void* stream);
-FD_API int fd_linattn_apply_fused(const void* x, const float* g1, const void* wq, const void* ctx_t, const void* wout,
-                                  const float* bias, const float* g2, void* out, int N, int HW, int C, float eps,
-                                  void* stream);
 
 /* Residual(PreNorm(LinearAttention)) (:81-87,127-135,216-244) for C in {64,128} on tcgen05 / TMEM / TMA: two passes over
  * x, no intermediate tensor in HBM (csrc/fd_linattn_tc.cu).

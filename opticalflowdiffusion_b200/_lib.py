@@ -64,7 +64,6 @@ SIGNATURES = {
     "fd_linattn_tc": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _P]),
     "fd_linattn": (c_int, [_P, _P, _P, _I, _I, _P]),
     "fd_linattn_context": (c_int, [_P, _I, _P, _P, _I, _I, _P]),
-    "fd_linattn_apply_fused": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _P]),
     "fd_attention": (c_int, [_P, _P, _I, _I, _P]),
     "fd_final_conv": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "fd_final_conv_crop": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),

@@ -25,8 +25,8 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr",
     "-DFD_BUILDING_LIB",
 ]
-if os.environ.get("FD_CONV_DIAG"):      # diagnostic build: compiles the FD_CONV_DBG switches into the conv kernels
-    NVCC_FLAGS.append("-DFD_CONV_DIAG")
+if os.environ.get("FD_DIAG"):           # diagnostic build: compiles the *_DBG switches into the kernels (fd_common.cuh)
+    NVCC_FLAGS.append("-DFD_DIAG")
 
 
 def _nvcc() -> str:

@@ -6,11 +6,7 @@
 //     (1) per pixel-chunk partial (running max, sum of exp, 32x32 context) with online rescaling,
 //     (2) combine chunks -> ctx (N,4,32,32) fp32,
 //     (3) apply: per pixel softmax_d(q) and the 32x32 product, ctx broadcast from shared memory.
-// Attention (:256-267): softmax(q^T k / sqrt(32)) v over N = HW tokens as a streaming
-//   (flash-style) kernel: S and P never leave registers, so the reference's N x N matrix (6.3 GB at
-//   batch 8, 440x1024) is never materialised.  bf16 mma.sync m16n8k16 with fp32 accumulation and
-//   online softmax; 1.6 % of the forward FLOPs.
-#include <stdlib.h>
+// Attention (:256-267): fd_attention / fd_attention_lse launch the tcgen05 kernel of fd_attention_tc.cu.
 
 #include "fd_mma.cuh"
 
@@ -315,237 +311,6 @@ __global__ void __launch_bounds__(128) linattn_apply_kernel(const __nv_bfloat16*
   }
 }
 
-// ------------------------------------------------------------------------------------------------
-// pass 3, fully fused for C in {64, 128} (the full- and half-resolution LinearAttention blocks):
-//   out = LayerNorm_g2( W_out * (softmax_d(W_q * LayerNorm_g1(x)) . ctx) + b_out ) + x
-// i.e. PreNorm (:127-135), the q third of to_qkv (:234), the q softmax and context product (:237-242), to_out's
-// 1x1 conv and LayerNorm (:224-227) and the Residual add (:81-87) -- one read of x, one write of out.  Three
-// chained bf16 mma.sync GEMMs per 16-pixel warp tile with the intermediate results kept in registers
-// (accumulator fragments are re-packed as the next GEMM's A fragments); weights live in shared memory.
-// ------------------------------------------------------------------------------------------------
-template <int C>
-struct ApCfg {
-  static constexpr int NW = C == 64 ? 8 : 4;                             // warps per block (16 pixels each)
-  static constexpr int TP = NW * 16;                                     // pixels per tile
-  static constexpr int XS = C + 8, WQS = C + 8, WOS = kHidden + 8;      // padded bf16 row strides
-  static constexpr int kXBytes = TP * XS * 2, kWqBytes = kHidden * WQS * 2, kCtBytes = kHidden * kCtStride * 2;
-  static constexpr int kWoBytes = C * WOS * 2, kVecBytes = 3 * C * 4;
-  static constexpr int kSmem = kXBytes + kWqBytes + kCtBytes + kWoBytes + kVecBytes;
-};
-
-template <int C>
-__global__ void __launch_bounds__(ApCfg<C>::NW * 32) linattn_apply_fused_kernel(
-    const __nv_bfloat16* __restrict__ x, const float* __restrict__ g1, const __nv_bfloat16* __restrict__ wq,
-    const __nv_bfloat16* __restrict__ ctx_t, const __nv_bfloat16* __restrict__ wout, const float* __restrict__ bias,
-    const float* __restrict__ g2, __nv_bfloat16* __restrict__ out, int HW, float eps) {
-  using A = ApCfg<C>;
-  constexpr int NTH = A::NW * 32, TP = A::TP;
-  constexpr int KS = C / 16;       // k-steps of the q GEMM
-  constexpr int NT = C / 8;        // n-tiles of the output GEMM
-  extern __shared__ __align__(16) uint8_t ap_smem[];
-  __nv_bfloat16* s_x = reinterpret_cast<__nv_bfloat16*>(ap_smem);
-  __nv_bfloat16* s_wq = reinterpret_cast<__nv_bfloat16*>(ap_smem + A::kXBytes);
-  __nv_bfloat16* s_ct = reinterpret_cast<__nv_bfloat16*>(ap_smem + A::kXBytes + A::kWqBytes);
-  __nv_bfloat16* s_wo = reinterpret_cast<__nv_bfloat16*>(ap_smem + A::kXBytes + A::kWqBytes + A::kCtBytes);
-  float* s_vec = reinterpret_cast<float*>(ap_smem + A::kXBytes + A::kWqBytes + A::kCtBytes + A::kWoBytes);
-  float* s_g1 = s_vec;
-  float* s_g2 = s_vec + C;
-  float* s_b = s_vec + 2 * C;
-  const int n = blockIdx.y;
-  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-  const int g = lane >> 2, tq = lane & 3;
-  // ---- stage weights once per block
-  for (int i = t; i < kHidden * (C / 8); i += NTH) {          // Wq: [128][C], 16-byte granules
-    const int r = i / (C / 8), c8 = i % (C / 8);
-    *reinterpret_cast<uint4*>(s_wq + r * A::WQS + c8 * 8) = __ldg(reinterpret_cast<const uint4*>(wq + (long)r * C) + c8);
-  }
-  for (int i = t; i < C * (kHidden / 8); i += NTH) {          // Wout: [C][128]
-    const int r = i / (kHidden / 8), c8 = i % (kHidden / 8);
-    *reinterpret_cast<uint4*>(s_wo + r * A::WOS + c8 * 8) = __ldg(reinterpret_cast<const uint4*>(wout + (long)r * kHidden) + c8);
-  }
-  for (int i = t; i < kHidden * (kD / 8); i += NTH) {         // ctx^T: [head*32 + e][d]
-    const int r = i / (kD / 8), c8 = i % (kD / 8);
-    *reinterpret_cast<uint4*>(s_ct + r * kCtStride + c8 * 8) =
-        __ldg(reinterpret_cast<const uint4*>(ctx_t + ((long)n * kHidden + r) * kD) + c8);
-  }
-  for (int i = t; i < C; i += NTH) {
-    s_g1[i] = g1[i];
-    s_g2[i] = g2[i];
-    s_b[i] = bias[i];
-  }
-  const __nv_bfloat16* xb = x + (long)n * HW * C;
-  __nv_bfloat16* ob = out + (long)n * HW * C;
-  const uint32_t sx = smem_addr(s_x);
-  const int ntiles = (HW + TP - 1) / TP;
-  for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-    const int p0 = tile * TP;
-    __syncthreads();       // previous tile written out; weights staged (first pass)
-    for (int i = t; i < TP * (C / 8); i += NTH) {
-      const int px = i / (C / 8), c8 = i % (C / 8);
-      const bool ok = p0 + px < HW;
-      cp_async16(sx + (px * A::XS + c8 * 8) * 2, xb + (long)(ok ? p0 + px : p0) * C + c8 * 8, ok);
-    }
-    cp_async_commit();
-    cp_async_wait<0>();
-    __syncthreads();
-    // ---- (1) PreNorm LayerNorm over channels, in A-fragment layout
-    const int mi = lane >> 3, r8 = lane & 7;
-    uint32_t xa[KS][4];
-#pragma unroll
-    for (int ks = 0; ks < KS; ++ks)
-      ldmatrix_x4(xa[ks], sx + ((warp * 16 + (mi & 1) * 8 + r8) * A::XS + ks * 16 + (mi >> 1) * 8) * 2);
-    float s0 = 0.f, s1 = 0.f;
-#pragma unroll
-    for (int ks = 0; ks < KS; ++ks) {
-      const float2 a0 = fd_unpack_bf16(xa[ks][0]), a1 = fd_unpack_bf16(xa[ks][1]);
-      const float2 a2 = fd_unpack_bf16(xa[ks][2]), a3 = fd_unpack_bf16(xa[ks][3]);
-      s0 += a0.x + a0.y + a2.x + a2.y;
-      s1 += a1.x + a1.y + a3.x + a3.y;
-    }
-    s0 += __shfl_xor_sync(0xffffffffu, s0, 1); s0 += __shfl_xor_sync(0xffffffffu, s0, 2);
-    s1 += __shfl_xor_sync(0xffffffffu, s1, 1); s1 += __shfl_xor_sync(0xffffffffu, s1, 2);
-    const float mu0 = s0 * (1.f / C), mu1 = s1 * (1.f / C);
-    float v0 = 0.f, v1 = 0.f;
-#pragma unroll
-    for (int ks = 0; ks < KS; ++ks) {
-      const float2 a0 = fd_unpack_bf16(xa[ks][0]), a1 = fd_unpack_bf16(xa[ks][1]);
-      const float2 a2 = fd_unpack_bf16(xa[ks][2]), a3 = fd_unpack_bf16(xa[ks][3]);
-      v0 += (a0.x - mu0) * (a0.x - mu0) + (a0.y - mu0) * (a0.y - mu0) + (a2.x - mu0) * (a2.x - mu0) + (a2.y - mu0) * (a2.y - mu0);
-      v1 += (a1.x - mu1) * (a1.x - mu1) + (a1.y - mu1) * (a1.y - mu1) + (a3.x - mu1) * (a3.x - mu1) + (a3.y - mu1) * (a3.y - mu1);
-    }
-    v0 += __shfl_xor_sync(0xffffffffu, v0, 1); v0 += __shfl_xor_sync(0xffffffffu, v0, 2);
-    v1 += __shfl_xor_sync(0xffffffffu, v1, 1); v1 += __shfl_xor_sync(0xffffffffu, v1, 2);
-    const float r0 = rsqrtf(v0 * (1.f / C) + eps), r1 = rsqrtf(v1 * (1.f / C) + eps);
-#pragma unroll
-    for (int ks = 0; ks < KS; ++ks) {
-      const int c = ks * 16 + 2 * tq;
-      const float ga = s_g1[c], gb = s_g1[c + 1], gc = s_g1[c + 8], gd = s_g1[c + 9];
-      const float2 a0 = fd_unpack_bf16(xa[ks][0]), a1 = fd_unpack_bf16(xa[ks][1]);
-      const float2 a2 = fd_unpack_bf16(xa[ks][2]), a3 = fd_unpack_bf16(xa[ks][3]);
-      xa[ks][0] = fd_pack_bf16((a0.x - mu0) * r0 * ga, (a0.y - mu0) * r0 * gb);
-      xa[ks][1] = fd_pack_bf16((a1.x - mu1) * r1 * ga, (a1.y - mu1) * r1 * gb);
-      xa[ks][2] = fd_pack_bf16((a2.x - mu0) * r0 * gc, (a2.y - mu0) * r0 * gd);
-      xa[ks][3] = fd_pack_bf16((a3.x - mu1) * r1 * gc, (a3.y - mu1) * r1 * gd);
-    }
-    // ---- (2) per head: q = y Wq^T, softmax over d, out_h = softmax(q) ctx_h ; collected as A fragments (K = 128)
-    uint32_t oa[8][4];
-#pragma unroll
-    for (int h = 0; h < kHeads; ++h) {
-      float q[4][4];
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) q[nt][j] = 0.f;
-#pragma unroll
-      for (int ks = 0; ks < KS; ++ks)
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
-          const __nv_bfloat16* wr = s_wq + (h * kD + nt * 8 + g) * A::WQS + ks * 16 + 2 * tq;
-          mma_bf16(q[nt], xa[ks], *reinterpret_cast<const uint32_t*>(wr), *reinterpret_cast<const uint32_t*>(wr + 8));
-        }
-      float m0 = q[0][0], m1 = q[0][2];
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt) {
-        m0 = fmaxf(m0, fmaxf(q[nt][0], q[nt][1]));
-        m1 = fmaxf(m1, fmaxf(q[nt][2], q[nt][3]));
-      }
-      m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 1)); m0 = fmaxf(m0, __shfl_xor_sync(0xffffffffu, m0, 2));
-      m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 1)); m1 = fmaxf(m1, __shfl_xor_sync(0xffffffffu, m1, 2));
-      float e0 = 0.f, e1 = 0.f;
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt) {
-        q[nt][0] = __expf(q[nt][0] - m0); q[nt][1] = __expf(q[nt][1] - m0);
-        q[nt][2] = __expf(q[nt][2] - m1); q[nt][3] = __expf(q[nt][3] - m1);
-        e0 += q[nt][0] + q[nt][1];
-        e1 += q[nt][2] + q[nt][3];
-      }
-      e0 += __shfl_xor_sync(0xffffffffu, e0, 1); e0 += __shfl_xor_sync(0xffffffffu, e0, 2);
-      e1 += __shfl_xor_sync(0xffffffffu, e1, 1); e1 += __shfl_xor_sync(0xffffffffu, e1, 2);
-      const float i0 = __fdividef(1.f, e0), i1 = __fdividef(1.f, e1);
-      float o[4][4];
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) o[nt][j] = 0.f;
-#pragma unroll
-      for (int kk = 0; kk < 2; ++kk) {
-        uint32_t qa[4];
-        qa[0] = fd_pack_bf16(q[2 * kk][0] * i0, q[2 * kk][1] * i0);
-        qa[1] = fd_pack_bf16(q[2 * kk][2] * i1, q[2 * kk][3] * i1);
-        qa[2] = fd_pack_bf16(q[2 * kk + 1][0] * i0, q[2 * kk + 1][1] * i0);
-        qa[3] = fd_pack_bf16(q[2 * kk + 1][2] * i1, q[2 * kk + 1][3] * i1);
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
-          const __nv_bfloat16* cr = s_ct + (h * kD + nt * 8 + g) * kCtStride + kk * 16 + 2 * tq;
-          mma_bf16(o[nt], qa, *reinterpret_cast<const uint32_t*>(cr), *reinterpret_cast<const uint32_t*>(cr + 8));
-        }
-      }
-#pragma unroll
-      for (int kk = 0; kk < 2; ++kk) {
-        oa[2 * h + kk][0] = fd_pack_bf16(o[2 * kk][0], o[2 * kk][1]);
-        oa[2 * h + kk][1] = fd_pack_bf16(o[2 * kk][2], o[2 * kk][3]);
-        oa[2 * h + kk][2] = fd_pack_bf16(o[2 * kk + 1][0], o[2 * kk + 1][1]);
-        oa[2 * h + kk][3] = fd_pack_bf16(o[2 * kk + 1][2], o[2 * kk + 1][3]);
-      }
-    }
-    // ---- (3) to_out 1x1 conv: o2 = out Wout^T + b
-    float o2[NT][4];
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      const float b0 = s_b[nt * 8 + 2 * tq], b1 = s_b[nt * 8 + 2 * tq + 1];
-      o2[nt][0] = b0; o2[nt][1] = b1; o2[nt][2] = b0; o2[nt][3] = b1;
-    }
-#pragma unroll
-    for (int ks = 0; ks < 8; ++ks)
-#pragma unroll
-      for (int nt = 0; nt < NT; ++nt) {
-        const __nv_bfloat16* wr = s_wo + (nt * 8 + g) * A::WOS + ks * 16 + 2 * tq;
-        mma_bf16(o2[nt], oa[ks], *reinterpret_cast<const uint32_t*>(wr), *reinterpret_cast<const uint32_t*>(wr + 8));
-      }
-    // ---- (4) LayerNorm over the C outputs of each pixel, gain g2, + residual x
-    float t0 = 0.f, t1 = 0.f;
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      t0 += o2[nt][0] + o2[nt][1];
-      t1 += o2[nt][2] + o2[nt][3];
-    }
-    t0 += __shfl_xor_sync(0xffffffffu, t0, 1); t0 += __shfl_xor_sync(0xffffffffu, t0, 2);
-    t1 += __shfl_xor_sync(0xffffffffu, t1, 1); t1 += __shfl_xor_sync(0xffffffffu, t1, 2);
-    const float n0 = t0 * (1.f / C), n1 = t1 * (1.f / C);
-    float w0 = 0.f, w1 = 0.f;
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      w0 += (o2[nt][0] - n0) * (o2[nt][0] - n0) + (o2[nt][1] - n0) * (o2[nt][1] - n0);
-      w1 += (o2[nt][2] - n1) * (o2[nt][2] - n1) + (o2[nt][3] - n1) * (o2[nt][3] - n1);
-    }
-    w0 += __shfl_xor_sync(0xffffffffu, w0, 1); w0 += __shfl_xor_sync(0xffffffffu, w0, 2);
-    w1 += __shfl_xor_sync(0xffffffffu, w1, 1); w1 += __shfl_xor_sync(0xffffffffu, w1, 2);
-    const float q0 = rsqrtf(w0 * (1.f / C) + eps), q1 = rsqrtf(w1 * (1.f / C) + eps);
-    __nv_bfloat16* row0 = s_x + (warp * 16 + g) * A::XS;
-    __nv_bfloat16* row1 = row0 + 8 * A::XS;
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      const int c = nt * 8 + 2 * tq;
-      const float ga = s_g2[c], gb = s_g2[c + 1];
-      const float2 x0 = fd_unpack_bf16(*reinterpret_cast<const uint32_t*>(row0 + c));     // residual: this thread's own elements
-      const float2 x1 = fd_unpack_bf16(*reinterpret_cast<const uint32_t*>(row1 + c));
-      *reinterpret_cast<uint32_t*>(row0 + c) = fd_pack_bf16((o2[nt][0] - n0) * q0 * ga + x0.x, (o2[nt][1] - n0) * q0 * gb + x0.y);
-      *reinterpret_cast<uint32_t*>(row1 + c) = fd_pack_bf16((o2[nt][2] - n1) * q1 * ga + x1.x, (o2[nt][3] - n1) * q1 * gb + x1.y);
-    }
-    __syncwarp();
-    // ---- (5) the warp's 16 rows -> global, 16-byte coalesced
-#pragma unroll
-    for (int it = 0; it < (16 * (C / 8)) / 32; ++it) {
-      const int idx = it * 32 + lane;
-      const int px = idx / (C / 8), c8 = idx % (C / 8);
-      const int p = p0 + warp * 16 + px;
-      if (p < HW)
-        *reinterpret_cast<uint4*>(ob + (long)p * C + c8 * 8) =
-            *reinterpret_cast<const uint4*>(s_x + (warp * 16 + px) * A::XS + c8 * 8);
-    }
-  }
-}
-
 int la_chunks(int N, int HW, int* chunk_px) {
   // one wave: at most 3 resident blocks per SM (68 KB smem each) in total, chunk a multiple of the tile
   int want = (FD_NUM_SMS * 3) / N;
@@ -555,172 +320,6 @@ int la_chunks(int N, int HW, int* chunk_px) {
   if (px < kLaTile) px = kLaTile;
   *chunk_px = px;
   return (HW + px - 1) / px;
-}
-
-// ------------------------------------------------------------------------------------------------
-// full attention (flash-style), mma.sync m16n8k16 bf16
-//   block = 8 warps x 16 queries, K/V tiles of 64 keys double-buffered with cp.async (one __syncthreads per tile);
-//   Q fragments live in registers, K fragments come from ldmatrix, V fragments from ldmatrix.trans (V stays
-//   row-major [key][d] in smem), S / P never leave registers; online softmax in the exp2 domain.
-// ------------------------------------------------------------------------------------------------
-constexpr int kBQ = 128, kBK = 64;
-constexpr int kKvStride = kD + 8;                  // bf16 per K / V row: 80 B, conflict-free ldmatrix
-constexpr int kKvTile = kBK * kKvStride;           // elements per K (or V) tile
-
-__global__ void __launch_bounds__(256) attention_kernel(const __nv_bfloat16* __restrict__ qkv,
-                                                        __nv_bfloat16* __restrict__ out, float* __restrict__ lse, int HW,
-                                                        float scale_log2) {
-  __shared__ __align__(16) __nv_bfloat16 s_k[2][kKvTile];
-  __shared__ __align__(16) __nv_bfloat16 s_v[2][kKvTile];
-  const int n = blockIdx.z, head = blockIdx.y;
-  const int q0 = blockIdx.x * kBQ;
-  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-  const int g = lane >> 2, tq = lane & 3;
-  const __nv_bfloat16* base = qkv + (long)n * HW * kQkv;
-  const int row0 = q0 + warp * 16 + g, row1 = row0 + 8;
-
-  uint32_t qa[2][4];
-#pragma unroll
-  for (int kk = 0; kk < 2; ++kk) {
-    const int c0 = head * kD + kk * 16 + 2 * tq;
-    qa[kk][0] = row0 < HW ? __ldg(reinterpret_cast<const uint32_t*>(base + (long)row0 * kQkv + c0)) : 0u;
-    qa[kk][1] = row1 < HW ? __ldg(reinterpret_cast<const uint32_t*>(base + (long)row1 * kQkv + c0)) : 0u;
-    qa[kk][2] = row0 < HW ? __ldg(reinterpret_cast<const uint32_t*>(base + (long)row0 * kQkv + c0 + 8)) : 0u;
-    qa[kk][3] = row1 < HW ? __ldg(reinterpret_cast<const uint32_t*>(base + (long)row1 * kQkv + c0 + 8)) : 0u;
-  }
-  float o[4][4];
-#pragma unroll
-  for (int dt = 0; dt < 4; ++dt)
-#pragma unroll
-    for (int i = 0; i < 4; ++i) o[dt][i] = 0.f;
-  float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-
-  const uint32_t sk = smem_addr(&s_k[0][0]), sv = smem_addr(&s_v[0][0]);
-  auto issue_tile = [&](int k0, int buf) {
-    // 64 keys x (4 + 4) granules of 16 B: 512 cp.async for 256 threads
-#pragma unroll
-    for (int it = 0; it < 2; ++it) {
-      const int idx = it * 256 + t;
-      const int key = (idx >> 2) & 63, part = idx & 3, is_v = idx >> 8;
-      const int kg = k0 + key;
-      const bool ok = kg < HW;
-      const __nv_bfloat16* src = base + (long)(ok ? kg : 0) * kQkv + (1 + is_v) * kHidden + head * kD + part * 8;
-      cp_async16((is_v ? sv : sk) + (buf * kKvTile + key * kKvStride + part * 8) * 2, src, ok);
-    }
-    cp_async_commit();
-  };
-  const int ntiles = (HW + kBK - 1) / kBK;
-  issue_tile(0, 0);
-  const int mi = lane >> 3, r8 = lane & 7;
-  for (int ti = 0; ti < ntiles; ++ti) {
-    const int buf = ti & 1, k0 = ti * kBK;
-    cp_async_wait<0>();
-    __syncthreads();                       // tile ti landed for everyone; everyone is done with tile ti-1
-    if (ti + 1 < ntiles) issue_tile(k0 + kBK, buf ^ 1);
-    const uint32_t kb = sk + buf * kKvTile * 2, vb = sv + buf * kKvTile * 2;
-
-    float s[8][4];
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) s[nt][i] = 0.f;
-      uint32_t kf[4];    // m0 (keys 0-7, d 0-7) m1 (d 8-15) m2 (d 16-23) m3 (d 24-31): b0,b1 of k-step 0 then 1
-      ldmatrix_x4(kf, kb + ((nt * 8 + r8) * kKvStride + mi * 8) * 2);
-      mma_bf16(s[nt], qa[0], kf[0], kf[1]);
-      mma_bf16(s[nt], qa[1], kf[2], kf[3]);
-    }
-    float mx0 = -INFINITY, mx1 = -INFINITY;
-    const bool tail = k0 + kBK > HW;
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const bool ok = !tail || (k0 + nt * 8 + 2 * tq + (i & 1)) < HW;
-        s[nt][i] = ok ? s[nt][i] * scale_log2 : -INFINITY;
-      }
-      mx0 = fmaxf(mx0, fmaxf(s[nt][0], s[nt][1]));
-      mx1 = fmaxf(mx1, fmaxf(s[nt][2], s[nt][3]));
-    }
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-    const float mn0 = fmaxf(m0, mx0), mn1 = fmaxf(m1, mx1);
-    const float c0 = (m0 == -INFINITY) ? 0.f : exp2f(m0 - mn0);
-    const float c1 = (m1 == -INFINITY) ? 0.f : exp2f(m1 - mn1);
-    m0 = mn0;
-    m1 = mn1;
-    l0 *= c0;
-    l1 *= c1;
-#pragma unroll
-    for (int dt = 0; dt < 4; ++dt) {
-      o[dt][0] *= c0; o[dt][1] *= c0; o[dt][2] *= c1; o[dt][3] *= c1;
-    }
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-      s[nt][0] = exp2f(s[nt][0] - mn0);
-      s[nt][1] = exp2f(s[nt][1] - mn0);
-      s[nt][2] = exp2f(s[nt][2] - mn1);
-      s[nt][3] = exp2f(s[nt][3] - mn1);
-      l0 += s[nt][0] + s[nt][1];
-      l1 += s[nt][2] + s[nt][3];
-    }
-#pragma unroll
-    for (int kk = 0; kk < 4; ++kk) {
-      uint32_t pa[4];
-      pa[0] = fd_pack_bf16(s[2 * kk][0], s[2 * kk][1]);
-      pa[1] = fd_pack_bf16(s[2 * kk][2], s[2 * kk][3]);
-      pa[2] = fd_pack_bf16(s[2 * kk + 1][0], s[2 * kk + 1][1]);
-      pa[3] = fd_pack_bf16(s[2 * kk + 1][2], s[2 * kk + 1][3]);
-      uint32_t v01[4], v23[4];   // (trans) m0 (keys 0-7, d 0-7) m1 (keys 8-15, d 0-7) m2 (keys 0-7, d 8-15) m3 (keys 8-15, d 8-15)
-      const uint32_t va = vb + ((kk * 16 + (mi & 1) * 8 + r8) * kKvStride + (mi >> 1) * 8) * 2;
-      ldmatrix_x4_trans(v01, va);
-      ldmatrix_x4_trans(v23, va + 16 * 2);
-      mma_bf16(o[0], pa, v01[0], v01[1]);
-      mma_bf16(o[1], pa, v01[2], v01[3]);
-      mma_bf16(o[2], pa, v23[0], v23[1]);
-      mma_bf16(o[3], pa, v23[2], v23[3]);
-    }
-  }
-  l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
-  l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-  l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-  const float i0 = 1.f / l0, i1 = 1.f / l1;
-  if (lse != nullptr && tq == 0) {      // log2-domain log-sum-exp of the scaled scores, saved for the backward pass
-    float* lp = lse + ((long)n * kHeads + head) * HW;
-    if (row0 < HW) lp[row0] = m0 + log2f(l0);
-    if (row1 < HW) lp[row1] = m1 + log2f(l1);
-  }
-  __nv_bfloat16* ob = out + (long)n * HW * kHidden + head * kD;
-#pragma unroll
-  for (int dt = 0; dt < 4; ++dt) {
-    if (row0 < HW)
-      *reinterpret_cast<uint32_t*>(ob + (long)row0 * kHidden + dt * 8 + 2 * tq) = fd_pack_bf16(o[dt][0] * i0, o[dt][1] * i0);
-    if (row1 < HW)
-      *reinterpret_cast<uint32_t*>(ob + (long)row1 * kHidden + dt * 8 + 2 * tq) = fd_pack_bf16(o[dt][2] * i1, o[dt][3] * i1);
-  }
-}
-
-template <int C>
-int launch_apply_fused(const void* x, const float* g1, const void* wq, const void* ctx_t, const void* wout,
-                              const float* bias, const float* g2, void* out, int N, int HW, float eps, cudaStream_t st) {
-  using A = ApCfg<C>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    FD_CUDA(cudaFuncSetAttribute(linattn_apply_fused_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, A::kSmem));
-    attr_set = true;
-  }
-  int bx = (HW + A::TP - 1) / A::TP;
-  const int per_sm = A::kSmem > 76 * 1024 ? 2 : 3;
-  const int cap = (FD_NUM_SMS * per_sm) / N > 0 ? (FD_NUM_SMS * per_sm) / N : 1;
-  if (bx > cap) bx = cap;
-  linattn_apply_fused_kernel<C><<<dim3(bx, N), A::NW * 32, A::kSmem, st>>>(
-      static_cast<const __nv_bfloat16*>(x), g1, static_cast<const __nv_bfloat16*>(wq),
-      static_cast<const __nv_bfloat16*>(ctx_t), static_cast<const __nv_bfloat16*>(wout), bias, g2,
-      static_cast<__nv_bfloat16*>(out), HW, eps);
-  FD_LAUNCH_CHECK();
-  return FD_OK;
 }
 
 }  // namespace
@@ -804,16 +403,6 @@ int fd_linattn_save(const void* qkv, void* out, float* stats, float* workspace, 
   return FD_OK;
 }
 
-int fd_linattn_apply_fused(const void* x, const float* g1, const void* wq, const void* ctx_t, const void* wout,
-                           const float* bias, const float* g2, void* out, int N, int HW, int C, float eps, void* stream) {
-  FD_REQUIRE(x && g1 && wq && ctx_t && wout && bias && g2 && out && N > 0 && HW > 0, "linattn_apply_fused: bad argument");
-  cudaStream_t st = (cudaStream_t)stream;
-  if (C == 64) return launch_apply_fused<64>(x, g1, wq, ctx_t, wout, bias, g2, out, N, HW, eps, st);
-  if (C == 128) return launch_apply_fused<128>(x, g1, wq, ctx_t, wout, bias, g2, out, N, HW, eps, st);
-  FD_REQUIRE(false, "linattn_apply_fused: C=%d not in {64, 128}", C);
-  return FD_EINVAL;
-}
-
 int fd_attention(const void* qkv, void* out, int N, int HW, void* stream) {
   return fd_attention_lse(qkv, out, nullptr, N, HW, stream);
 }
@@ -821,20 +410,7 @@ int fd_attention(const void* qkv, void* out, int N, int HW, void* stream) {
 int fd_attention_lse(const void* qkv, void* out, float* lse, int N, int HW, void* stream) {
   FD_REQUIRE(qkv && out && N > 0 && HW > 0, "attention: bad argument");
   FD_REQUIRE(N <= 65535, "attention: batch too large");
-  {
-    // default: the tcgen05 / TMEM / TMA kernel (fd_attention_tc.cu); FD_ATTN_TC=0 selects the mma.sync kernel below
-    static int tc = -1;
-    if (tc < 0) {
-      const char* e = getenv("FD_ATTN_TC");
-      tc = e ? atoi(e) : 1;
-    }
-    if (tc) return fd_attention_tc_launch(qkv, out, lse, N, HW, (cudaStream_t)stream);
-  }
-  const float scale_log2 = 0.17677669529663687f * 1.4426950408889634f;   // 32^-0.5 * log2(e)
-  attention_kernel<<<dim3((HW + kBQ - 1) / kBQ, kHeads, N), 256, 0, (cudaStream_t)stream>>>(
-      static_cast<const __nv_bfloat16*>(qkv), static_cast<__nv_bfloat16*>(out), lse, HW, scale_log2);
-  FD_LAUNCH_CHECK();
-  return FD_OK;
+  return fd_attention_tc_launch(qkv, out, lse, N, HW, (cudaStream_t)stream);
 }
 
 }  // extern "C"

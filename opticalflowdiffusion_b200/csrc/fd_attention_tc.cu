@@ -24,8 +24,6 @@
 //   4.26e12 MUFU ops/s = 372 us; the MUFU pipe is 53 % busy: two softmax warps per scheduler do not cover each other's TMEM-load
 //   and barrier latencies).  Tried and slower: one softmax group PER HEAD with 64-key steps (16 softmax warps; the 640-thread
 //   register allocation leaves 92 registers per thread, the score row spills: 1006 us).
-#include <stdlib.h>
-
 #include "fd_tc.cuh"
 
 using namespace fdtc;
@@ -106,7 +104,7 @@ struct AtParams {
   int N, HW, qblocks, nkv;
   __nv_bfloat16* out;      // (N, HW, 128)
   float* lse;              // [N][4][HW] log2-domain log-sum-exp of the scaled scores, or null
-  int dbg;
+  int dbg;                 // FD_ATTN_DBG in FD_DIAG builds: 2 = no PV MMAs
 };
 
 __global__ void __launch_bounds__(kAtThreads, 1) attention_tc_kernel(const __grid_constant__ CUtensorMap map_q,
@@ -150,7 +148,6 @@ __global__ void __launch_bounds__(kAtThreads, 1) attention_tc_kernel(const __gri
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *s_tmem;
-  fd_grid_dependency_wait();
 
   if (warp == 0) {
     if (elect_one_sync()) {
@@ -203,7 +200,7 @@ __global__ void __launch_bounds__(kAtThreads, 1) attention_tc_kernel(const __gri
         const uint32_t od = (uint32_t)opaque32((int)(tmem_base + 256 + h * 32));
         mbar_wait(pfull(t & 1), (t >> 1) & 1);
         tc_fence_after();
-        if (!(p.dbg & 2)) {
+        if (!(kDiag && (p.dbg & 2))) {
 #pragma unroll
           for (int ks = 0; ks < 8; ++ks) at_umma_ts(od, pa[ks], vd[ks], id_pv, (j | ks) != 0 ? 1u : 0u);
         }
@@ -355,10 +352,9 @@ int fd_attention_tc_launch(const void* qkv, void* out, float* lse, int N, int HW
     FD_CUDA(cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kAtSmemBytes));
     attr_set = true;
   }
-  static int dbg = -1;
-  if (dbg < 0) { const char* e = getenv("FD_ATTN_DBG"); dbg = e ? atoi(e) : 0; }
+  static const int dbg = fd_diag_bits("FD_ATTN_DBG");
   AtParams p{N, HW, qblocks, qblocks, static_cast<__nv_bfloat16*>(out), lse, dbg};
-  FD_CUDA(fd_launch_pdl(attention_tc_kernel, dim3(N * qblocks), dim3(kAtThreads), kAtSmemBytes, st, map_q, map_k, map_v, p));
+  attention_tc_kernel<<<N * qblocks, kAtThreads, kAtSmemBytes, st>>>(map_q, map_k, map_v, p);
   FD_LAUNCH_CHECK();
   return FD_OK;
 }

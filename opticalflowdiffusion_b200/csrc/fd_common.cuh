@@ -39,42 +39,21 @@ extern unsigned long long g_fd_launches;   // kernels launched by this library (
 
 static inline int fd_ceil_div(long a, long b) { return (int)((a + b - 1) / b); }
 
-// ---- programmatic dependent launch ---------------------------------------------------------------------------------
-// A kernel launched through fd_launch_pdl may be scheduled while its stream predecessor is still draining (its blocks start
-// as soon as SM resources free up) and runs its prologue -- barrier initialisation, TMEM allocation, tensor-map prefetch --
-// under the predecessor's tail; it MUST call fd_grid_dependency_wait() before its first access to global memory (reads of
-// the predecessor's output and writes to buffers the predecessor may still read alike).  Measured on the DDIM-50 benchmark
-// (conv, strip-conv and gn_silu kernels = 107 of the 159 launches of a forward, eager and under CUDA-graph replay): 6.753
-// flows/s with the attribute against 6.756 without -- the persistent conv CTAs fill an SM's shared memory, so there is
-// nothing for a successor to overlap with, and the launch gaps are already hidden by the graph.  Therefore OFF by default;
-// FD_PDL=1 turns the attribute on (without it the wait is a no-op and the launch an ordinary stream-ordered one).
+// ---- diagnostic builds ----------------------------------------------------------------------------------------------
+// A build with -DFD_DIAG (FD_DIAG=1 python -m opticalflowdiffusion_b200.build) compiles timing-isolation switches into the
+// conv, LinearAttention, attention and warp-window kernels: a bit mask read once from FD_CONV_DBG, FD_LA_DBG, FD_ATTN_DBG or
+// FD_WARP_WIN_DBG skips parts of the work (the results are garbage).  Every test of a mask is written `kDiag && (p.dbg & k)`,
+// so the default build contains none of them.
+#ifdef FD_DIAG
 #include <stdlib.h>
-#include <utility>
-static inline bool fd_pdl_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("FD_PDL");
-    on = (e != nullptr && atoi(e) != 0) ? 1 : 0;
-  }
-  return on != 0;
+constexpr bool kDiag = true;
+static inline int fd_diag_bits(const char* name) {
+  const char* e = getenv(name);
+  return e ? atoi(e) : 0;
 }
-template <class... KArgs, class... Args>
-static inline cudaError_t fd_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                        Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = fd_pdl_enabled() ? 1 : 0;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-#ifdef __CUDACC__
-__device__ __forceinline__ void fd_grid_dependency_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+#else
+constexpr bool kDiag = false;
+static inline int fd_diag_bits(const char*) { return 0; }
 #endif
 
 __device__ __forceinline__ float fd_warp_sum(float v) {

@@ -23,8 +23,6 @@
 //     warp 1    TMEM allocator + MMA issuer (one lane issues tcgen05.mma, tcgen05.commit frees slots)
 //     warps 2-5 epilogue: tcgen05.ld -> +bias (+residual) -> GroupNorm partial statistics
 //               (sum, sum of squares per (sample, group), :176,181) -> bf16 NHWC store
-#include <stdlib.h>
-
 #include "fd_conv_epi.cuh"
 
 using namespace fdtc;
@@ -32,11 +30,6 @@ using namespace fdtc;
 namespace {
 
 constexpr int kBlockK = 64;
-#ifdef FD_CONV_DIAG
-constexpr bool kDiag = true;    // FD_CONV_DBG switches compiled in (diagnostic builds only: they cost cycles in the issue loops)
-#else
-constexpr bool kDiag = false;
-#endif
 constexpr int kATileBytes = kBlockM * kBlockK * 2;  // 16 KiB
 constexpr int kThreads = 64 + kEpiThreads + 32;     // warp 0 TMA (A), warp 1 MMA, warps 2..9 epilogue, warp 10 TMA (B)
 
@@ -54,7 +47,7 @@ struct ConvParams {
   const __nv_bfloat16* residual;
   double* gn_stats;   // [N][8][2] or null
   int shuffle_cq;     // > 0: pixel-shuffle store, out is (N, 2H, 2W, Cout/4)
-  int dbg;            // FD_CONV_DBG (diagnostics only, results are garbage): 1 = skip A loads, 2 = skip B loads, 4 = skip MMAs,
+  int dbg;            // FD_CONV_DBG in FD_DIAG builds (results are garbage): 1 = skip A loads, 2 = skip B loads, 4 = skip MMAs,
                       // 8 = skip the epilogue's work (barrier handshakes only)
   // residual transform (fd_conv_igemm_rt): `residual` is a raw conv output whose GroupNorm + SiLU the epilogue applies
   const double* rt_stats;
@@ -140,7 +133,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_const
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *s_tmem;
-  fd_grid_dependency_wait();      // the prologue above may overlap the previous kernel's tail (fd_launch_pdl)
 
   if (warp == 0 || warp == 10) {
     // ===================== TMA producers: warp 0 loads the activation tiles, warp 10 the weight tiles ==============
@@ -442,7 +434,6 @@ conv_igemm_pair_kernel(const __grid_constant__ CUtensorMap map_a0, const __grid_
   cluster_sync_all();                                   // peers' barriers are initialised before anyone signals them
   tc_fence_after();
   const uint32_t tmem_base = *s_tmem;
-  fd_grid_dependency_wait();
 
   if (warp == 0 || warp == 10) {
     // ===================== TMA producers (both CTAs): warp 0 activation tiles, warp 10 weight half-tiles ==========
@@ -609,8 +600,7 @@ int launch_pair(const CUtensorMap& ma0, const CUtensorMap& ma1, const CUtensorMa
   const int units = p.total_tiles / MT;                  // CTA-sized work units
   int grid = units < sms ? units : sms;
   grid &= ~1;
-  FD_CUDA(fd_launch_pdl(conv_igemm_pair_kernel<BLOCK_N, GPT, MT>, dim3(grid), dim3(kThreads), C::kSmemBytes, st, ma0, ma1, mb, mo,
-                        p));
+  conv_igemm_pair_kernel<BLOCK_N, GPT, MT><<<grid, kThreads, C::kSmemBytes, st>>>(ma0, ma1, mb, mo, p);
   FD_LAUNCH_CHECK();
   return FD_OK;
 }
@@ -662,7 +652,7 @@ int launch(const CUtensorMap& ma0, const CUtensorMap& ma1, const CUtensorMap& mb
     attr_set = true;
   }
   const int grid = p.total_tiles < sms ? p.total_tiles : sms;
-  FD_CUDA(fd_launch_pdl(conv_igemm_kernel<BLOCK_N, GPT, SH>, dim3(grid), dim3(kThreads), C::kSmemBytes, st, ma0, ma1, mb, mo, p));
+  conv_igemm_kernel<BLOCK_N, GPT, SH><<<grid, kThreads, C::kSmemBytes, st>>>(ma0, ma1, mb, mo, p);
   FD_LAUNCH_CHECK();
   return FD_OK;
 }
@@ -671,8 +661,7 @@ int launch(const CUtensorMap& ma0, const CUtensorMap& ma1, const CUtensorMap& mb
 
 int fd_conv3x3_strip_launch(const void* src0, int C0, const void* src1, int C1, const void* wpacked, const float* bias,
                             const void* residual,
-                            void* out, double* gn_stats, int N, int H, int W, int base_offset_mode,
-                            cudaStream_t st);   // fd_conv_strip.cu
+                            void* out, double* gn_stats, int N, int H, int W, cudaStream_t st);   // fd_conv_strip.cu
 
 struct HeadArgs {           // fd_conv_igemm_rt_head: see EpiCtx::head_*
   float* out;
@@ -764,17 +753,11 @@ static int conv_igemm_impl(const void* src0, int C0, const void* src1, int C1, c
   FD_REQUIRE(KH >= 1 && KW >= 1 && KH * KW <= 64, "conv_igemm: bad kernel %dx%d", KH, KW);
   {
     // large-image {64,128} -> 64 3x3 layers: rolling-strip kernel (each input pixel is fetched from L2 once
-    // instead of nine times; the 64 -> 64 weights stay resident in shared memory).  FD_CONV_STRIP=0 disables it.
-    static int strip_mode = -1;
-    if (strip_mode < 0) {
-      const char* e = getenv("FD_CONV_STRIP");
-      strip_mode = e ? atoi(e) : 2;      // 2: default, 1: base_offset experiment (measured wrong), 0: off
-    }
+    // instead of nine times; the 64 -> 64 weights stay resident in shared memory)
     const bool chans_ok = (C0 == 64 && (C1 == 0 || C1 == 64)) || (C0 == 128 && C1 == 0);
-    if (strip_mode > 0 && mode == 0 && KH == 3 && KW == 3 && pad_h == 1 && pad_w == 1 && chans_ok && Cout == 64 &&
-        W >= 128 && out_mode == 0 && rt_stats == nullptr)
-      return fd_conv3x3_strip_launch(src0, C0, src1, C1, wpacked, bias, residual, out, gn_stats, N, H, W, strip_mode,
-                                     (cudaStream_t)stream);
+    if (mode == 0 && KH == 3 && KW == 3 && pad_h == 1 && pad_w == 1 && chans_ok && Cout == 64 && W >= 128 && out_mode == 0 &&
+        rt_stats == nullptr)
+      return fd_conv3x3_strip_launch(src0, C0, src1, C1, wpacked, bias, residual, out, gn_stats, N, H, W, (cudaStream_t)stream);
   }
   static int sms = 0;
   if (sms == 0) {
@@ -853,23 +836,15 @@ static int conv_igemm_impl(const void* src0, int C0, const void* src1, int C1, c
   p.total_tiles = (int)total;
   const bool stats_ = gn_stats != nullptr;
   const bool store_heavy_ = !stats_ && p.taps * (p.chunks0 + p.chunks1) <= 4;
-  static int pair_mode = -1;
-  if (pair_mode < 0) {
-    const char* e = getenv("FD_CONV_PAIR");
-    pair_mode = e == nullptr ? 2 : atoi(e);
-  }
   // CTA pairs (cta_group::2): needs an even number of M-tiles (two per pair).  Measured at batch 8, 440x1024 shapes
   // (after the elect.sync fix removed the single-thread issue overhead, which had made the leader the bottleneck):
   // N = 256 tiles +2 % (those layers already run at the power-limited practical peak, cuBLAS burst = 1.65 PF/s);
   // N = 128 tiles 0.97-0.99 PF/s vs 0.93-0.96 single (+3-4 %: each CTA stages only half of B, so the TMA fill traffic
-  // per MMA drops).  Default: pairs for both (FD_CONV_PAIR=1 pairs N = 256 only, FD_CONV_PAIR=0 disables pairing).
-  {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("FD_CONV_DBG"); dbg = e ? atoi(e) : 0; }
-    p.dbg = dbg;
-  }
-  const bool use_pair = pair_mode && (block_n == 256 || (block_n == 128 && pair_mode >= 2)) && !store_heavy_ && out_mode != 1 &&
-                        ((long)p.N * p.tiles_w * p.tiles_h) % 2 == 0 && p.total_tiles >= 2;
+  // per MMA drops).  Both widths therefore run as pairs.
+  static const int dbg = fd_diag_bits("FD_CONV_DBG");
+  p.dbg = dbg;
+  const bool use_pair = block_n >= 128 && !store_heavy_ && out_mode != 1 && ((long)p.N * p.tiles_w * p.tiles_h) % 2 == 0 &&
+                        p.total_tiles >= 2;
   {
     const uint64_t K = (uint64_t)p.taps * (C0 + C1);
     const uint64_t dims[2] = {K, (uint64_t)Cout};
@@ -914,8 +889,8 @@ static int conv_igemm_impl(const void* src0, int C0, const void* src1, int C1, c
     return p.n_tiles == 1 ? launch_pair<256, 8>(ma0, ma1, mb, mo, p, sms, st) : launch_pair<256, 4>(ma0, ma1, mb, mo, p, sms, st);
   }
   if (use_pair) {
-    // four M-tiles per pair (two per CTA) when the M-tile count allows it: FD_CONV_PAIR=3 keeps two (A/B measurements)
-    const bool mt2 = pair_mode != 3 && ((long)p.N * p.tiles_w * p.tiles_h) % 4 == 0 && p.total_tiles >= 4;
+    // four M-tiles per pair (two per CTA) when the M-tile count allows it
+    const bool mt2 = ((long)p.N * p.tiles_w * p.tiles_h) % 4 == 0 && p.total_tiles >= 4;
     if (mt2) return stats ? launch_pair<128, 8, 2>(ma0, ma1, mb, mo, p, sms, st) : launch_pair<128, 0, 2>(ma0, ma1, mb, mo, p, sms, st);
     return stats ? launch_pair<128, 8>(ma0, ma1, mb, mo, p, sms, st) : launch_pair<128, 0>(ma0, ma1, mb, mo, p, sms, st);
   }

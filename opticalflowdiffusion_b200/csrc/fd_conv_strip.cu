@@ -17,11 +17,11 @@
 // 144 KB of weights per tile instead was measured to be no faster than the generic kernel (chip-level L2->SM
 // bandwidth), while two resident-weight passes cost 0.75 ms instead of 1.09 ms.
 //
-// Two issuer variants (template parameter TS): the original one feeds both MMA operands from shared memory (SS) and is
-// shared-memory-bandwidth bound as analysed below; the default one stages the strips in tensor memory (tcgen05.cp) and issues
-// the A-from-TMEM form of tcgen05.mma, which removes three quarters of the operand reads (see the TS issuer branch).
+// The MMA issuer stages the strips in tensor memory (tcgen05.cp) and issues the A-from-TMEM ("TS") form of tcgen05.mma.  An
+// earlier issuer fed both MMA operands from shared memory ("SS"); it was shared-memory-bandwidth bound as analysed below, and
+// the TS form removes three quarters of those operand reads (see the issuer branch).
 //
-// Where the time goes in the SS variant (ncu + scripts/micro/umma_rate.cu, profiles/r1_umma_rate.txt): an SS-mode 128xNx16 UMMA reads
+// Where the time went in the SS variant (ncu + scripts/micro/umma_rate.cu, profiles/r1_umma_rate.txt): an SS-mode 128xNx16 UMMA reads
 // (128 + N) * 32 bytes of shared memory at 128 B/clk, so an N = 64 instruction takes 48 cycles, not 32.  Per 128-pixel tile
 // the 36 MMAs read 216 KB, TMA writes 16.6 KB, the epilogue writes and the TMA store reads 16 KB each: 265 KB = 2070
 // cycles of the shared-memory pipe out of the 2680 the tile takes (l1tex throughput 77 %, tensor pipe "active" 51 %).
@@ -29,19 +29,12 @@
 // one N = 192 instruction per kernel row on the unshifted strip with the kx shift done in the epilogue by warp shuffles --
 // 44 % less operand traffic, but 192 accumulator columns leave room for only two TMEM stages and the longer epilogue
 // (3 x tcgen05.ld, quarter-to-quarter row exchange) then sits on the critical path.
-#include <stdlib.h>
-
 #include "fd_conv_epi.cuh"
 
 using namespace fdtc;
 
 namespace {
 
-#ifdef FD_CONV_DIAG
-constexpr bool kDiag = true;
-#else
-constexpr bool kDiag = false;
-#endif
 constexpr int kC = 64;                         // input = output channels
 constexpr int kTileW = 128;                    // output pixels per tile (one image row segment)
 constexpr int kStripPx = kTileW + 2;           // + left/right halo
@@ -50,8 +43,8 @@ constexpr int kStripBytes = 136 * 128;         // slot size: multiple of 1024 ke
 constexpr int kNS = 5;                         // strips in flight: 3 in use + 2 prefetched (6 measured no faster)
 constexpr int kWTapBytes = kC * kC * 2;        // one tap of weights: [64 cout][64 cin] bf16
 constexpr int kWBytes = 9 * kWTapBytes;        // 72 KB, resident
-constexpr int kThreads = 64 + kEpiThreads + 64;  // warp 0 TMA, warp 1 MMA issuer, warps 2..9 epilogue; warps 10, 11: second SS issuer /
-                                                 // the input transform of the fused GroupNorm + SiLU variant
+constexpr int kThreads = 64 + kEpiThreads + 64;  // warp 0 TMA, warp 1 MMA issuer, warps 2..9 epilogue; warps 10, 11: the input
+                                                 // transform of the fused GroupNorm + SiLU variant
 constexpr int kTail = 256 + 2 * kC * 4 + kEpiWarps * 16 * 4 + 64;
 constexpr int kSmemBytes = 1024 + kWBytes + kNS * kStripBytes + 2 * kSlabBytes + kTail;
 
@@ -69,14 +62,14 @@ __device__ __forceinline__ void umma_ts_bf16(uint32_t tmem_d, uint32_t tmem_a, u
       "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-constexpr int kATmemCol0 = 2 * kC;             // TS variant: accumulators in columns [0, 128), A ring in [128, 512)
+constexpr int kATmemCol0 = 2 * kC;             // accumulators in columns [0, 128), A ring in [128, 512)
 constexpr int kATmemSlotCols = 3 * (kC / 2);   // one strip = 3 kx-shifted copies x 32 columns (64 bf16 per lane)
 constexpr int kATmemSlots = 4;                 // 3 strips in use + 1 being staged
 
 // silu(z) = z sigmoid(z) = h + h tanh(h), h = z / 2: ONE MUFU op (tanh.approx, 2^-11 relative) instead of the ex2 + rcp of
 // (Round 2: FOUR transform warps, one per scheduler / MUFU unit, with their own 14-warp template variant, made the fused launch
 // faster when timed alone -- conv roofline fraction 0.80-0.83 vs 0.77-0.79 -- and left DDIM-50 unchanged on the same box,
-// 9.53 vs 9.51 flows/s (scripts/ab_bench.py with FD_LIBFLOWDIFF): the board is power-capped, the step is energy-bound.  Not kept.)
+// 9.53 vs 9.51 flows/s (two builds alternated on one box): the board is power-capped, the step is energy-bound.  Not kept.)
 // fd_silu.  The fused input transform runs on two warps = two of the SM's four MUFU units; with two MUFU ops per element it
 // needed ~2100 cycles per strip (more than a tile's MMAs), with one ~1050.  The result differs from fd_silu by < 2^-10
 // relative before the bf16 rounding (2^-9) that follows.
@@ -91,13 +84,12 @@ struct StripParams {
   int N, H, W;
   int wblocks, total_rows;   // column blocks per image; N * wblocks * H output rows in (image, column block, row) order
   int tile_w;                // output pixels per tile
-  int base_offset_mode;      // 2 (default): base_offset 0 -- correct; 1: (addr >> 7) & 7 -- measured WRONG, kept as an experiment
   int c_off;                 // first input channel of this pass inside the source tensor (0 or 64)
   int w_k0, w_kstride;       // weight K coordinate of tap t = t * w_kstride + w_k0
   const float* bias;
   const __nv_bfloat16* residual;
   double* gn_stats;
-  // fused input transform (TS variant only): the strips are activated in shared memory, x -> silu(a[c] x + b[c]) with the
+  // fused input transform: the strips are activated in shared memory, x -> silu(a[c] x + b[c]) with the
   // GroupNorm statistics of the INPUT tensor folded into a, b exactly as gn_silu_kernel does (Block.forward :176-187)
   const double* in_stats;    // [N][8][2] or null (no transform)
   const float* in_gamma;
@@ -105,8 +97,7 @@ struct StripParams {
   const float* in_ss;        // (scale | shift) rows or null
   long in_ss_stride;
   float in_eps;
-  int pf;                    // L2 prefetch distance in rows (0 = off)
-  int dbg;                   // FD_CONV_DBG in FD_CONV_DIAG builds: 4 = no MMAs, 8 = epilogue handshakes only, 64 = no tcgen05.cp
+  int dbg;                   // FD_CONV_DBG in FD_DIAG builds: 4 = no MMAs, 8 = epilogue handshakes only, 64 = no tcgen05.cp
 };
 
 // Work split: the N * wblocks * H output rows (128-pixel tiles), ordered (image, column block, row), are cut into gridDim.x
@@ -270,7 +261,7 @@ __device__ __forceinline__ void strip_epilogue2(const EpiCtx& ec, NextTile next_
   if ((ew & 3) == 0 && elect_one_sync()) tma_store_wait_all();
 }
 
-template <int GPT, bool TS>
+template <int GPT>
 __global__ void __launch_bounds__(kThreads, 1)
 conv3x3_strip_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_constant__ CUtensorMap map_w,
                      const __grid_constant__ CUtensorMap map_out, const StripParams p) {
@@ -287,7 +278,7 @@ conv3x3_strip_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_co
   auto tfull_bar = [&](int s) { return bar_base + 8u * (1 + 2 * kNS + s); };
   auto tempty_bar = [&](int s) { return bar_base + 8u * (3 + 2 * kNS + s); };
   auto xfull_bar = [&](int s) { return bar_base + 8u * (5 + 2 * kNS + s); };   // strip transformed (fused GroupNorm input)
-  const bool fuse_in = TS && p.in_stats != nullptr;
+  const bool fuse_in = p.in_stats != nullptr;
   uint8_t* gtail = gbase + kWBytes + kNS * kStripBytes + 2 * kSlabBytes + 256;
   float* s_bias = reinterpret_cast<float*>(gtail);
   float* s_stats = reinterpret_cast<float*>(gtail + 2 * kC * 4);
@@ -310,13 +301,12 @@ conv3x3_strip_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_co
     }
     fence_barrier_init();
   }
-  constexpr uint32_t kTmemCols = TS ? 512 : 2 * kC;
+  constexpr uint32_t kTmemCols = 512;
   if (warp == 1) tmem_alloc(smem_u32(s_tmem), kTmemCols);
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *s_tmem;
-  fd_grid_dependency_wait();      // the prologue above may overlap the previous kernel's tail (fd_launch_pdl)
 
   if (warp == 0) {
     // ===================== TMA producer: weights once, then one strip per input row =====================
@@ -328,21 +318,16 @@ conv3x3_strip_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_co
       StripWalk walk(p);
       int n, w0, ra, rb;
       while (walk.next(p, n, w0, ra, rb)) {
-        // The ring holds ~4 strips of lookahead = ~3 us of work, about the DRAM latency under load: rows are prefetched
-        // into L2 kPF rows ahead of their load so the loads themselves only see L2 latency.
-        if (p.pf > 0)
-          for (int y = ra - 1; y < ra - 1 + p.pf && y <= rb; ++y) tma_prefetch_l2_5d(&map_in, p.c_off, w0 - 1, y, n, 0);
         for (int y = ra - 1; y <= rb; ++y, ++seq) {
           const int slot = seq % kNS;
           const uint32_t phase = (seq / kNS) & 1u;
-          if (p.pf > 0 && y + p.pf <= rb) tma_prefetch_l2_5d(&map_in, p.c_off, w0 - 1, y + p.pf, n, 0);
           mbar_wait(empty_bar(slot), phase ^ 1u);
           mbar_expect_tx(full_bar(slot), kStripTx);
           tma_load_5d(s_smem + slot * kStripBytes, &map_in, full_bar(slot), p.c_off, w0 - 1, y, n, 0);
         }
       }
     }
-  } else if (TS && warp == 1) {
+  } else if (warp == 1) {
     // ===================== MMA issuer, A operand from tensor memory =====================
     // The SS form reads (128 + 64) * 32 B of shared memory per 128x64x16 instruction = 48 cycles at 128 B/clk, and the nine
     // taps re-read every strip nine times: 216 KB per tile, which made this kernel shared-memory bound (file header).  Here
@@ -517,7 +502,7 @@ conv3x3_strip_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_co
       }
     }
     __syncwarp();
-  } else if (TS && (warp == 10 || warp == 11)) {
+  } else if (warp == 10 || warp == 11) {
     // ===================== fused input transform: GroupNorm affine + SiLU on the landed strip, in place =====================
     // Replaces the separate gn_silu pass over the producer's output (one read + one write of the tensor) for the convs whose
     // input is only consumed here (ResnetBlock block1 -> block2, :202-214).  64 threads: thread = (8-channel granule q, row
@@ -597,58 +582,6 @@ conv3x3_strip_kernel(const __grid_constant__ CUtensorMap map_in, const __grid_co
         }
       }
     }
-  } else if (!TS && (warp == 1 || warp == 10)) {
-    // ===================== MMA issuers =====================
-    // A 128x64x16 UMMA occupies the tensor core for only 32 cycles, less than one thread needs to issue the next
-    // one (descriptor -> uniform-register traffic), so ONE issuer leaves the pipe ~60 % idle (ncu: 40 % active).
-    // Two issuer warps alternate tiles; tile parity == TMEM accumulator stage, so they never share an accumulator.
-    constexpr uint32_t idesc = umma_idesc_bf16(kBlockM, kC);
-    const int my_parity = warp == 1 ? 0 : 1;
-    mbar_wait(wfull_bar, 0);
-    uint32_t seq0 = 0;       // sequence number of the first strip (input row ra-1) of the current item
-    int iter = 0;
-    StripWalk walk(p);
-    int n, w0, ra, rb;
-    while (walk.next(p, n, w0, ra, rb)) {
-      const int rows = rb - ra;
-      for (int j = 0; j < rows; ++j, ++iter) {
-        const int as = iter & 1;
-        if (as != my_parity) continue;
-        const uint32_t aphase = (iter >> 1) & 1;
-        mbar_wait(tempty_bar(as), aphase ^ 1u);
-#pragma unroll
-        for (int ky = 0; ky < 3; ++ky) {
-          const uint32_t s = seq0 + j + ky;
-          mbar_wait(full_bar(s % kNS), (s / kNS) & 1u);
-        }
-        tc_fence_after();
-        if (elect_one_sync()) {
-          const uint32_t tmem_d = tmem_base + as * kC;
-#pragma unroll
-          for (int ky = 0; ky < 3; ++ky) {
-            const uint32_t strip = s_smem + ((seq0 + j + ky) % kNS) * kStripBytes;
-#pragma unroll
-            for (int kx = 0; kx < 3; ++kx) {
-              // output pixel i of the tile reads strip pixel i + kx: same strip, start shifted by kx rows of 128 B
-              const uint64_t adesc = p.base_offset_mode == 1 ? umma_desc_sw128_base_offset(strip + kx * 128)
-                                                             : umma_desc_sw128(strip + kx * 128);
-              const uint64_t bdesc = umma_desc_sw128(w_smem + (ky * 3 + kx) * kWTapBytes);
-#pragma unroll
-              for (int k = 0; k < kC / 16; ++k)
-                umma_bf16(tmem_d, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (ky | kx | k) != 0 ? 1u : 0u);
-            }
-          }
-          umma_commit(tfull_bar(as));
-          umma_commit(empty_bar((seq0 + j) % kNS));                 // input row ra-1+j is no longer needed
-          if (j == rows - 1) {
-            umma_commit(empty_bar((seq0 + j + 1) % kNS));
-            umma_commit(empty_bar((seq0 + j + 2) % kNS));
-          }
-        }
-        __syncwarp();
-      }
-      seq0 += rows + 2;
-    }
   } else if (warp >= 2 && warp < 2 + kEpiWarps) {
     // ===================== epilogue =====================
     EpiCtx ec;
@@ -706,12 +639,12 @@ struct StripInputNorm {           // fused GroupNorm + SiLU on the input (null s
 };
 
 static int strip_launch(const void* src0, int C0, const void* src1, int C1, const void* wpacked, const float* bias,
-                        const void* residual, void* out, double* gn_stats, int N, int H, int W, int base_offset_mode,
-                        const StripInputNorm& in, cudaStream_t st);
+                        const void* residual, void* out, double* gn_stats, int N, int H, int W, const StripInputNorm& in,
+                        cudaStream_t st);
 
 int fd_conv3x3_strip_launch(const void* src0, int C0, const void* src1, int C1, const void* wpacked, const float* bias,
-                            const void* residual, void* out, double* gn_stats, int N, int H, int W, int base_offset_mode, cudaStream_t st) {
-  return strip_launch(src0, C0, src1, C1, wpacked, bias, residual, out, gn_stats, N, H, W, base_offset_mode, StripInputNorm{}, st);
+                            const void* residual, void* out, double* gn_stats, int N, int H, int W, cudaStream_t st) {
+  return strip_launch(src0, C0, src1, C1, wpacked, bias, residual, out, gn_stats, N, H, W, StripInputNorm{}, st);
 }
 
 extern "C" int fd_conv3x3_gnsilu_in(const void* src, const double* in_stats, const float* in_gamma, const float* in_beta,
@@ -721,12 +654,12 @@ extern "C" int fd_conv3x3_gnsilu_in(const void* src, const double* in_stats, con
   FD_REQUIRE(src && in_stats && in_gamma && in_beta && wpacked && out && N > 0 && H > 0 && W >= 64,
              "conv3x3_gnsilu_in: bad argument (needs 64 -> 64 channels, W >= 64)");
   StripInputNorm in{in_stats, in_gamma, in_beta, in_scale_shift, in_ss_stride, in_eps};
-  return strip_launch(src, 64, nullptr, 0, wpacked, bias, residual, out, gn_stats, N, H, W, 2, in, (cudaStream_t)stream);
+  return strip_launch(src, 64, nullptr, 0, wpacked, bias, residual, out, gn_stats, N, H, W, in, (cudaStream_t)stream);
 }
 
 static int strip_launch(const void* src0, int C0, const void* src1, int C1, const void* wpacked, const float* bias,
-                        const void* residual, void* out, double* gn_stats, int N, int H, int W, int base_offset_mode,
-                        const StripInputNorm& in, cudaStream_t st) {
+                        const void* residual, void* out, double* gn_stats, int N, int H, int W, const StripInputNorm& in,
+                        cudaStream_t st) {
   static int sms = 0;
   if (sms == 0) {
     int dev = 0;
@@ -740,7 +673,6 @@ static int strip_launch(const void* src0, int C0, const void* src1, int C1, cons
   p.tile_w = kTileW;
   p.wblocks = (W + p.tile_w - 1) / p.tile_w;
   p.total_rows = N * p.wblocks * H;
-  p.base_offset_mode = base_offset_mode;
   p.w_kstride = cin;
   CUtensorMap mw, mo;
   {
@@ -757,32 +689,23 @@ static int strip_launch(const void* src0, int C0, const void* src1, int C1, cons
   const int grid = p.total_rows < sms ? p.total_rows : sms;
   static bool attr_set = false;
   if (!attr_set) {
-    FD_CUDA(cudaFuncSetAttribute(conv3x3_strip_kernel<8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    FD_CUDA(cudaFuncSetAttribute(conv3x3_strip_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    FD_CUDA(cudaFuncSetAttribute(conv3x3_strip_kernel<8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-    FD_CUDA(cudaFuncSetAttribute(conv3x3_strip_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    FD_CUDA(cudaFuncSetAttribute(conv3x3_strip_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    FD_CUDA(cudaFuncSetAttribute(conv3x3_strip_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
     attr_set = true;
   }
-  // Default: A operand from tensor memory (see the TS issuer).  Measured at 8x440x1024: 64->64 0.214 ms against 0.226 for the
-  // shared-memory-operand (SS) variant, 128->64 0.510 against 0.535; the outputs are bit-identical.  With the operand reads gone
-  // the layer is held by the single issuing thread (it runs only 2-3 MMAs ahead of the pipe) and by its HBM traffic (922 MB =
-  // 0.141 ms at the copy peak, 0.175 ms measured with MMAs and copies disabled).  FD_STRIP_TS=0 selects the SS variant (read
-  // per call so that tests can exercise both).
-  const char* ets = getenv("FD_STRIP_TS");
-  const bool ts = in.stats != nullptr || ((ets == nullptr || atoi(ets) != 0) && base_offset_mode != 1);   // the fused input transform lives in the TS issuer
+  // A operand from tensor memory.  Measured at 8x440x1024: 64->64 0.214 ms against 0.226 for the former shared-memory-operand
+  // (SS) issuer, 128->64 0.510 against 0.535; the outputs were bit-identical.  With the operand reads gone the layer is held by
+  // the single issuing thread (it runs only 2-3 MMAs ahead of the pipe) and by its HBM traffic (922 MB = 0.141 ms at the copy
+  // peak, 0.175 ms measured with MMAs and copies disabled).  An L2 prefetch of the input rows ahead of their TMA loads was
+  // measured no faster (0.229 -> 0.231 ms).
   p.in_stats = in.stats;
   p.in_gamma = in.gamma;
   p.in_beta = in.beta;
   p.in_ss = in.scale_shift;
   p.in_ss_stride = in.ss_stride;
   p.in_eps = in.eps;
-  {
-    const char* e = getenv("FD_STRIP_PF");           // L2 prefetch distance in rows; measured no gain (0.229 -> 0.231 ms), off
-    p.pf = e ? atoi(e) : 0;
-    static int dbg = -1;
-    if (dbg < 0) { const char* d = getenv("FD_CONV_DBG"); dbg = d ? atoi(d) : 0; }
-    p.dbg = dbg;
-  }
+  static const int dbg = fd_diag_bits("FD_CONV_DBG");
+  p.dbg = dbg;
   for (int pass = 0; pass < passes; ++pass) {
     const bool last = pass == passes - 1;
     const bool from1 = pass == 1 && C1 > 0;                 // second half comes from the second tensor
@@ -799,13 +722,8 @@ static int strip_launch(const void* src0, int C0, const void* src1, int C1, cons
     // pass 0 adds the caller's residual (if any), pass 1 the partial sum of pass 0
     p.residual = static_cast<const __nv_bfloat16*>(pass > 0 ? out : residual);
     p.gn_stats = last ? gn_stats : nullptr;
-    if (p.gn_stats != nullptr) {
-      if (ts) FD_CUDA(fd_launch_pdl(conv3x3_strip_kernel<8, true>, dim3(grid), dim3(kThreads), kSmemBytes, st, mi, mw, mo, p));
-      else FD_CUDA(fd_launch_pdl(conv3x3_strip_kernel<8, false>, dim3(grid), dim3(kThreads), kSmemBytes, st, mi, mw, mo, p));
-    } else {
-      if (ts) FD_CUDA(fd_launch_pdl(conv3x3_strip_kernel<0, true>, dim3(grid), dim3(kThreads), kSmemBytes, st, mi, mw, mo, p));
-      else FD_CUDA(fd_launch_pdl(conv3x3_strip_kernel<0, false>, dim3(grid), dim3(kThreads), kSmemBytes, st, mi, mw, mo, p));
-    }
+    if (p.gn_stats != nullptr) conv3x3_strip_kernel<8><<<grid, kThreads, kSmemBytes, st>>>(mi, mw, mo, p);
+    else conv3x3_strip_kernel<0><<<grid, kThreads, kSmemBytes, st>>>(mi, mw, mo, p);
     FD_LAUNCH_CHECK();
   }
   return FD_OK;

@@ -20,8 +20,6 @@
 //   in TMEM for the whole range, then the 128 x BN block is added into dW with coalesced fp32 atomics (lanes =
 //   consecutive ci).  Jobs that share a pixel range are adjacent in blockIdx so they run together and the
 //   activation tiles are served by L2.
-#include <stdlib.h>
-
 #include "fd_tc.cuh"
 
 using namespace fdtc;
@@ -264,12 +262,7 @@ int fd_conv_wgrad(const void* src0, int C0, const void* src1, int C1, const void
   if (mode == 0 && KH == 3 && KW == 3 && pad_h == 1 && pad_w == 1 && W >= 64 && Cout <= 128) {
     // rolling-strip kernel: every source / dy row is loaded once instead of once per tap (measured: 800-880 TFLOP/s vs
     // 140-410 for Cout <= 128; the N = 256 tiles of the generic kernel stay ahead for Cout >= 256: 700-800 vs 630-650)
-    static int use_strip = -1;
-    if (use_strip < 0) {
-      const char* e = getenv("FD_WGRAD_STRIP");
-      use_strip = (e == nullptr || atoi(e) != 0) ? 1 : 0;
-    }
-    if (use_strip) return fd_conv_wgrad_strip_launch(src0, C0, src1, C1, dy, dw, N, H, W, Cout, stream);
+    return fd_conv_wgrad_strip_launch(src0, C0, src1, C1, dy, dw, N, H, W, Cout, stream);
   }
   WgradParams p{};
   p.Cout = Cout;

@@ -26,8 +26,6 @@
 // Warp roles in both passes (576 threads, one CTA per SM, contiguous tile ranges inside one sample):
 //   warp 0 TMA producer, warp 1 TMEM allocator + single-thread tcgen05.mma issuer, warps 2..17 epilogue (TMEM lane quarter =
 //   warp % 4; the four warps of a quarter split the columns, 32 each).
-#include <stdlib.h>
-
 #include "fd_tc.cuh"
 
 using namespace fdtc;
@@ -222,7 +220,7 @@ struct CtxParams {
   const float* sk;
   const float* mk;
   float* partial;             // [N * cps][128 d][C + 4]: G[d][0..C), T[d], den[d]
-  int dbg;                    // FD_LA_DBG (diagnostics, results are garbage): 1 skip epilogue math, 2 skip MMA2 + aux, 4 skip row
+  int dbg;                    // FD_LA_DBG & 15 in FD_DIAG builds (results are garbage): 1 skip epilogue math, 2 skip MMA2 + aux, 4 skip row
                               // statistics, 8 skip MMA1
 };
 
@@ -280,7 +278,6 @@ linattn_ctx_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
   tc_fence_after();
   const uint32_t tmem_base = *s_tmem;
   // TMEM columns: D1 (k logits) 2 x 128 at 0 / 128, D2 (G) C columns at 256, D3 (T, den) 16 columns at 384
-  fd_grid_dependency_wait();
 
   if (warp == 0) {
     if (elect_one_sync()) {
@@ -307,7 +304,7 @@ linattn_ctx_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
         mbar_wait(xfull(s), (i / S) & 1);
         tc_fence_after();
         const uint64_t xd = umma_desc_sw128(x_smem + s * Cf::kXBytes);
-        if (!(p.dbg & 8)) {
+        if (!(kDiag && (p.dbg & 8))) {
 #pragma unroll
           for (int ch = 0; ch < NCH; ++ch)
 #pragma unroll
@@ -326,7 +323,7 @@ linattn_ctx_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
         const uint64_t pd = la_desc_mn(p_smem + pb * Cf::kPBytes, 16384);
         const uint64_t xd = la_desc_mn(x_smem + s * Cf::kXBytes, 16384);
         const uint64_t ad = umma_desc_sw128(aux_smem + pb * Cf::kAuxBytes);
-        if (!(p.dbg & 2)) {
+        if (!(kDiag && (p.dbg & 2))) {
 #pragma unroll
           for (int ks = 0; ks < 8; ++ks)       // 16 pixels per step = two 8-pixel atoms = 2048 B
             umma_bf16(tmem_base + 256, pd + (uint64_t)(ks * 128), xd + (uint64_t)(ks * 128), id2, (i | ks) != 0 ? 1u : 0u);
@@ -362,7 +359,7 @@ linattn_ctx_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
       const int s = i % S, u = i >> 1, pb = i % NP;
       mbar_wait(xfull(s), (i / S) & 1);
       float mu = 0.f, r = 1.f, sigma = 1.f;
-      if (!(p.dbg & 4))
+      if (!(kDiag && (p.dbg & 4)))
         la_row_stats2<C>(x_smem + s * Cf::kXBytes, row, half, 4 + grp * 4 + quarter, s_sx + (u & 1) * 256, p.eps, mu, r, sigma);
       const bool valid = (t0 + i) * kTilePx + row < p.HW;
       const uint64_t nrm2 = pk2(-r * mu, -r * mu), r2 = pk2(r, r);
@@ -380,7 +377,7 @@ linattn_ctx_kernel(const __grid_constant__ CUtensorMap map_x, const __grid_const
           tc_fence_before();
           mbar_arrive(d1empty(as));
         }
-        if (p.dbg & 1) continue;
+        if (kDiag && (p.dbg & 1)) continue;
         uint32_t pk[16];
 #pragma unroll
         for (int j4 = 0; j4 < 8; ++j4) {
@@ -563,7 +560,7 @@ struct ApParams {
   const float* sq;
   const float* bout;
   const float* g2;
-  int dbg;
+  int dbg;                    // FD_LA_DBG >> 4 in FD_DIAG builds (results are garbage)
 };
 
 template <int C>
@@ -629,7 +626,6 @@ linattn_apply_kernel_tc(const __grid_constant__ CUtensorMap map_x, const __grid_
   tc_fence_after();
   const uint32_t tmem_base = *s_tmem;
   // TMEM columns: D1 (q logits) 2 x 128 at 0 / 128, D2 (q_hat M) 2 x C at 256 / 384
-  fd_grid_dependency_wait();
 
   if (warp == 0) {
     if (elect_one_sync()) {
@@ -656,7 +652,7 @@ linattn_apply_kernel_tc(const __grid_constant__ CUtensorMap map_x, const __grid_
         mbar_wait(xfull(s), (i / S) & 1);
         tc_fence_after();
         const uint64_t xd = umma_desc_sw128(x_smem + s * Cf::kXBytes);
-        if (!(p.dbg & 8)) {
+        if (!(kDiag && (p.dbg & 8))) {
 #pragma unroll
           for (int ch = 0; ch < NCH; ++ch)
 #pragma unroll
@@ -674,7 +670,7 @@ linattn_apply_kernel_tc(const __grid_constant__ CUtensorMap map_x, const __grid_
         mbar_wait(d2empty(as), ((i >> 1) & 1) ^ 1u);
         tc_fence_after();
         const uint64_t qd = umma_desc_sw128(q_smem + qb * Cf::kQBytes);
-        if (!(p.dbg & 2)) {
+        if (!(kDiag && (p.dbg & 2))) {
 #pragma unroll
           for (int ks = 0; ks < 8; ++ks)       // K = 128 d: two 64-d chunks x four 16-element steps
             umma_bf16(tmem_base + 256 + as * 128, qd + (uint64_t)((ks >> 2) * 1024 + 2 * (ks & 3)),
@@ -718,7 +714,7 @@ linattn_apply_kernel_tc(const __grid_constant__ CUtensorMap map_x, const __grid_
         tmem_ld_wait();
         tc_fence_before();
         mbar_arrive(d1empty(as));
-        if (p.dbg & 1) {
+        if (kDiag && (p.dbg & 1)) {
           fence_proxy_async_smem();
           mbar_arrive(qfull(qb));
           continue;
@@ -782,7 +778,7 @@ linattn_apply_kernel_tc(const __grid_constant__ CUtensorMap map_x, const __grid_
         const int sj = j % S;
         mbar_wait(xfull(sj), (j / S) & 1);
         float mu = 0.f, r = 1.f, sigma = 1.f;
-        if (!(p.dbg & 4)) la_row_stats2<C>(x_smem + sj * Cf::kXBytes, row, half, 8 + quarter, s_sx + (j & 1) * 256, p.eps, mu, r, sigma);
+        if (!(kDiag && (p.dbg & 4))) la_row_stats2<C>(x_smem + sj * Cf::kXBytes, row, half, 8 + quarter, s_sx + (j & 1) * 256, p.eps, mu, r, sigma);
         if (half == 0) s_rs[(j & 1) * 128 + row] = make_float2(mu, r);
         mbar_arrive(sfull(j & 1));
       };
@@ -811,7 +807,7 @@ linattn_apply_kernel_tc(const __grid_constant__ CUtensorMap map_x, const __grid_
         mbar_arrive(d2empty(as));
         const uint32_t ob = slab_count % NO;
         ++slab_count;
-        if (p.dbg & 16) {
+        if (kDiag && (p.dbg & 16)) {
           mbar_arrive(xempty(s));
           continue;
         }
@@ -852,7 +848,7 @@ linattn_apply_kernel_tc(const __grid_constant__ CUtensorMap map_x, const __grid_
         fence_proxy_async_smem();
         mbar_arrive(xempty(s));              // this group's reads of the x tile (the residual) are done
         named_bar_sync(3, kLaEpi / 2);
-        if (gw == 0 && elect_one_sync() && !(p.dbg & 32)) {
+        if (gw == 0 && elect_one_sync() && !(kDiag && (p.dbg & 32))) {
           for (int ch = 0; ch < NCH; ++ch)
             la_tma_store_3d(&map_out, o_smem + ob * Cf::kOBytes + ch * 16384, ch * 64, (t0 + i) * kTilePx, n);
           tma_store_commit();
@@ -912,16 +908,14 @@ int run_tc(const void* x, const void* wk, const float* sk, const float* mk, cons
     FD_CUDA(cudaFuncSetAttribute(linattn_apply_kernel_tc<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, ApTcCfg<C>::kSmemBytes));
     attr_set = true;
   }
-  static int la_dbg = -1;
-  if (la_dbg < 0) { const char* e = getenv("FD_LA_DBG"); la_dbg = e ? atoi(e) : 0; }
+  static const int la_dbg = fd_diag_bits("FD_LA_DBG");
   CtxParams cp{N, HW, cps, tiles, eps, sk, mk, partial, la_dbg & 15};
-  FD_CUDA(fd_launch_pdl(linattn_ctx_kernel<C>, dim3(N * cps), dim3(kLaThreads), CtxCfg<C>::kSmemBytes, st, map_x, map_wk, cp));
+  linattn_ctx_kernel<C><<<N * cps, kLaThreads, CtxCfg<C>::kSmemBytes, st>>>(map_x, map_wk, cp);
   FD_LAUNCH_CHECK();
   linattn_tc_combine_kernel<C><<<dim3(N, 4), 256, 0, st>>>(partial, wv, wout, mt, cps, HW);
   FD_LAUNCH_CHECK();
   ApParams ap{N, HW, cps, tiles, eps, sq, bout, g2, la_dbg >> 4};
-  FD_CUDA(fd_launch_pdl(linattn_apply_kernel_tc<C>, dim3(N * cps), dim3(kLaThreads), ApTcCfg<C>::kSmemBytes, st, map_x, map_wq, map_m,
-                        map_out, ap));
+  linattn_apply_kernel_tc<C><<<N * cps, kLaThreads, ApTcCfg<C>::kSmemBytes, st>>>(map_x, map_wq, map_m, map_out, ap);
   FD_LAUNCH_CHECK();
   return FD_OK;
 }

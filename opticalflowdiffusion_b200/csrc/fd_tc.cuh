@@ -103,13 +103,6 @@ __device__ __forceinline__ void tma_load_5d(uint32_t dst, const CUtensorMap* m, 
       : "memory");
 }
 
-// global -> L2 only (no shared-memory destination, no completion to wait for): hides the DRAM latency of a later load
-__device__ __forceinline__ void tma_prefetch_l2_5d(const CUtensorMap* m, int c0, int c1, int c2, int c3, int c4) {
-  asm volatile("cp.async.bulk.prefetch.tensor.5d.L2.global.tile [%0, {%1, %2, %3, %4, %5}];" ::"l"(m), "r"(c0), "r"(c1), "r"(c2),
-               "r"(c3), "r"(c4)
-               : "memory");
-}
-
 // smem -> global tensor store (clips to the tensor bounds); bulk-group completion
 __device__ __forceinline__ void tma_store_5d(const CUtensorMap* m, uint32_t src, int c0, int c1, int c2, int c3, int c4) {
   asm volatile("cp.async.bulk.tensor.5d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5, %6}], [%1];" ::"l"(m), "r"(src),
@@ -168,7 +161,7 @@ __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.
 
 // K-major operand tile, rows of 64 bf16 (128 B) written by TMA with 128-byte swizzle:
 // 8-row groups are 1024 B apart (SBO), LBO unused, descriptor version 1 (sm_100), layout SWIZZLE_128B.
-// MEASURED on B200 (tests/test_gpu_conv.py with FD_CONV_STRIP=1 vs 2): the tensor core applies the 128B swizzle
+// MEASURED on B200 (the strip conv's shifted-start descriptors): the tensor core applies the 128B swizzle
 // XOR to the ABSOLUTE shared-memory address bits [7:9], exactly like TMA does when writing, so a descriptor may
 // start at any 128-byte row of a 1024-byte-aligned TMA tile (rows shifted by 1 or 2 pixels for the conv taps)
 // with base_offset = 0; setting base_offset = (addr >> 7) & 7 for such starts gives WRONG results.
@@ -178,9 +171,6 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t saddr) {
   d |= 1ull << 46;
   d |= 2ull << 61;
   return d;
-}
-__device__ __forceinline__ uint64_t umma_desc_sw128_base_offset(uint32_t saddr) {   // kept for the experiment above
-  return umma_desc_sw128(saddr) | ((uint64_t)((saddr >> 7) & 7u) << 49);
 }
 // instruction descriptor: D fp32, A/B bf16, both K-major, M x N
 __host__ __device__ constexpr uint32_t umma_idesc_bf16(int M, int N) {

@@ -263,7 +263,6 @@ __global__ void __launch_bounds__(256) gn_silu_kernel(const __nv_bfloat16* __res
                                                       const float* __restrict__ scale_shift, long ss_stride,
                                                       const __nv_bfloat16* __restrict__ residual,
                                                       __nv_bfloat16* __restrict__ out, long HW, int C, float eps) {
-  fd_grid_dependency_wait();               // launched with fd_launch_pdl: everything below touches global memory
   const int n = blockIdx.y;
   const int chunks = C >> 3;
   const int chunk = threadIdx.x % chunks;
@@ -679,14 +678,10 @@ static int gn_silu_launch(bool tanh_form, const void* x, const double* gn_stats,
   const long cap = (long)FD_NUM_SMS * 16 / N + 1;
   if (bx > cap) bx = cap;
   dim3 grid((unsigned)bx, (unsigned)N);
-  if (tanh_form)
-    FD_CUDA(fd_launch_pdl(gn_silu_kernel<true>, grid, dim3(ppb * chunks), 0, (cudaStream_t)stream,
-                          static_cast<const __nv_bfloat16*>(x), gn_stats, gamma, beta, scale_shift, ss_stride,
-                          static_cast<const __nv_bfloat16*>(residual), static_cast<__nv_bfloat16*>(out), (long)HW, C, eps));
-  else
-    FD_CUDA(fd_launch_pdl(gn_silu_kernel<false>, grid, dim3(ppb * chunks), 0, (cudaStream_t)stream,
-                          static_cast<const __nv_bfloat16*>(x), gn_stats, gamma, beta, scale_shift, ss_stride,
-                          static_cast<const __nv_bfloat16*>(residual), static_cast<__nv_bfloat16*>(out), (long)HW, C, eps));
+  auto kernel = tanh_form ? gn_silu_kernel<true> : gn_silu_kernel<false>;
+  kernel<<<grid, ppb * chunks, 0, (cudaStream_t)stream>>>(static_cast<const __nv_bfloat16*>(x), gn_stats, gamma, beta, scale_shift,
+                                                          ss_stride, static_cast<const __nv_bfloat16*>(residual),
+                                                          static_cast<__nv_bfloat16*>(out), (long)HW, C, eps);
   FD_LAUNCH_CHECK();
   return FD_OK;
 }

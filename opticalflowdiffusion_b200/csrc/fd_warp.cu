@@ -4,7 +4,7 @@
 // Gather/scatter work on fp32 NCHW planes.  The FORWARD operations on three-channel frames with W % 4 == 0 run the
 // shared-memory window kernels of fd_warp_win.cu (TMA-staged frame, 1.5-2x faster on the config-#4 white-noise flow);
 // the kernels in this file serve every other shape and all the backward passes.  Layout choices:
-//   * one thread owns VEC (1, 2 or 4 when W allows; 2 by default) consecutive pixels of a row, so flow / flow_gt /
+//   * one thread owns VEC (2 when W is even, else 1) consecutive pixels of a row, so flow / flow_gt /
 //     frame1 / out / mask move as wide coalesced accesses; a block walks (row, segment) jobs, no per-thread divisions;
 //   * the 4-tap gathers of the warped frame go through the read-only path (L1/L2 resident: a
 //     warp's taps fall in a few rows of the source plane);
@@ -14,8 +14,6 @@
 // The coordinate / weight / accumulation sequence is written with explicit round-to-nearest
 // intrinsics in the exact order ATen's CPU grid_sampler_2d evaluates it, which makes the forward
 // bit-identical to the reference's CPU output (oracle/flowdiff_oracle.py:backwarp).
-#include <stdlib.h>
-
 #include <initializer_list>
 
 #include "fd_warp_common.cuh"
@@ -40,17 +38,6 @@ struct Vec<2> {
     v[0] = t.x; v[1] = t.y;
   }
   __device__ __forceinline__ void store(float* p) const { *reinterpret_cast<float2*>(p) = make_float2(v[0], v[1]); }
-};
-template <>
-struct Vec<4> {
-  float v[4];
-  __device__ __forceinline__ void load(const float* p) {
-    const float4 t = __ldg(reinterpret_cast<const float4*>(p));
-    v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
-  }
-  __device__ __forceinline__ void store(float* p) const {
-    *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
-  }
 };
 
 // Work decomposition without per-thread divisions.  A "row job" = (image row r = b * H + y, segment of blockDim.x * VEC
@@ -80,7 +67,7 @@ static unsigned row_segs(int W, int vec, int threads) { return (unsigned)((W / v
 // forward: out, mask
 // ---------------------------------------------------------------------------------------------
 template <int VEC, int CT>
-__global__ void __launch_bounds__(256, VEC == 4 ? 2 : 4) backwarp_fwd_kernel(const float* __restrict__ image,
+__global__ void __launch_bounds__(256, 4) backwarp_fwd_kernel(const float* __restrict__ image,
                                                            const float* __restrict__ flow,
                                                            float* __restrict__ out, float* __restrict__ mask,
                                                            int B, int C, BwGeom g, unsigned segs, unsigned jobs) {
@@ -119,7 +106,7 @@ __global__ void __launch_bounds__(256, VEC == 4 ? 2 : 4) backwarp_fwd_kernel(con
 // backward of sum(out * gout): gimage (scatter), gflow (gather)
 // ---------------------------------------------------------------------------------------------
 template <int VEC, int CT>
-__global__ void __launch_bounds__(256, VEC == 4 ? 1 : 3) backwarp_bwd_kernel(const float* __restrict__ image,
+__global__ void __launch_bounds__(256, 3) backwarp_bwd_kernel(const float* __restrict__ image,
                                                            const float* __restrict__ flow,
                                                            const float* __restrict__ gout,
                                                            float* __restrict__ gimage, float* __restrict__ gflow,
@@ -208,7 +195,7 @@ static int photo_grid(long items) {        // items = row jobs
 }
 
 template <int VEC, int CT>
-__global__ void __launch_bounds__(kPhotoThreads, VEC == 4 ? 2 : 4) photo_epe_fwd_kernel(
+__global__ void __launch_bounds__(kPhotoThreads, 4) photo_epe_fwd_kernel(
     const float* __restrict__ frame1, const float* __restrict__ frame2, const float* __restrict__ flow,
     const float* __restrict__ flow_gt, float* __restrict__ partials, int B, int C, BwGeom g, unsigned segs, unsigned jobs) {
   __shared__ float red[3 * 32];
@@ -289,7 +276,7 @@ __global__ void __launch_bounds__(256) finalize_sums_kernel(const float* __restr
 }
 
 template <int VEC, int CT>
-__global__ void __launch_bounds__(256, VEC == 4 ? 1 : 3) photo_epe_bwd_kernel(
+__global__ void __launch_bounds__(256, 3) photo_epe_bwd_kernel(
     const float* __restrict__ frame1, const float* __restrict__ frame2, const float* __restrict__ flow,
     const float* __restrict__ flow_gt, const float* __restrict__ sums, float g_photo, float g_epe,
     float* __restrict__ gflow, float* __restrict__ gframe2, int B, int C, BwGeom g, unsigned segs, unsigned jobs) {
@@ -386,24 +373,13 @@ static int stream_grid(long items, int threads) {        // items = row jobs (on
   return (int)blocks;
 }
 
-// pixels per thread: 4 or 2 consecutive pixels when W allows (FD_WARP_VEC overrides for experiments)
-static int pick_vec(int W) {
-  static int forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("FD_WARP_VEC");
-    forced = e ? atoi(e) : 0;
-  }
-  int v = forced > 0 ? forced : 2;
-  while (v > 1 && W % v != 0) v >>= 1;
-  return v;
-}
+// pixels per thread: 2 consecutive pixels when W allows
+static int pick_vec(int W) { return W % 2 == 0 ? 2 : 1; }
 
 // kernel<VEC, CT> for the runtime (vec, C): CT = 3 unrolls the RGB case
 #define FD_WARP_DISPATCH(kern, ...)                       \
   do {                                                    \
-    if (vec == 4) {                                       \
-      if (C == 3) kern<4, 3> __VA_ARGS__; else kern<4, 0> __VA_ARGS__; \
-    } else if (vec == 2) {                                \
+    if (vec == 2) {                                       \
       if (C == 3) kern<2, 3> __VA_ARGS__; else kern<2, 0> __VA_ARGS__; \
     } else {                                              \
       if (C == 3) kern<1, 3> __VA_ARGS__; else kern<1, 0> __VA_ARGS__; \
@@ -454,16 +430,11 @@ int fd_warp_bwd_win2(int mode, const float* frame1, const float* frame2, const f
                      const float* fsums, float g_photo, float g_epe, float* gflow, float* gimage, float* acc, int B, int H, int W,
                      cudaStream_t st);
 
-// FD_WARP_WIN=0 selects the one-thread-per-pixel-group gather kernels for every shape
+// the window kernels take three-channel frames, W % 4 == 0 and 16-byte aligned planes; the gather kernels everything else
 static bool use_win(int C, int W, const void* a, const void* b, const void* c, const void* d, const void* e2 = nullptr,
                     const void* f = nullptr) {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("FD_WARP_WIN");
-    on = e ? atoi(e) : 1;
-  }
   auto al = [](const void* q) { return q == nullptr || (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
-  return on && C == 3 && W % 4 == 0 && W >= 64 && al(a) && al(b) && al(c) && al(d) && al(e2) && al(f);
+  return C == 3 && W % 4 == 0 && W >= 64 && al(a) && al(b) && al(c) && al(d) && al(e2) && al(f);
 }
 
 extern "C" {

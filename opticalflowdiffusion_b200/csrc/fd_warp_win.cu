@@ -17,8 +17,6 @@
 // Geometry, weights and the accumulation order are fd_warp_common.cuh's (the reference's op sequence), so `out` / `mask` stay
 // bit-identical to fd_warp.cu and to the reference.  Three-channel frames with W % 4 == 0 only (else fd_warp.cu runs).
 #include <cuda.h>
-#include <stdlib.h>
-
 #include <atomic>
 
 #include "fd_tc.cuh"
@@ -60,7 +58,7 @@ struct WinParams {
   float* acc;              // (B, H, W, 4) pixel-interleaved gradient of the sampled frame, zeroed by the host; may be null
   BwGeom g;
   int B, tiles_x, tiles_y, ntiles;
-  int dbg;                 // FD_WARP_WIN_DBG: 1 = no compute, 2 = no TMA (timing isolation only: wrong results)
+  int dbg;                 // FD_WARP_WIN_DBG in FD_DIAG builds: 1 = no compute, 2 = no TMA (timing isolation only: wrong results)
 };
 
 template <int N> struct VecT;
@@ -164,7 +162,7 @@ __global__ void __launch_bounds__(kThreads, 1) warp_win_fwd_kernel(const __grid_
   const int step_y = (int)(g1 - (unsigned)step_b * p.tiles_y) * kTH;
   const int lim_x = p.tiles_x * kTW, lim_y = p.tiles_y * kTH;
   if (tile < p.ntiles) {
-    if (tid == 0 && !(p.dbg & 2)) issue(ta_next, 0);
+    if (tid == 0 && !(kDiag && (p.dbg & 2))) issue(ta_next, 0);
     load_own(ta_next, nxt);
   }
   for (int it = 0; tile < p.ntiles; ++it, tile += gridDim.x) {
@@ -180,15 +178,15 @@ __global__ void __launch_bounds__(kThreads, 1) warp_win_fwd_kernel(const __grid_
       const int cy1 = ta_next.y0 >= lim_y;
       ta_next.y0 -= cy1 * lim_y;
       ta_next.b += step_b + cy1;
-      if (tid == 0 && !(p.dbg & 2)) {
+      if (tid == 0 && !(kDiag && (p.dbg & 2))) {
         // buffer buf ^ 1 was last read by tile it - 1: its (it - 1) / 2-th use
         if (it > 0) mbar_wait(bar0 + 16 + 8 * (buf ^ 1), (uint32_t)((it - 1) >> 1) & 1u);
         issue(ta_next, buf ^ 1);
       }
       load_own(ta_next, nxt);
     }
-    if (!(p.dbg & 2)) mbar_wait(bar0 + 8 * buf, (uint32_t)(it >> 1) & 1u);
-    if (cur.exists && !(p.dbg & 1)) {
+    if (!(kDiag && (p.dbg & 2))) mbar_wait(bar0 + 8 * buf, (uint32_t)(it >> 1) & 1u);
+    if (cur.exists && !(kDiag && (p.dbg & 1))) {
       const int y = a.y0 + ry, x = a.x0 + cx;
       const int wy0 = a.y0 - kR, wx0 = a.x0 - kR;
       const uint32_t w0 = win0 + buf * kBufBytes;
@@ -471,11 +469,8 @@ int fd_warp_fwd_win(int mode, const float* frame1, const float* frame2, const fl
   const long tiles = (long)B * p.tiles_x * p.tiles_y;
   FD_REQUIRE(tiles < (1L << 31), "warp_win: too many tiles");
   p.ntiles = (int)tiles;
-  {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("FD_WARP_WIN_DBG"); dbg = e ? atoi(e) : 0; }
-    p.dbg = dbg;
-  }
+  static const int dbg = fd_diag_bits("FD_WARP_WIN_DBG");
+  p.dbg = dbg;
   CUtensorMap map;
   {
     const uint64_t dims[3] = {(uint64_t)W, (uint64_t)H, (uint64_t)B * kC};

@@ -25,8 +25,6 @@
 // Same formulas and operation order per pixel as fd_warp.cu; the frame gradient is a sum of the same terms in a different
 // order (tests: tolerance of the atomics, as before).  Three-channel frames with W % 4 == 0 only.
 #include <cuda.h>
-#include <stdlib.h>
-
 #include "fd_tc.cuh"
 #include "fd_warp_common.cuh"
 
@@ -58,7 +56,7 @@ struct BwdParams {
   float* gimage;           // gradient of the sampled frame (zeroed by the host); may be null
   BwGeom g;
   int B, tiles_x, tiles_y, ntiles;
-  int dbg;                 // FD_WARP_WIN_DBG (isolation runs, wrong results): 4 = no TMA reduction, 8 = no shared-memory scatter, 16 = no TMA loads, 64 = no zeroing / proxy fence
+  int dbg;                 // FD_WARP_WIN_DBG in FD_DIAG builds (isolation runs, wrong results): 4 = no TMA reduction, 8 = no shared-memory scatter, 16 = no TMA loads, 64 = no zeroing / proxy fence
 };
 
 struct TileAt {
@@ -165,7 +163,7 @@ __global__ void __launch_bounds__(kThreads, 1) warp_win_bwd_kernel(const __grid_
     for (int c = 0; c < kC; ++c) o.a[c] = __ldg(reinterpret_cast<const float4*>(src + po + c * HW));
   };
   auto issue_load = [&](const TileAt& a, int c, unsigned u) {      // thread 0: frame window of unit u
-    if (p.dbg & 16) return;
+    if (kDiag && (p.dbg & 16)) return;
     const uint32_t bar = bar0 + 8 * (u % kFr);
     mbar_expect_tx(bar, kTxBytes);
     tma_load_3d(frame0 + (u % kFr) * kWinBytes, &map_in, bar, a.x0 - kR, a.y0 - kR, a.b * kC + c);
@@ -215,9 +213,9 @@ __global__ void __launch_bounds__(kThreads, 1) warp_win_bwd_kernel(const __grid_
     for (int c = 0; c < kC; ++c, ++u) {
       __syncthreads();            // unit u - 1 is complete in shared memory: its scatters, its reads of frame slot (u - 1) % kFr
       const bool pv_manual = pv_x < 0 || pv_y < 0;      // (block-uniform)
-      if (want_gi && u > 0 && pv_manual && !(p.dbg & 4)) flush_manual((int)((u - 1) % kAcc), pv_x, pv_y, pv_p);
+      if (want_gi && u > 0 && pv_manual && !(kDiag && (p.dbg & 4))) flush_manual((int)((u - 1) % kAcc), pv_x, pv_y, pv_p);
       if (tid == 0) {
-        if (want_gi && u > 0 && !(p.dbg & 4)) {
+        if (want_gi && u > 0 && !(kDiag && (p.dbg & 4))) {
           if (!pv_manual) tma_reduce_add_3d(&map_grad, acc0 + ((u - 1) % kAcc) * kWinBytes, pv_x, pv_y, pv_p);
           tma_store_commit();            // (an empty group for a thread-flushed unit: keeps the group count per unit uniform)
           tma_store_wait_read<1>();      // the reduction of unit u - 2 has read its window: it may be zeroed during unit u + 1
@@ -248,7 +246,7 @@ __global__ void __launch_bounds__(kThreads, 1) warp_win_bwd_kernel(const __grid_
         ta_next.b += step_b + c2;
         load_own(ta_next, nxt);
       }
-      if (!(p.dbg & 16)) mbar_wait(bar0 + 8 * (u % kFr), (u / kFr) & 1u);
+      if (!(kDiag && (p.dbg & 16))) mbar_wait(bar0 + 8 * (u % kFr), (u / kFr) & 1u);
       const uint32_t fw = frame0 + (u % kFr) * kWinBytes, aw = acc0 + (u % kAcc) * kWinBytes;
       if (cur.exists) {
         const float4 ac = c == 0 ? cur.a[0] : (c == 1 ? cur.a[1] : cur.a[2]);      // (no dynamic indexing: registers)
@@ -284,7 +282,7 @@ __global__ void __launch_bounds__(kThreads, 1) warp_win_bwd_kernel(const __grid_
             diy[j] += gw * ((v.sw - v.nw) * ex + (v.se - v.ne) * wx[j]);
           }
           if (want_gi && (MODE == 0 || gw != 0.f)) {
-            if (inw[j] && (p.dbg & 8)) {
+            if (inw[j] && kDiag && (p.dbg & 8)) {
             } else if (inw[j]) {
               reds_f32(aw + cell[j], gw * wnw);
               reds_f32(aw + cell[j] + 4, gw * wne);
@@ -302,7 +300,7 @@ __global__ void __launch_bounds__(kThreads, 1) warp_win_bwd_kernel(const __grid_
           }
         }
       }
-      if (want_gi && !(p.dbg & 64)) {
+      if (want_gi && !(kDiag && (p.dbg & 64))) {
         zero_acc((int)((u + 1) % kAcc));       // last used by unit u - 3, whose reduction has finished reading (see above)
         fence_proxy_async_smem();              // this unit's red.shared results -> visible to the TMA reduction issued after the barrier
       }
@@ -331,7 +329,7 @@ __global__ void __launch_bounds__(kThreads, 1) warp_win_bwd_kernel(const __grid_
     }
   }
   __syncthreads();
-  if (want_gi && u > 0 && !(p.dbg & 4)) {
+  if (want_gi && u > 0 && !(kDiag && (p.dbg & 4))) {
     const bool pv_manual = pv_x < 0 || pv_y < 0;
     if (pv_manual) flush_manual((int)((u - 1) % kAcc), pv_x, pv_y, pv_p);
     if (tid == 0) {
@@ -358,17 +356,14 @@ int fd_warp_bwd_win(int mode, const float* frame1, const float* frame2, const fl
   const long tiles = (long)B * p.tiles_x * p.tiles_y;
   FD_REQUIRE(tiles < (1L << 31), "warp_win_bwd: too many tiles");
   p.ntiles = (int)tiles;
-  {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("FD_WARP_WIN_DBG"); dbg = e ? atoi(e) : 0; }
-    p.dbg = dbg;
-  }
+  static const int dbg = fd_diag_bits("FD_WARP_WIN_DBG");
+  p.dbg = dbg;
   CUtensorMap map_in, map_grad;
   const uint64_t dims[3] = {(uint64_t)W, (uint64_t)H, (uint64_t)B * kC};
   const uint64_t str[2] = {(uint64_t)W * 4, (uint64_t)H * W * 4};
   const uint32_t box[3] = {(uint32_t)kWW, (uint32_t)kWH, 1u};
   if (int e = make_tmap_f32_plain(&map_in, frame2, 3, dims, str, box)) return e;
-  if (int e = make_tmap_f32_plain(&map_grad, gimage != nullptr ? (const void*)gimage : (const void*)frame2, 3, dims, str, box, (p.dbg & 32) != 0)) return e;
+  if (int e = make_tmap_f32_plain(&map_grad, gimage != nullptr ? (const void*)gimage : (const void*)frame2, 3, dims, str, box, kDiag && (p.dbg & 32) != 0)) return e;
   const int grid = (int)(tiles < FD_NUM_SMS ? tiles : FD_NUM_SMS);
   static bool attr_done[2] = {false, false};
   if (mode == 0) {

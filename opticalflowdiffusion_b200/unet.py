@@ -19,8 +19,6 @@ from __future__ import annotations
 
 from typing import Dict, List, Optional, Tuple
 
-import os
-
 import torch
 
 from . import _lib
@@ -47,25 +45,10 @@ class Unet(UnetParams, TrainMixin):
     """Unet(dim=64, channels=C_in, out_dim=2): same constructor meaning as the reference (:272-293)."""
 
     GN_EPS = 1e-5       # nn.GroupNorm default (:176)
-    # block1's GroupNorm + SiLU applied inside the block2.proj strip conv (fd_conv3x3_gnsilu_in, inference path): removes five
-    # full-resolution gn_silu passes per forward.  Measured on the DDIM-50 benchmark: 7.08-7.11 vs 6.96 flows/s (the first
-    # two versions of the in-kernel transform were slower than the separate pass; see DESIGN.md section 6).  FD_FUSE_GN=0
-    # selects the two-pass form.
-    FUSE_GN_INPUT = os.environ.get("FD_FUSE_GN", "1") != "0"
-    # block2's GroupNorm + SiLU applied to the residual input inside the res_conv's epilogue (fd_conv_igemm_rt, inference
-    # path): the 9 ResnetBlocks that have a res_conv (ups.*, final_res_block) lose their second gn_silu pass -- 4.4 GB of
-    # HBM traffic per batch-8 forward at 440x1024.  FD_FUSE_GN_RES=0 selects the two-pass form.
-    FUSE_GN_RESIDUAL = os.environ.get("FD_FUSE_GN_RES", "1") != "0"
-    GN_SILU_EXP = os.environ.get("FD_GN_SILU_EXP", "0") != "0"
-    # Residual(PreNorm(LinearAttention)) for C in {64, 128} as two tcgen05 / TMA passes over x (fd_linattn_tc, inference
-    # path): no LayerNorm output, qkv or attention tensor in HBM.  FD_LINATTN_TC=0 selects the mma.sync kernels.
-    LINATTN_TC = os.environ.get("FD_LINATTN_TC", "1") != "0"
-    # Upsample (nearest x2 + 3x3 conv, :89-93) as four 2x2 phase convolutions on the low-resolution tensor (fd_conv_igemm_up,
-    # inference path): 2.25x fewer MACs for 12.5 % of the forward's conv FLOPs, no up-sampled tensor.  FD_UPCONV=0: two passes.
-    UPCONV_PHASES = os.environ.get("FD_UPCONV", "1") != "0"
-    # final ResnetBlock's res_conv + final_conv + un-pad crop as one launch (fd_conv_igemm_rt_head, inference path): the last
-    # 64-channel activation (461 MB at batch 8, 440x1024) is neither written nor re-read.  FD_FUSE_HEAD=0: two launches.
-    FUSE_HEAD = os.environ.get("FD_FUSE_HEAD", "1") != "0"
+    # Upsample (nearest x2 + 3x3 conv, :89-93) runs as four 2x2 phase convolutions on the low-resolution tensor
+    # (fd_conv_igemm_up, inference path): 2.25x fewer MACs for 12.5 % of the forward's conv FLOPs, no up-sampled tensor.
+    # bench.py reads this to count the forward's conv launches.
+    UPCONV_PHASES = True
     WS_EPS = 1e-5       # WeightStandardizedConv2d with fp32 input (:107)
     LN_EPS = 1e-5       # LayerNorm with fp32 input (:122)
 
@@ -106,25 +89,11 @@ class Unet(UnetParams, TrainMixin):
                 add(name + ".res_conv", rb.res_conv)
             self._resblocks.append((name, rb))
 
-        class _Slice:
-            """A row range of a conv weight, presented like a bias-free conv module."""
-
-            def __init__(self, conv, lo, hi):
-                self._conv, self._lo, self._hi, self.bias = conv, lo, hi, None
-
-            @property
-            def weight(self):
-                return self._conv.weight[self._lo:self._hi]
-
         def add_attn(name, res):
             fn = res.fn.fn
             linear = isinstance(fn.to_out, torch.nn.Sequential)
             add(name + ".to_qkv", fn.to_qkv)
             add(name + ".to_out", fn.to_out[0] if linear else fn.to_out)
-            if linear and fn.dim in (64, 128):
-                # fused LinearAttention tail (fd_linattn_apply_fused): k|v and q thirds of to_qkv are packed apart
-                add(name + ".to_kv", _Slice(fn.to_qkv, 128, 384))
-                add(name + ".to_q", _Slice(fn.to_qkv, 0, 128))
 
         self._resblocks = []
         add("init_conv", self.init_conv, kind=2)
@@ -311,10 +280,10 @@ class Unet(UnetParams, TrainMixin):
         n, h, w, c = x.shape
         out = torch.empty_like(x)
         ss_ptr = ss.data_ptr() + 4 * ss_off if ss is not None else None
-        # inference forward: the one-MUFU SiLU of the fused kernels (FD_GN_SILU_EXP=1: the exp form everywhere); the training
-        # forward (exact=True from unet_train._t_gn_silu; grad mode cannot tell the two apart, it is off inside
-        # autograd.Function.forward) keeps the exp form its parity tests were pinned on
-        fn = self._lib.fd_gn_silu if (exact or self.GN_SILU_EXP) else self._lib.fd_gn_silu_fast
+        # inference forward: the one-MUFU SiLU of the fused kernels; the training forward (exact=True from
+        # unet_train._t_gn_silu; grad mode cannot tell the two apart, it is off inside autograd.Function.forward) keeps the
+        # exp form its parity tests were pinned on
+        fn = self._lib.fd_gn_silu if exact else self._lib.fd_gn_silu_fast
         _lib.check(fn(_lib.ptr(x), _lib.ptr(stats), _lib.ptr(norm.weight), _lib.ptr(norm.bias), ss_ptr,
                       ss.shape[1] if ss is not None else 0, _lib.ptr(residual), _lib.ptr(out), n, h * w, c, self.GN_EPS, self._st))
         return out
@@ -353,28 +322,30 @@ class Unet(UnetParams, TrainMixin):
         st1, st2 = self._next_stats(), self._next_stats()
         h1 = self._conv(name + ".block1.proj", x0, x1, stats=st1)
         pc2 = self._convs[name + ".block2.proj"]
-        if h1.shape[-1] == 64 and pc2.cout == 64 and h1.shape[2] >= 128 and self.FUSE_GN_INPUT:
+        if h1.shape[-1] == 64 and pc2.cout == 64 and h1.shape[2] >= 128:
             # 64 -> 64 at full resolution: GroupNorm + scale/shift + SiLU of h1 is applied to the input strips inside the
-            # conv (fd_conv3x3_gnsilu_in), the activated tensor never goes through HBM
+            # conv (fd_conv3x3_gnsilu_in), the activated tensor never goes through HBM.  Measured on the DDIM-50 benchmark:
+            # 7.08-7.11 vs 6.96 flows/s for the separate gn_silu pass (DESIGN.md section 6)
             h2 = self._conv_gnsilu_in(name + ".block2.proj", h1, st1, rb.block1.norm, ss, self._tproj_off[name], st2)
         else:
             a1 = self._gn_silu(h1, st1, rb.block1.norm, ss, self._tproj_off[name], None)
             h2 = self._conv(name + ".block2.proj", a1, stats=st2)
         if (name + ".res_conv") in self._convs:
-            if self.FUSE_GN_RESIDUAL:
-                if head is not None:
-                    return self._conv_res_gn_head(name + ".res_conv", x0, x1, h2, st2, rb.block2.norm, head)
-                return self._conv_res_gn(name + ".res_conv", x0, x1, h2, st2, rb.block2.norm)
-            a2 = self._gn_silu(h2, st2, rb.block2.norm, None, 0, None)
-            return self._conv(name + ".res_conv", x0, x1, residual=a2)
+            # block2's GroupNorm + SiLU rides in the res_conv's epilogue: no second gn_silu pass for the 9 ResnetBlocks with a
+            # res_conv (ups.*, final_res_block), 4.4 GB less HBM traffic per batch-8 forward at 440x1024
+            if head is not None:
+                return self._conv_res_gn_head(name + ".res_conv", x0, x1, h2, st2, rb.block2.norm, head)
+            return self._conv_res_gn(name + ".res_conv", x0, x1, h2, st2, rb.block2.norm)
         assert x1 is None
         return self._gn_silu(h2, st2, rb.block2.norm, None, 0, x0)
 
     def _linear_attention(self, name: str, res, x: Tensor) -> Tensor:
         """Residual(PreNorm(LinearAttention)) (:81-87,127-135,229-244)."""
         n, h, w, c = x.shape
-        ent = self._la_tc.get(name) if self.LINATTN_TC and not getattr(self, "_no_fused_attn", False) else None
+        ent = self._la_tc.get(name)
         if ent is not None:
+            # C in {64, 128}: two tcgen05 / TMA passes over x (fd_linattn_tc), no LayerNorm output, qkv or attention tensor
+            # in HBM
             fn = res.fn.fn
             out = torch.empty_like(x)
             ws = torch.empty(self._lib.fd_linattn_tc_workspace_floats(n, h * w, c), device=x.device, dtype=torch.float32)
@@ -382,22 +353,6 @@ class Unet(UnetParams, TrainMixin):
                                                _lib.ptr(ent["wq"]), _lib.ptr(ent["sq"]), _lib.ptr(ent["wv"]),
                                                _lib.ptr(fn.to_out[0].weight), _lib.ptr(fn.to_out[0].bias), _lib.ptr(fn.to_out[1].g),
                                                _lib.ptr(out), _lib.ptr(ws), n, h * w, c, self.LN_EPS, self._st))
-            return out
-        if (name + ".to_kv") in self._convs and not getattr(self, "_no_fused_attn", False):
-            # C in {64,128}: k|v through the conv engine, then ONE fused pass for q / softmax / context / to_out /
-            # LayerNorm / residual (the q third of to_qkv and to_out run as in-kernel GEMMs)
-            y = self._chan_ln(x, res.fn.norm.g)
-            kv = self._conv(name + ".to_kv", y)
-            del y
-            ws = torch.empty(self._lib.fd_linattn_workspace_floats(n, h * w), device=x.device, dtype=torch.float32)
-            ctx_t = torch.empty(n, 4, 32, 32, device=x.device, dtype=BF16)
-            _lib.check(self._lib.fd_linattn_context(_lib.ptr(kv), 256, _lib.ptr(ctx_t), _lib.ptr(ws), n, h * w, self._st))
-            out = torch.empty_like(x)
-            to_out = self._convs[name + ".to_out"]
-            _lib.check(self._lib.fd_linattn_apply_fused(
-                _lib.ptr(x), _lib.ptr(res.fn.norm.g), _lib.ptr(self._convs[name + ".to_q"].w), _lib.ptr(ctx_t),
-                _lib.ptr(to_out.w), _lib.ptr(to_out.bias), _lib.ptr(res.fn.fn.to_out[1].g), _lib.ptr(out), n, h * w, c,
-                self.LN_EPS, self._st))
             return out
         y = self._chan_ln(x, res.fn.norm.g)
         qkv = self._conv(name + ".to_qkv", y)
@@ -518,7 +473,7 @@ class Unet(UnetParams, TrainMixin):
             h = self._resnet(f"ups.{i}.0", b1, h, skips.pop(), ss)
             h = self._resnet(f"ups.{i}.1", b2, h, skips.pop(), ss)
             h = self._linear_attention(f"ups.{i}.2", attn, h)
-            if i < n_levels - 1 and self.UPCONV_PHASES:
+            if i < n_levels - 1:
                 n_, hh, ww, cc = h.shape
                 pc = self._convs[f"ups.{i}.3"]
                 up_o = torch.empty(n_, 2 * hh, 2 * ww, pc.cout, device=dev, dtype=BF16)
@@ -532,18 +487,13 @@ class Unet(UnetParams, TrainMixin):
                 if timing is not None:
                     ev[1].record()
                 h = up_o
-            elif i < n_levels - 1:
-                n_, hh, ww, cc = h.shape
-                up_t = torch.empty(n_, 2 * hh, 2 * ww, cc, device=dev, dtype=BF16)
-                _lib.check(lib.fd_upsample2x(_lib.ptr(h), _lib.ptr(up_t), n_, hh, ww, cc, st))
-                h = self._conv(f"ups.{i}.3", up_t)
-                del up_t
             else:
                 h = self._conv(f"ups.{i}.3", h)
         fc = self.final_conv
-        if (self.FUSE_HEAD and self.FUSE_GN_RESIDUAL and not return_taps and self.dim == 64 and self.out_dim <= 4 and
+        if (not return_taps and self.dim == 64 and self.out_dim <= 4 and
                 "final_res_block.res_conv" in self._convs and self._convs["final_res_block.res_conv"].kh == 1):
-            # final ResnetBlock's res_conv + residual + final_conv + crop in one launch (the 64-channel tensor is never stored)
+            # final ResnetBlock's res_conv + residual + final_conv + crop in one launch: the last 64-channel activation
+            # (461 MB at batch 8, 440x1024) is neither written nor re-read.  return_taps needs that activation: two launches
             out = self._resnet("final_res_block", self.final_res_block, h, r, ss, head=(fc, H0, W0, pad[2], pad[0]))
             self._stats = None
             return out

@@ -125,7 +125,7 @@ class TrainMixin:
         lib, st = self._lib, _lib.stream()
         recs, blocks = [], [0]
         for name, pc in self._convs.items():
-            if pc.kind >= 2 or name.endswith((".to_kv", ".to_q")):
+            if pc.kind >= 2:
                 continue
             cout, k = pc.w.shape
             taps = 1 if pc.kind == 1 else pc.kh * pc.kw
@@ -358,11 +358,8 @@ class TrainMixin:
         a1 = self._t_gn_silu(tape, h1, st1, rb.block1.norm, ss, dss, self._tproj_off[name], None, rb.block1.proj.bias)
         h2 = self._t_conv(tape, name + ".block2.proj", a1, stats=st2)
         if (name + ".res_conv") in self._convs:
-            if self.FUSE_GN_RESIDUAL:
-                return self._t_conv(tape, name + ".res_conv", x0, x1, need_dgrad=need_dgrad,
-                                    res_gn=(h2, st2, rb.block2.norm, rb.block2.proj.bias))
-            a2 = self._t_gn_silu(tape, h2, st2, rb.block2.norm, None, None, 0, None, rb.block2.proj.bias)
-            return self._t_conv(tape, name + ".res_conv", x0, x1, residual=a2, need_dgrad=need_dgrad)
+            return self._t_conv(tape, name + ".res_conv", x0, x1, need_dgrad=need_dgrad,
+                                res_gn=(h2, st2, rb.block2.norm, rb.block2.proj.bias))
         assert x1 is None
         return self._t_gn_silu(tape, h2, st2, rb.block2.norm, None, None, 0, x0, rb.block2.proj.bias)
 

@@ -8,8 +8,6 @@ SURVEY.md section 2).  All tensors must be CUDA fp32; there is no CPU path.
 """
 from __future__ import annotations
 
-import os
-
 from typing import Optional, Sequence, Tuple
 
 import torch
@@ -188,10 +186,6 @@ def softsplat(tenIn: Tensor, tenFlow: Tensor, tenMetric: Optional[Tensor], strMo
     return tenOut
 
 
-# warp_forward_flow on three-channel images through the fused two-launch path (FD_SPLAT_SUM3=0: prepare / splat / finish)
-FUSED_SUM3 = os.environ.get("FD_SPLAT_SUM3", "1") != "0"
-
-
 class _ForwardWarpSumFn(torch.autograd.Function):
     """warp_forward_flow(warp_style='sum') as three launches: prepare (NaN -> weight 0, append the
     weight channel), splat, finish (holes -> NaN).  Gradient flows to ``flow`` only (cond has no
@@ -203,7 +197,7 @@ class _ForwardWarpSumFn(torch.autograd.Function):
         B, C, H, W = first.shape
         lib = _lib.load()
         st = _lib.stream()
-        if C == 3 and FUSED_SUM3:
+        if C == 3:
             # two launches, pixel-interleaved accumulation (one 128-bit reduction per tap): fd_forward_warp_sum3
             Ho, Wo = H // scale, W // scale
             need_bwd = bool(ctx.needs_input_grad[0] or ctx.needs_input_grad[1])

@@ -1,6 +1,7 @@
 """Times fd_linattn_tc (tcgen05 LinearAttention, csrc/fd_linattn_tc.cu) per launch at the UNet's shapes: CUDA events around the
-three launches separately is not possible through the C ABI, so the whole block is timed and FD_LA_DBG (diagnostic switches
-compiled into the kernels, see CtxParams::dbg) isolates the parts."""
+three launches separately is not possible through the C ABI, so the whole block is timed and FD_LA_DBG (diagnostic switches,
+see CtxParams::dbg) isolates the parts.  FD_LA_DBG only acts in a diagnostic build of the library:
+FD_DIAG=1 python -m opticalflowdiffusion_b200.build --force."""
 import json
 import os
 import sys

@@ -1,5 +1,4 @@
-"""CUDA-event timing of fd_conv_wgrad on the training shapes (batch 8, 368x768 crops).  FD_WGRAD_STRIP=0 selects the
-generic one-job-per-tap kernel for the 3x3 shapes."""
+"""CUDA-event timing of fd_conv_wgrad on the training shapes (batch 8, 368x768 crops)."""
 import os
 import sys
 

@@ -98,6 +98,9 @@ CASES = [
     (2, (64, 64), 128, 16, 128, (3, 3), (1, 1), True, True, True),      # ... two sources + residual
     (1, (128,), 128, 24, 64, (3, 3), (1, 1), True, False, True),        # 12 M-tiles: one M-tile per CTA (count % 4 != 0 is 0 here -> 2 per CTA), 3 super-tiles
     (1, (128,), 128, 20, 64, (3, 3), (1, 1), False, False, False),      # 10 M-tiles: % 4 != 0 -> one M-tile per CTA
+    (2, (64,), 64, 37, 256, (3, 3), (1, 1), True, False, True),         # rolling-strip kernel (A operand in tensor memory)
+    (1, (64, 64), 64, 21, 200, (3, 3), (1, 1), True, True, True),       # ... two passes, ragged last column block, residual
+    (3, (128,), 64, 5, 130, (3, 3), (1, 1), True, False, False),        # ... fewer rows than CTAs: some ranges are one row
 ]
 
 
@@ -131,36 +134,6 @@ def test_conv_pixel_unshuffle(L, case):
     bias = torch.randn(Cout, generator=g).cuda()
     out, _ = run_conv(L, [x], w, bias, (0, 0), mode=1)
     close(out, ref_conv([x], w, bias, (0, 0), mode=1))
-
-
-STRIP_CASES = [
-    # N, Cins, H, W, residual, stats  (3x3, pad 1, Cout 64, W >= 64: the rolling-strip kernel)
-    (2, (64,), 37, 256, False, True),
-    (1, (64, 64), 21, 200, True, True),        # two passes, ragged last column block, caller's residual
-    (3, (128,), 5, 130, False, False),         # fewer rows than CTAs: some ranges are a single row
-]
-
-
-@pytest.mark.parametrize("case", STRIP_CASES)
-def test_strip_conv_tensor_memory_operand(L, case, monkeypatch):
-    """The default strip-conv issuer stages the activation strips in tensor memory (tcgen05.cp) and issues the A-from-TMEM
-    form of tcgen05.mma; FD_STRIP_TS=0 selects the shared-memory-operand variant.  Same products in the same order, so the
-    two outputs must be equal bit for bit."""
-    N, cins, H, W, has_res, stats = case
-    g = torch.Generator().manual_seed(H * W)
-    xs = [torch.randn(N, c, H, W, generator=g).cuda() for c in cins]
-    cin = sum(cins)
-    w = (torch.randn(64, cin, 3, 3, generator=g) / (cin * 9) ** 0.5).cuda()
-    bias = torch.randn(64, generator=g).cuda()
-    res = torch.randn(N, 64, H, W, generator=g).cuda() if has_res else None
-    monkeypatch.setenv("FD_STRIP_TS", "0")
-    out_ss, gn_ss = run_conv(L, xs, w, bias, (1, 1), res, stats)
-    monkeypatch.setenv("FD_STRIP_TS", "1")
-    out_ts, gn_ts = run_conv(L, xs, w, bias, (1, 1), res, stats)
-    close(out_ss, ref_conv(xs, w, bias, (1, 1), res))
-    assert torch.equal(out_ss, out_ts)
-    if stats:
-        assert torch.allclose(gn_ss, gn_ts, rtol=1e-12, atol=1e-9)
 
 
 @pytest.mark.parametrize("case", [(2, 37, 256, True), (1, 21, 200, False), (3, 5, 130, True), (1, 70, 64, True)])

@@ -89,9 +89,9 @@ def test_unet_vs_oracle_64x128():
 
 
 def test_unet_fused_output_head_padded_shape():
-    """Inference forward at a shape that needs replicate padding (44x140 -> 48x144): the fused tail (FD_FUSE_HEAD:
-    res_conv + GroupNorm residual + final_conv + crop in one launch) == the two-launch tail == the oracle (InputPadder
-    pad / unpad around the fp32 forward, utils.py:6-27 + denoising_diffusion.py:414-417)."""
+    """Inference forward at a shape that needs replicate padding (44x140 -> 48x144): the fused tail (res_conv + GroupNorm
+    residual + final_conv + crop in one launch) == the two-launch tail that return_taps=True takes == the oracle
+    (InputPadder pad / unpad around the fp32 forward, utils.py:6-27 + denoising_diffusion.py:414-417)."""
     import torch.nn.functional as F
     net = build_unet(3, 5)
     sd = {k: v.clone() for k, v in net.state_dict().items()}
@@ -106,14 +106,8 @@ def test_unet_fused_output_head_padded_shape():
     with torch.no_grad():
         ref = O.unet_forward(sd, F.pad(x, pad, mode="replicate"), F.pad(cond, pad, mode="replicate"), t)
         ref = ref[..., pad[2]:pad[2] + H, pad[0]:pad[0] + W]
-        if not (net.FUSE_HEAD and net.FUSE_GN_RESIDUAL):
-            pytest.skip("the fused tail is switched off by FD_FUSE_HEAD / FD_FUSE_GN_RES")
         fused = net(x.cuda(), cond.cuda(), t.cuda())
-        net.FUSE_HEAD = False
-        try:
-            two = net(x.cuda(), cond.cuda(), t.cuda())
-        finally:
-            del net.FUSE_HEAD
+        two = net(x.cuda(), cond.cuda(), t.cuda(), return_taps=True)[0]
     assert fused.shape == two.shape == (B, 2, H, W)
     assert (fused.cpu() - ref).abs().max().item() < 3e-2
     assert (two.cpu() - ref).abs().max().item() < 3e-2
