@@ -154,10 +154,8 @@ FD_API int fd_ddpm_step(const float* x, const float* model_out, const float* noi
  * (:297,374), emitted as the 7-tap "row-im2col" tensor packed[b,h,w, kx*Cpad + c] = in[b,c,h,w+kx-3]
  * (bf16, 64 channels per pixel, zero outside the image / above Cpad*7).  x:(B,Cx,H,W) cond:(B,Cc,H,W)
  * fp32 NCHW; if nan_mask: NaNs of x become 0 and a channel any_c(isnan(x)) is inserted after x.
- * Ctot = Cx + nan_mask + Cc must be <= 9. */
-FD_API int fd_pack_input(const float* x, const float* cond, void* packed, int B, int Cx, int Cc, int H, int W,
-                  int nan_mask, void* stream);
-/* Same, with x / cond given as H0 x W0 planes that sit at (pad_top, pad_left) inside the H x W frame the UNet runs on
+ * Ctot = Cx + nan_mask + Cc must be <= 9.
+ * x / cond are H0 x W0 planes that sit at (pad_top, pad_left) inside the H x W frame the UNet runs on
  * (H, W multiples of 8: three pixel-unshuffle downsamples, :95-99); the border is replicate-padded on the fly, i.e.
  * InputPadder(mode='sintel') (future/raft_utils.py:7-25) folded into the packing: 436x1024 -> 440x1024 costs no pass. */
 FD_API int fd_pack_input_pad(const float* x, const float* cond, void* packed, int B, int Cx, int Cc, int H0, int W0,
@@ -309,11 +307,9 @@ FD_API int fd_attention(const void* qkv, void* out, int N, int HW, void* stream)
 FD_API size_t fd_tensor_stats_workspace_floats(long inner);
 FD_API int fd_tensor_stats(const float* x, int B, long inner, float* out4, float* workspace, void* stream);
 
-/* final 1x1 conv (:361,417) 64 -> Cout (<= 64; four output channels per launch) from bf16 NHWC to fp32 NCHW */
-FD_API int fd_final_conv(const void* x, const float* w, const float* bias, float* out, int N, int HW, int Cin,
-                  int Cout, void* stream);
-/* Same on an (N,H,W,64) frame, writing only the H0 x W0 window at (pad_top, pad_left) as fp32 (N,Cout,H0,W0): the
- * InputPadder.unpad crop (future/raft_utils.py:20-25) folded into the store. */
+/* final 1x1 conv (:361,417) 64 -> Cout (<= 64; four output channels per launch) on a bf16 NHWC (N,H,W,64) frame, writing
+ * only the H0 x W0 window at (pad_top, pad_left) as fp32 (N,Cout,H0,W0): the InputPadder.unpad crop
+ * (future/raft_utils.py:20-25) folded into the store. */
 FD_API int fd_final_conv_crop(const void* x, const float* w, const float* bias, float* out, int N, int H, int W, int Cin,
                        int Cout, int pad_top, int pad_left, int H0, int W0, void* stream);
 
@@ -357,7 +353,7 @@ FD_API int fd_upsample2x_bwd(const void* dy, void* dx, int N, int H, int W, int 
 FD_API int fd_add_bf16(const void* a, const void* b, void* out, long n, void* stream);
 /* db[C] += sum over pixels of dy (bf16 [npix][C]) */
 FD_API int fd_bias_grad(const void* dy, float* db, long npix, int C, void* stream);
-/* backward of fd_final_conv: dout fp32 NCHW (N,Cout,HW) -> dx bf16 (N,HW,64); dw[Cout][64], db[Cout] += */
+/* backward of fd_final_conv_crop over the whole frame: dout fp32 NCHW (N,Cout,HW) -> dx bf16 (N,HW,64); dw[Cout][64], db[Cout] += */
 FD_API int fd_final_conv_bwd(const void* x, const float* w, const float* dout, void* dx, float* dw, float* db,
                       int N, int HW, int Cin, int Cout, void* stream);
 /* dgrad weights from the forward's packed weights: wd[ci][(T-1-tap)*Cout + co] = wpacked[co][tap*Cin + ci]

@@ -48,7 +48,6 @@ SIGNATURES = {
     "fd_ddim_step": (c_int, [_P, _P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _I, _P]),
     "fd_ddpm_step": (c_int, [_P, _P, _P, _P, _P, _L, _F, _F, _F, _P]),
     "fd_dpmpp_step": (c_int, [_P, _P, _P, _P, _P, _P, _L, _F, _F, _F, _F, _I, _P]),
-    "fd_pack_input": (c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _P]),
     "fd_pack_input_pad": (c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
     "fd_pack_input_wide": (c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
     "fd_prep_weight": (c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _F, _P]),
@@ -65,7 +64,6 @@ SIGNATURES = {
     "fd_linattn": (c_int, [_P, _P, _P, _I, _I, _P]),
     "fd_linattn_context": (c_int, [_P, _I, _P, _P, _I, _I, _P]),
     "fd_attention": (c_int, [_P, _P, _I, _I, _P]),
-    "fd_final_conv": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "fd_final_conv_crop": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
     "fd_nchw_to_nhwc_bf16": (c_int, [_P, _P, _I, _I, _I, _P]),
     "fd_nhwc_bf16_to_nchw": (c_int, [_P, _P, _I, _I, _I, _P]),

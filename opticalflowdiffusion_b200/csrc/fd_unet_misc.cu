@@ -597,19 +597,6 @@ __global__ void __launch_bounds__(256) nhwc_to_nchw_kernel(const __nv_bfloat16* 
 
 extern "C" {
 
-int fd_pack_input(const float* x, const float* cond, void* packed, int B, int Cx, int Cc, int H, int W, int nan_mask,
-                  void* stream) {
-  FD_REQUIRE(x && packed && B > 0 && H > 0 && W > 0 && Cx > 0 && Cc >= 0, "pack_input: bad argument");
-  FD_REQUIRE(cond != nullptr || Cc == 0, "pack_input: Cc > 0 needs cond");
-  FD_REQUIRE(Cx + (nan_mask ? 1 : 0) + Cc <= 9, "pack_input: at most 9 input channels (7 taps x 9 <= 64)");
-  const int segs = (W + kPackPx - 1) / kPackPx;
-  FD_REQUIRE((long)B * H * segs < (1L << 31), "pack_input: too many rows");
-  pack_input_kernel<<<(unsigned)((long)B * H * segs), 256, 0, (cudaStream_t)stream>>>(
-      x, cond, static_cast<__nv_bfloat16*>(packed), B, Cx, Cc, H, W, nan_mask, segs, H, W, 0, 0);
-  FD_LAUNCH_CHECK();
-  return FD_OK;
-}
-
 int fd_pack_input_pad(const float* x, const float* cond, void* packed, int B, int Cx, int Cc, int H0, int W0, int pad_top,
                       int pad_left, int H, int W, int nan_mask, void* stream) {
   FD_REQUIRE(x && packed && B > 0 && H0 > 0 && W0 > 0 && Cx > 0 && Cc >= 0, "pack_input_pad: bad argument");
@@ -743,19 +730,6 @@ int fd_time_proj(const float* temb, const float* w, const float* bias, float* ou
   const long threads = (long)B * J * 32;
   time_proj_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(temb, w, bias, out, B, time_dim, J);
   FD_LAUNCH_CHECK();
-  return FD_OK;
-}
-
-int fd_final_conv(const void* x, const float* w, const float* bias, float* out, int N, int HW, int Cin, int Cout,
-                  void* stream) {
-  FD_REQUIRE(x && w && bias && out && N > 0 && HW > 0 && Cin % 8 == 0 && Cout >= 1 && Cout <= 64, "final_conv: bad argument");
-  FD_REQUIRE(Cin == 64, "final_conv: the UNet's final conv has 64 input channels (got %d)", Cin);
-  FD_REQUIRE((long)N * HW < (1L << 31), "final_conv: too many pixels");
-  for (int o = 0; o < Cout; o += 4) {
-    final_conv_kernel<16><<<egrid((long)N * HW * 4, 256), 256, 0, (cudaStream_t)stream>>>(
-        static_cast<const __nv_bfloat16*>(x), w, bias, out, N, (long)HW, Cout, HW, 1, HW, 0, 0, o);
-    FD_LAUNCH_CHECK();
-  }
   return FD_OK;
 }
 

@@ -17,13 +17,14 @@ There is no PyTorch fallback: a missing library or a non-sm_100 device raises.
 """
 from __future__ import annotations
 
+from functools import partial
 from typing import Dict, List, Optional, Tuple
 
 import torch
 
 from . import _lib
 from .unet_params import UnetParams, _ResnetBlock
-from .unet_train import TrainMixin, UnetFunction
+from .unet_train import TrainMixin, UnetFunction, _batch_table
 
 Tensor = torch.Tensor
 BF16 = torch.bfloat16
@@ -66,8 +67,12 @@ class Unet(UnetParams, TrainMixin):
         self._tproj_w: Optional[Tensor] = None
         self._tproj_b: Optional[Tensor] = None
         self._tproj_off: Dict[str, int] = {}
+        self._up_w: Dict[int, Tensor] = {}       # phase-decomposed Upsample weights (fd_prep_weight_upconv)
+        self._la_tc: Dict[str, Dict[str, Tensor]] = {}       # tcgen05 LinearAttention operands (fd_linattn_tc_prep)
+        self._prep_table = None
         self._prepared_versions = None
         self.weights_epoch = 0      # bumped by optimisers that update the parameters through raw pointers
+        self._conv_timing: Optional[list] = None     # bench.py's roofline pass sets a list: see _launch_conv
 
     # ------------------------------------------------------------------ weight preparation
     def _build_conv_table(self):
@@ -156,12 +161,8 @@ class Unet(UnetParams, TrainMixin):
                                               pc.kind, int(pc.ws), self.WS_EPS, st))
             pc.bias = pc.src.bias.detach().float().contiguous() if pc.src.bias is not None else None
         if recs:
-            key = tuple(tuple(r) for r in recs)
-            cur = getattr(self, "_prep_table", None)
-            if cur is None or cur[0] != key or cur[1].device != dev:
-                cur = (key, torch.tensor(recs, dtype=torch.int64).to(dev), torch.tensor(blocks, dtype=torch.int32).to(dev))
-                self._prep_table = cur
-            _lib.check(lib.fd_prep_weight_batch(_lib.ptr(cur[1]), _lib.ptr(cur[2]), len(recs), blocks[-1], self.WS_EPS, st))
+            table, blk = _batch_table(self, "_prep_table", recs, blocks, dev)
+            _lib.check(lib.fd_prep_weight_batch(_lib.ptr(table), _lib.ptr(blk), len(recs), blocks[-1], self.WS_EPS, st))
         ws, bs, off = [], [], 0
         self._tproj_off = {}
         for name, rb in self._resblocks:
@@ -173,9 +174,7 @@ class Unet(UnetParams, TrainMixin):
             ws.append(lin.weight.detach().float())
             bs.append(lin.bias.detach().float())
         # phase-decomposed weights of the Upsample convs (fd_prep_weight_upconv), rewritten in place
-        up = getattr(self, "_up_w", None)
-        if up is None:
-            up = self._up_w = {}
+        up = self._up_w
         for i, stage in enumerate(self.ups):
             if i >= len(self.ups) - 1:
                 continue
@@ -187,9 +186,7 @@ class Unet(UnetParams, TrainMixin):
                 buf = up[i] = torch.empty(4, cout, 4 * cin, device=wt.device, dtype=BF16)
             _lib.check(lib.fd_prep_weight_upconv(_lib.ptr(wt.detach().float().contiguous()), _lib.ptr(buf), cout, cin, st))
         # operands of the tcgen05 LinearAttention blocks (fd_linattn_tc_prep): buffers allocated once, rewritten in place
-        la = getattr(self, "_la_tc", None)
-        if la is None:
-            la = self._la_tc = {}
+        la = self._la_tc
         for name, res in self._linattn_blocks():
             fn = res.fn.fn
             if fn.dim not in (64, 128):
@@ -217,6 +214,23 @@ class Unet(UnetParams, TrainMixin):
         self._prepared_versions = ver
 
     # ------------------------------------------------------------------ kernel wrappers
+    def _launch_conv(self, name: str, npix: int, fn, *args):
+        """``fn(*args)``: the launch of conv ``name`` with ``npix`` output pixels.  While ``_conv_timing`` is a list
+        (bench.py's roofline pass) it also appends ``(name, algorithmic FLOPs, (start, end) CUDA events)``."""
+        timing = self._conv_timing
+        if timing is None:
+            _lib.check(fn(*args))
+            return
+        pc = self._convs[name]
+        # algorithmic K: init_conv's packing pads it to 7 or 49 taps of 64 channels; an Upsample counts as the reference's
+        # 3x3 conv on the up-sampled tensor, whatever its phase decomposition launches
+        k = pc.w.shape[1] if pc.kind < 2 else 49 * self.channels
+        ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
+        timing.append((name, 2.0 * npix * pc.cout * k, ev))
+        ev[0].record()
+        _lib.check(fn(*args))
+        ev[1].record()
+
     def _conv(self, name: str, src0: Tensor, src1: Optional[Tensor] = None, residual: Optional[Tensor] = None,
               stats: Optional[Tensor] = None) -> Tensor:
         pc = self._convs[name]
@@ -225,17 +239,9 @@ class Unet(UnetParams, TrainMixin):
         if pc.mode == 1:
             h, w = h // 2, w // 2
         out = torch.empty(n, h, w, pc.cout, device=src0.device, dtype=BF16)
-        timing = getattr(self, "_conv_timing", None)
-        if timing is not None:      # bench.py's roofline pass: CUDA events around every conv launch
-            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-            flops = 2.0 * n * h * w * pc.cout * pc.w.shape[1] if pc.kind < 2 else 2.0 * n * h * w * pc.cout * 49 * self.channels
-            timing.append((name, flops, ev))
-            ev[0].record()
-        _lib.check(self._lib.fd_conv_igemm(_lib.ptr(src0), c0, _lib.ptr(src1), c1, _lib.ptr(pc.w), _lib.ptr(pc.bias),
-                                           _lib.ptr(residual), _lib.ptr(out), _lib.ptr(stats), n, h, w, pc.cout,
-                                           pc.kh, pc.kw, pc.pad[0], pc.pad[1], pc.mode, self._st))
-        if timing is not None:
-            ev[1].record()
+        self._launch_conv(name, n * h * w, self._lib.fd_conv_igemm, _lib.ptr(src0), c0, _lib.ptr(src1), c1, _lib.ptr(pc.w),
+                          _lib.ptr(pc.bias), _lib.ptr(residual), _lib.ptr(out), _lib.ptr(stats), n, h, w, pc.cout,
+                          pc.kh, pc.kw, pc.pad[0], pc.pad[1], pc.mode, self._st)
         return out
 
     def _conv_gnsilu_in(self, name: str, src: Tensor, in_stats: Tensor, norm, ss: Optional[Tensor], ss_off: int,
@@ -243,17 +249,10 @@ class Unet(UnetParams, TrainMixin):
         pc = self._convs[name]
         n, h, w, _ = src.shape
         out = torch.empty(n, h, w, pc.cout, device=src.device, dtype=BF16)
-        timing = getattr(self, "_conv_timing", None)
-        if timing is not None:
-            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-            timing.append((name, 2.0 * n * h * w * pc.cout * pc.w.shape[1], ev))
-            ev[0].record()
         ss_ptr = ss.data_ptr() + 4 * ss_off if ss is not None else None
-        _lib.check(self._lib.fd_conv3x3_gnsilu_in(_lib.ptr(src), _lib.ptr(in_stats), _lib.ptr(norm.weight), _lib.ptr(norm.bias),
-                                                  ss_ptr, ss.shape[1] if ss is not None else 0, self.GN_EPS, _lib.ptr(pc.w),
-                                                  _lib.ptr(pc.bias), None, _lib.ptr(out), _lib.ptr(stats), n, h, w, self._st))
-        if timing is not None:
-            ev[1].record()
+        self._launch_conv(name, n * h * w, self._lib.fd_conv3x3_gnsilu_in, _lib.ptr(src), _lib.ptr(in_stats),
+                          _lib.ptr(norm.weight), _lib.ptr(norm.bias), ss_ptr, ss.shape[1] if ss is not None else 0, self.GN_EPS,
+                          _lib.ptr(pc.w), _lib.ptr(pc.bias), None, _lib.ptr(out), _lib.ptr(stats), n, h, w, self._st)
         return out
 
     def _conv_res_gn(self, name: str, src0: Tensor, src1: Optional[Tensor], raw: Tensor, raw_stats: Tensor, norm) -> Tensor:
@@ -262,17 +261,9 @@ class Unet(UnetParams, TrainMixin):
         n, h, w, c0 = src0.shape
         c1 = src1.shape[-1] if src1 is not None else 0
         out = torch.empty(n, h, w, pc.cout, device=src0.device, dtype=BF16)
-        timing = getattr(self, "_conv_timing", None)
-        if timing is not None:
-            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-            timing.append((name, 2.0 * n * h * w * pc.cout * pc.w.shape[1], ev))
-            ev[0].record()
-        _lib.check(self._lib.fd_conv_igemm_rt(_lib.ptr(src0), c0, _lib.ptr(src1), c1, _lib.ptr(pc.w), _lib.ptr(pc.bias),
-                                              _lib.ptr(raw), _lib.ptr(raw_stats), _lib.ptr(norm.weight), _lib.ptr(norm.bias),
-                                              self.GN_EPS, _lib.ptr(out), n, h, w, pc.cout, pc.kh, pc.kw, pc.pad[0], pc.pad[1],
-                                              self._st))
-        if timing is not None:
-            ev[1].record()
+        self._launch_conv(name, n * h * w, self._lib.fd_conv_igemm_rt, _lib.ptr(src0), c0, _lib.ptr(src1), c1, _lib.ptr(pc.w),
+                          _lib.ptr(pc.bias), _lib.ptr(raw), _lib.ptr(raw_stats), _lib.ptr(norm.weight), _lib.ptr(norm.bias),
+                          self.GN_EPS, _lib.ptr(out), n, h, w, pc.cout, pc.kh, pc.kw, pc.pad[0], pc.pad[1], self._st)
         return out
 
     def _gn_silu(self, x: Tensor, stats: Tensor, norm, ss: Optional[Tensor], ss_off: int,
@@ -303,17 +294,30 @@ class Unet(UnetParams, TrainMixin):
         c1 = src1.shape[-1] if src1 is not None else 0
         fc, h0, w0, pt, pl = head
         out = torch.empty(n, self.out_dim, h0, w0, device=src0.device, dtype=torch.float32)
-        timing = getattr(self, "_conv_timing", None)
-        if timing is not None:
-            ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-            timing.append((name, 2.0 * n * h * w * pc.cout * pc.w.shape[1], ev))
-            ev[0].record()
-        _lib.check(self._lib.fd_conv_igemm_rt_head(_lib.ptr(src0), c0, _lib.ptr(src1), c1, _lib.ptr(pc.w), _lib.ptr(pc.bias),
-                                                   _lib.ptr(raw), _lib.ptr(raw_stats), _lib.ptr(norm.weight), _lib.ptr(norm.bias),
-                                                   self.GN_EPS, _lib.ptr(fc.weight), _lib.ptr(fc.bias), self.out_dim, _lib.ptr(out),
-                                                   n, h, w, h0, w0, pt, pl, self._st))
-        if timing is not None:
-            ev[1].record()
+        self._launch_conv(name, n * h * w, self._lib.fd_conv_igemm_rt_head, _lib.ptr(src0), c0, _lib.ptr(src1), c1,
+                          _lib.ptr(pc.w), _lib.ptr(pc.bias), _lib.ptr(raw), _lib.ptr(raw_stats), _lib.ptr(norm.weight),
+                          _lib.ptr(norm.bias), self.GN_EPS, _lib.ptr(fc.weight), _lib.ptr(fc.bias), self.out_dim, _lib.ptr(out),
+                          n, h, w, h0, w0, pt, pl, self._st)
+        return out
+
+    def _upsample(self, i: int, x: Tensor) -> Tensor:
+        """Upsample ``ups.{i}.3`` (nearest x2 + 3x3 conv, :89-93) as the four phase convolutions of fd_conv_igemm_up."""
+        pc = self._convs[f"ups.{i}.3"]
+        n, h, w, c = x.shape
+        out = torch.empty(n, 2 * h, 2 * w, pc.cout, device=x.device, dtype=BF16)
+        self._launch_conv(f"ups.{i}.3", n * 4 * h * w, self._lib.fd_conv_igemm_up, _lib.ptr(x), c, _lib.ptr(self._up_w[i]),
+                          _lib.ptr(pc.bias), _lib.ptr(out), n, h, w, pc.cout, self._st)
+        return out
+
+    def _final_conv_crop(self, x: Tensor, frame: Tuple[int, int, int, int]) -> Tensor:
+        """final_conv (:361,417) on the padded frame, storing only the H0 x W0 window at (pad_top, pad_left) of
+        ``frame = (H0, W0, pad_top, pad_left)``: InputPadder.unpad folded into the store."""
+        n, h, w, _ = x.shape
+        H0, W0, pt, pl = frame
+        fc = self.final_conv
+        out = torch.empty(n, self.out_dim, H0, W0, device=x.device, dtype=torch.float32)
+        _lib.check(self._lib.fd_final_conv_crop(_lib.ptr(x), _lib.ptr(fc.weight), _lib.ptr(fc.bias), _lib.ptr(out), n, h, w,
+                                                self.dim, self.out_dim, pt, pl, H0, W0, self._st))
         return out
 
     def _resnet(self, name: str, rb: _ResnetBlock, x0: Tensor, x1: Optional[Tensor], ss: Optional[Tensor],
@@ -392,44 +396,49 @@ class Unet(UnetParams, TrainMixin):
                     "UNets (flow_pred.py:23-37) are used frozen (flow_diffuser.py:93-94): call them under torch.no_grad() or "
                     "set requires_grad_(False)")
             return UnetFunction.apply(self, x, external_cond, time, nan_mask, *self.parameters())
-        with _lib.nvtx_range("unet.forward"):
-            return self._forward_infer(x, external_cond, time, nan_mask, return_taps)
+        with _lib.nvtx_range("unet.forward"), torch.no_grad():
+            self._begin(x, external_cond, time)
+            blocks = _InferBlocks(self, {} if return_taps else None)
+            out = self._walk(blocks, x, external_cond, time, nan_mask)
+            if return_taps:
+                return out, {k: (v if v.dim() == 2 else v.permute(0, 3, 1, 2).float()) for k, v in blocks.taps.items()}
+            return out
 
-    @torch.no_grad()
-    def _forward_infer(self, x: Tensor, external_cond: Optional[Tensor], time: Optional[Tensor], nan_mask: bool = False,
-                       return_taps: bool = False):
+    def _begin(self, x: Tensor, external_cond: Optional[Tensor], time: Optional[Tensor]):
+        """Input checks, weight preparation and the launch stream: the start of both forwards."""
         _lib.require_cuda(x, external_cond, time)
         if self.time_in and time is None:
             raise ValueError("when Unet takes time arg, time argument must be passed in")      # :378-379
         self.prepare()
         self._lib = _lib.load()
         self._st = _lib.stream()
+
+    def _walk(self, blocks, x: Tensor, external_cond: Optional[Tensor], time: Optional[Tensor], nan_mask: bool):
+        """The body of ``Unet.forward`` (:363-417) for both forwards.  ``blocks`` runs the blocks: ``_InferBlocks`` (fused
+        kernels, nothing kept) or ``unet_train._TrainBlocks`` (records the tape for the backward).  ``blocks.group``
+        marks where a gradient bucket of the training backward starts; ``blocks.tap`` offers an activation to
+        ``return_taps``."""
         lib, st = self._lib, self._st
         B, Cx, H0, W0 = x.shape
         Cc = external_cond.shape[1] if external_cond is not None else 0
         assert Cx + int(nan_mask) + Cc == self.channels, (Cx, nan_mask, Cc, self.channels)
         dev = x.device
-        x = x.float()
-        cond = external_cond.float() if external_cond is not None else None
+        x = x.detach().float().contiguous()
+        cond = external_cond.detach().float().contiguous() if external_cond is not None else None
         # three 2x pixel-unshuffle downsamples (:95-99) need H, W % 8 == 0 (436 -> 440): replicate-pad like the
         # repo's own InputPadder(mode='sintel') (future/raft_utils.py:7-25) and crop the prediction back -- both folded
-        # into the first / last kernel (fd_pack_input_pad clamps its reads, fd_final_conv_crop writes the window only)
+        # into the first / last kernel (the input packing clamps its reads, the output head writes the window only)
         mult = 2 ** (len(self.downs) - 1)                # 8, or 4 for the three-level autoencoder UNets (flow_pred.py:23-37)
         ph, pw = (-H0) % mult, (-W0) % mult
-        pad = (pw // 2, pw - pw // 2, ph // 2, ph - ph // 2)
-        x = x.contiguous()
-        cond = cond.contiguous() if cond is not None else None
+        pt, pl = ph // 2, pw // 2
         H, W = H0 + ph, W0 + pw
-        taps = {}
 
+        blocks.group("front")
         # time embedding (:319-324) and every block's (scale, shift) (:206-208); none at all for Unet(time_in=False)
-        ss = temb = None
+        ss = None
         if self.time_in:
-            time = time.to(torch.int64).contiguous()
-            temb = torch.empty(B, self.time_dim, device=dev, dtype=torch.float32)
-            tm = self.time_mlp
-            _lib.check(lib.fd_time_embed(_lib.ptr(time), _lib.ptr(tm[1].weight), _lib.ptr(tm[1].bias), _lib.ptr(tm[3].weight),
-                                         _lib.ptr(tm[3].bias), _lib.ptr(temb), B, self.dim, self.time_dim, st))
+            temb = blocks.time_embedding(time.to(torch.int64).contiguous())
+            blocks.tap("temb", temb)
             J = self._tproj_w.shape[0]
             ss = torch.empty(B, J, device=dev, dtype=torch.float32)
             _lib.check(lib.fd_time_proj(_lib.ptr(temb), _lib.ptr(self._tproj_w), _lib.ptr(self._tproj_b), _lib.ptr(ss), B,
@@ -440,70 +449,77 @@ class Unet(UnetParams, TrainMixin):
         # init_conv 7x7 (:297,374) as a 7x1 conv over the horizontally unrolled input
         packed = torch.empty(B, H, W, 64, device=dev, dtype=BF16)
         pack = lib.fd_pack_input_wide if self._wide_input else lib.fd_pack_input_pad
-        _lib.check(pack(_lib.ptr(x), _lib.ptr(cond), _lib.ptr(packed), B, Cx, Cc, H0, W0, pad[2], pad[0], H, W, int(nan_mask), st))
-        h = self._conv("init_conv", packed)
+        _lib.check(pack(_lib.ptr(x), _lib.ptr(cond), _lib.ptr(packed), B, Cx, Cc, H0, W0, pt, pl, H, W, int(nan_mask), st))
+        h = r = blocks.init_conv(packed)
         del packed
-        r = h
-        if return_taps:
-            if temb is not None:
-                taps["temb"] = temb
-            taps["init_conv"] = h
+        blocks.tap("init_conv", h)
 
         skips: List[Tensor] = []
         n_levels = len(self.downs)
-        for i, (b1, b2, attn, down) in enumerate(self.downs):
-            h = self._resnet(f"downs.{i}.0", b1, h, None, ss)
+        for i, (b1, b2, attn, _) in enumerate(self.downs):
+            if i >= 2:
+                blocks.group(f"downs.{i}")
+            h = blocks.resnet(f"downs.{i}.0", b1, h, None, ss)
             skips.append(h)
-            if return_taps and i == 0:
-                taps["downs.0.0"] = h
-            h = self._resnet(f"downs.{i}.1", b2, h, None, ss)
-            h = self._linear_attention(f"downs.{i}.2", attn, h)
-            if return_taps and i == 0:
-                taps["downs.0.2"] = h
+            if i == 0:
+                blocks.tap("downs.0.0", h)
+            h = blocks.resnet(f"downs.{i}.1", b2, h, None, ss)
+            h = blocks.linear_attention(f"downs.{i}.2", attn, h)
+            if i == 0:
+                blocks.tap("downs.0.2", h)
             skips.append(h)
-            h = self._conv(f"downs.{i}.3", h)
-        h = self._resnet("mid_block1", self.mid_block1, h, None, ss)
-        if return_taps:
-            taps["mid_block1"] = h
-        h = self._attention("mid_attn", self.mid_attn, h)
-        if return_taps:
-            taps["mid_attn"] = h
-        h = self._resnet("mid_block2", self.mid_block2, h, None, ss)
-        for i, (b1, b2, attn, up) in enumerate(self.ups):
-            h = self._resnet(f"ups.{i}.0", b1, h, skips.pop(), ss)
-            h = self._resnet(f"ups.{i}.1", b2, h, skips.pop(), ss)
-            h = self._linear_attention(f"ups.{i}.2", attn, h)
-            if i < n_levels - 1:
-                n_, hh, ww, cc = h.shape
-                pc = self._convs[f"ups.{i}.3"]
-                up_o = torch.empty(n_, 2 * hh, 2 * ww, pc.cout, device=dev, dtype=BF16)
-                timing = getattr(self, "_conv_timing", None)
-                if timing is not None:       # (algorithmic FLOPs of the reference's conv on the up-sampled tensor)
-                    ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
-                    timing.append((f"ups.{i}.3", 2.0 * n_ * 4 * hh * ww * pc.cout * 9 * cc, ev))
-                    ev[0].record()
-                _lib.check(lib.fd_conv_igemm_up(_lib.ptr(h), cc, _lib.ptr(self._up_w[i]), _lib.ptr(pc.bias), _lib.ptr(up_o), n_, hh, ww,
-                                                pc.cout, st))
-                if timing is not None:
-                    ev[1].record()
-                h = up_o
-            else:
-                h = self._conv(f"ups.{i}.3", h)
-        fc = self.final_conv
-        if (not return_taps and self.dim == 64 and self.out_dim <= 4 and
-                "final_res_block.res_conv" in self._convs and self._convs["final_res_block.res_conv"].kh == 1):
+            h = blocks.conv(f"downs.{i}.3", h)
+        blocks.group("mid")
+        h = blocks.resnet("mid_block1", self.mid_block1, h, None, ss)
+        blocks.tap("mid_block1", h)
+        h = blocks.attention("mid_attn", self.mid_attn, h)
+        blocks.tap("mid_attn", h)
+        h = blocks.resnet("mid_block2", self.mid_block2, h, None, ss)
+        for i, (b1, b2, attn, _) in enumerate(self.ups):
+            if i <= 2:
+                blocks.group(("ups.0", "ups.1", "ups.23")[i])
+            h = blocks.resnet(f"ups.{i}.0", b1, h, skips.pop(), ss)
+            h = blocks.resnet(f"ups.{i}.1", b2, h, skips.pop(), ss)
+            h = blocks.linear_attention(f"ups.{i}.2", attn, h)
+            h = blocks.upsample(i, h) if i < n_levels - 1 else blocks.conv(f"ups.{i}.3", h)
+        blocks.group("final")
+        out = blocks.final(h, r, ss, (H0, W0, pt, pl))
+        self._stats = None
+        return out
+
+
+class _InferBlocks:
+    """``Unet._walk``'s blocks for the inference forward (sampling, validation): the fused kernels.  ``taps`` is None, or
+    the dict that collects ``return_taps``' activations."""
+
+    def __init__(self, unet: Unet, taps: Optional[Dict[str, Tensor]]):
+        self.unet, self.taps = unet, taps
+        self.init_conv = partial(unet._conv, "init_conv")
+        self.conv, self.resnet, self.upsample = unet._conv, unet._resnet, unet._upsample
+        self.linear_attention, self.attention = unet._linear_attention, unet._attention
+
+    def group(self, name: str):
+        pass
+
+    def tap(self, name: str, h: Tensor):
+        if self.taps is not None:
+            self.taps[name] = h
+
+    def time_embedding(self, time: Tensor) -> Tensor:
+        u = self.unet
+        tm = u.time_mlp
+        temb = torch.empty(time.shape[0], u.time_dim, device=time.device, dtype=torch.float32)
+        _lib.check(u._lib.fd_time_embed(_lib.ptr(time), _lib.ptr(tm[1].weight), _lib.ptr(tm[1].bias), _lib.ptr(tm[3].weight),
+                                        _lib.ptr(tm[3].bias), _lib.ptr(temb), time.shape[0], u.dim, u.time_dim, u._st))
+        return temb
+
+    def final(self, h: Tensor, r: Tensor, ss: Optional[Tensor], frame: Tuple[int, int, int, int]) -> Tensor:
+        u = self.unet
+        if (self.taps is None and u.dim == 64 and u.out_dim <= 4 and
+                "final_res_block.res_conv" in u._convs and u._convs["final_res_block.res_conv"].kh == 1):
             # final ResnetBlock's res_conv + residual + final_conv + crop in one launch: the last 64-channel activation
             # (461 MB at batch 8, 440x1024) is neither written nor re-read.  return_taps needs that activation: two launches
-            out = self._resnet("final_res_block", self.final_res_block, h, r, ss, head=(fc, H0, W0, pad[2], pad[0]))
-            self._stats = None
-            return out
-        h = self._resnet("final_res_block", self.final_res_block, h, r, ss)
-        if return_taps:
-            taps["final_res_block"] = h
-        out = torch.empty(B, self.out_dim, H0, W0, device=dev, dtype=torch.float32)
-        _lib.check(lib.fd_final_conv_crop(_lib.ptr(h), _lib.ptr(fc.weight), _lib.ptr(fc.bias), _lib.ptr(out), B, H, W, self.dim,
-                                          self.out_dim, pad[2], pad[0], H0, W0, st))
-        self._stats = None
-        if return_taps:
-            return out, {k: (v if v.dim() == 2 else v.permute(0, 3, 1, 2).float()) for k, v in taps.items()}
-        return out
+            return u._resnet("final_res_block", u.final_res_block, h, r, ss, head=(u.final_conv,) + frame)
+        h = u._resnet("final_res_block", u.final_res_block, h, r, ss)
+        self.tap("final_res_block", h)
+        return u._final_conv_crop(h, frame)

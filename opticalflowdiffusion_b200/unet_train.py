@@ -20,6 +20,7 @@ views of it, so ``p.grad`` is filled exactly as autograd would and any ``torch.o
 """
 from __future__ import annotations
 
+from functools import partial
 from typing import Callable, Dict, List, Optional
 
 import torch
@@ -75,6 +76,8 @@ class Tape:
         self.st = unet._st
         self.steps: List[Callable[[], None]] = []
         self.g: Dict[int, Tensor] = {}
+        self.temb: Optional[Tensor] = None      # time embedding and d(scale, shift) of every block (Unet(time_in=True))
+        self.dss: Optional[Tensor] = None
 
     def record(self, fn: Callable[[], None]):
         self.steps.append(fn)
@@ -272,7 +275,7 @@ class TrainMixin:
             if mod.bias is not None and stats is None:      # with statistics the GroupNorm backward delivers it
                 _lib.check(lib.fd_bias_grad(_lib.ptr(dy), _lib.ptr(gb.of(mod.bias)), n * h * w, cout, st))
             # packed weight gradient into this conv's slice of the workspace (zeroed at the start of the backward); the
-            # unpacking + weight-standardisation backward of ALL convs is one launch at the end (forward_train.backward)
+            # unpacking + weight-standardisation backward is one launch per gradient bucket (_t_group_boundary)
             gw = self._gw_ws["views"][name]
             _lib.check(lib.fd_conv_wgrad(_lib.ptr(src0), c0, _lib.ptr(src1), c1, _lib.ptr(dy), _lib.ptr(gw), n, h, w, cout,
                                          pc.kh, pc.kw, pc.pad[0], pc.pad[1], pc.mode, st))
@@ -342,9 +345,9 @@ class TrainMixin:
         tape.record(bwd)
         return out
 
-    def _t_resnet(self, tape: Tape, name: str, rb, x0: Tensor, x1: Optional[Tensor], ss: Tensor, dss: Tensor,
-                  need_dgrad: bool = True) -> Tensor:
+    def _t_resnet(self, tape: Tape, name: str, rb, x0: Tensor, x1: Optional[Tensor], ss: Optional[Tensor]) -> Tensor:
         st1, st2 = self._next_stats(), self._next_stats()
+        dss = tape.dss
         if rb.mlp is not None and ss is not None:
             lin, temb, gb, lib, st = rb.mlp[1], tape.temb, self._gb, self._lib, self._st
 
@@ -354,12 +357,11 @@ class TrainMixin:
                                                lin.weight.shape[0], self.time_dim, 1, st))
 
             tape.record(mlp_bwd)
-        h1 = self._t_conv(tape, name + ".block1.proj", x0, x1, stats=st1, need_dgrad=need_dgrad)
+        h1 = self._t_conv(tape, name + ".block1.proj", x0, x1, stats=st1)
         a1 = self._t_gn_silu(tape, h1, st1, rb.block1.norm, ss, dss, self._tproj_off[name], None, rb.block1.proj.bias)
         h2 = self._t_conv(tape, name + ".block2.proj", a1, stats=st2)
         if (name + ".res_conv") in self._convs:
-            return self._t_conv(tape, name + ".res_conv", x0, x1, need_dgrad=need_dgrad,
-                                res_gn=(h2, st2, rb.block2.norm, rb.block2.proj.bias))
+            return self._t_conv(tape, name + ".res_conv", x0, x1, res_gn=(h2, st2, rb.block2.norm, rb.block2.proj.bias))
         assert x1 is None
         return self._t_gn_silu(tape, h2, st2, rb.block2.norm, None, None, 0, x0, rb.block2.proj.bias)
 
@@ -406,147 +408,105 @@ class TrainMixin:
         tape.record(bwd)
         return self._t_conv(tape, name + ".to_out", att, residual=x)
 
+    def _t_upsample(self, tape: Tape, i: int, x: Tensor) -> Tensor:
+        """Upsample ``ups.{i}.3`` (:89-93) as nearest x2 (fd_upsample2x) + the 3x3 conv on the up-sampled tensor."""
+        lib, st = self._lib, self._st
+        n, h, w, c = x.shape
+        up = torch.empty(n, 2 * h, 2 * w, c, device=x.device, dtype=BF16)
+        _lib.check(lib.fd_upsample2x(_lib.ptr(x), _lib.ptr(up), n, h, w, c, st))
+
+        def bwd():
+            d = tape.pop(up)
+            dx = torch.empty_like(x)
+            _lib.check(lib.fd_upsample2x_bwd(_lib.ptr(d), _lib.ptr(dx), n, h, w, c, st))
+            tape.add_grad(x, dx)
+
+        tape.record(bwd)
+        return self._t_conv(tape, f"ups.{i}.3", up)
+
     # ------------------------------------------------------------------ forward (training)
     def forward_train(self, x: Tensor, external_cond: Optional[Tensor], time: Tensor, nan_mask: bool = False):
         """``Unet.forward`` keeping the tape.  Returns ``(out, backward)`` where ``backward(dout)`` accumulates every
         parameter gradient into ``self.grad_buffer`` (caller zero-fills) and returns nothing: the network input
         (noised target + conditioning frames) carries no gradient in the reference's training step."""
-        _lib.require_cuda(x, external_cond, time)
-        if self.time_in and time is None:
-            raise ValueError("when Unet takes time arg, time argument must be passed in")
-        self.prepare()
-        self._lib = _lib.load()
-        self._st = _lib.stream()
+        self._begin(x, external_cond, time)
         self._prepare_dgrad()
         self._grad_buffer()
-        lib, st = self._lib, self._st
-        B, Cx, H0, W0 = x.shape
-        Cc = external_cond.shape[1] if external_cond is not None else 0
-        assert Cx + int(nan_mask) + Cc == self.channels, (Cx, nan_mask, Cc, self.channels)
-        dev = x.device
-        x = x.detach().float()
-        cond = external_cond.detach().float() if external_cond is not None else None
-        ph, pw = (-H0) % 8, (-W0) % 8
-        pad = (pw // 2, pw - pw // 2, ph // 2, ph - ph // 2)
-        if ph or pw:
-            x = torch.nn.functional.pad(x, pad, mode="replicate")
-            if cond is not None:
-                cond = torch.nn.functional.pad(cond, pad, mode="replicate")
-        x = x.contiguous()
-        cond = cond.contiguous() if cond is not None else None
-        H, W = H0 + ph, W0 + pw
-        tape = Tape(self)
-        gb = self._gb
-        ss = dss = None
-        self._t_group_boundary(tape, "front")        # first record = last to run: after init_conv and the time MLP
-        if self.time_in:
-            time = time.to(torch.int64).contiguous()
+        blocks = _TrainBlocks(self)
+        return self._walk(blocks, x, external_cond, time, nan_mask), blocks.backward
 
-            temb = torch.empty(B, self.time_dim, device=dev, dtype=torch.float32)
-            pe = torch.empty(B, self.dim, device=dev, dtype=torch.float32)
-            pre = torch.empty(B, self.time_dim, device=dev, dtype=torch.float32)
-            tm = self.time_mlp
-            _lib.check(lib.fd_time_embed_save(_lib.ptr(time), _lib.ptr(tm[1].weight), _lib.ptr(tm[1].bias), _lib.ptr(tm[3].weight),
-                                              _lib.ptr(tm[3].bias), _lib.ptr(temb), _lib.ptr(pe), _lib.ptr(pre), B, self.dim,
-                                              self.time_dim, st))
-            J = self._tproj_w.shape[0]
-            ss = torch.empty(B, J, device=dev, dtype=torch.float32)
-            dss = torch.zeros(B, J, device=dev, dtype=torch.float32)
-            _lib.check(lib.fd_time_proj(_lib.ptr(temb), _lib.ptr(self._tproj_w), _lib.ptr(self._tproj_b), _lib.ptr(ss), B,
-                                        self.time_dim, J, st))
 
-            tape.temb = temb
+class _TrainBlocks:
+    """``Unet._walk``'s blocks for the training forward: every op records its backward on ``tape``, and the gradient
+    buckets (``TrainMixin.GRAD_GROUPS``) start at ``group``."""
 
-            def time_bwd():
-                # (each ResnetBlock's mlp Linear gradient was taken inside its own block: _t_resnet.mlp_bwd)
-                td = self.time_dim
-                dtemb = torch.empty(B, td, device=dev, dtype=torch.float32)
-                _lib.check(lib.fd_linear_bwd_x(_lib.ptr(dss), J, _lib.ptr(self._tproj_w), _lib.ptr(temb), td, _lib.ptr(dtemb), td,
-                                               B, J, td, 1, st))
-                _lib.check(lib.fd_linear_bwd_w(_lib.ptr(dtemb), td, _lib.ptr(pre), td, _lib.ptr(gb.of(tm[3].weight)),
-                                               _lib.ptr(gb.of(tm[3].bias)), B, td, td, 2, st))
-                dpre = torch.empty(B, td, device=dev, dtype=torch.float32)
-                _lib.check(lib.fd_linear_bwd_x(_lib.ptr(dtemb), td, _lib.ptr(tm[3].weight), _lib.ptr(pre), td, _lib.ptr(dpre), td,
-                                               B, td, td, 2, st))
-                _lib.check(lib.fd_linear_bwd_w(_lib.ptr(dpre), td, _lib.ptr(pe), self.dim, _lib.ptr(gb.of(tm[1].weight)),
-                                               _lib.ptr(gb.of(tm[1].bias)), B, td, self.dim, 0, st))
+    def __init__(self, unet):
+        self.unet, self.gb = unet, unet._gb
+        tape = self.tape = Tape(unet)
+        self.group = partial(unet._t_group_boundary, tape)
+        self.init_conv = partial(unet._t_conv, tape, "init_conv", need_dgrad=False)    # the network input takes no gradient
+        self.conv = partial(unet._t_conv, tape)
+        self.resnet = partial(unet._t_resnet, tape)
+        self.linear_attention = partial(unet._t_linear_attention, tape)
+        self.attention = partial(unet._t_attention, tape)
+        self.upsample = partial(unet._t_upsample, tape)
 
-            tape.record(time_bwd)          # runs last: every block's d(scale, shift) is in dss by then
+    def tap(self, name: str, h: Tensor):
+        pass
 
-        self._stats = torch.zeros(2 * len(self._resblocks), B, 8, 2, device=dev, dtype=torch.float64)
-        self._stats_i = 0
-        packed = torch.empty(B, H, W, 64, device=dev, dtype=BF16)
-        if self._wide_input:
-            _lib.check(lib.fd_pack_input_wide(_lib.ptr(x), _lib.ptr(cond), _lib.ptr(packed), B, Cx, Cc, H, W, 0, 0, H, W,
-                                              int(nan_mask), st))
-        else:
-            _lib.check(lib.fd_pack_input(_lib.ptr(x), _lib.ptr(cond), _lib.ptr(packed), B, Cx, Cc, H, W, int(nan_mask), st))
-        h = self._t_conv(tape, "init_conv", packed, need_dgrad=False)
-        r = h
-        skips: List[Tensor] = []
-        n_levels = len(self.downs)
-        for i, (b1, b2, attn, down) in enumerate(self.downs):
-            if i >= 2:
-                self._t_group_boundary(tape, f"downs.{i}")
-            h = self._t_resnet(tape, f"downs.{i}.0", b1, h, None, ss, dss)
-            skips.append(h)
-            h = self._t_resnet(tape, f"downs.{i}.1", b2, h, None, ss, dss)
-            h = self._t_linear_attention(tape, f"downs.{i}.2", attn, h)
-            skips.append(h)
-            h = self._t_conv(tape, f"downs.{i}.3", h)
-        self._t_group_boundary(tape, "mid")
-        h = self._t_resnet(tape, "mid_block1", self.mid_block1, h, None, ss, dss)
-        h = self._t_attention(tape, "mid_attn", self.mid_attn, h)
-        h = self._t_resnet(tape, "mid_block2", self.mid_block2, h, None, ss, dss)
-        for i, (b1, b2, attn, up) in enumerate(self.ups):
-            if i <= 2:
-                self._t_group_boundary(tape, ("ups.0", "ups.1", "ups.23")[i])
-            h = self._t_resnet(tape, f"ups.{i}.0", b1, h, skips.pop(), ss, dss)
-            h = self._t_resnet(tape, f"ups.{i}.1", b2, h, skips.pop(), ss, dss)
-            h = self._t_linear_attention(tape, f"ups.{i}.2", attn, h)
-            if i < n_levels - 1:
-                n_, hh, ww, cc = h.shape
-                up_t = torch.empty(n_, 2 * hh, 2 * ww, cc, device=dev, dtype=BF16)
-                _lib.check(lib.fd_upsample2x(_lib.ptr(h), _lib.ptr(up_t), n_, hh, ww, cc, st))
+    def time_embedding(self, time: Tensor) -> Tensor:
+        u, tape, gb = self.unet, self.tape, self.gb
+        lib, st = tape.lib, tape.st
+        B, td, dev = time.shape[0], u.time_dim, time.device
+        tm = u.time_mlp
+        temb = torch.empty(B, td, device=dev, dtype=torch.float32)
+        pe = torch.empty(B, u.dim, device=dev, dtype=torch.float32)
+        pre = torch.empty(B, td, device=dev, dtype=torch.float32)
+        _lib.check(lib.fd_time_embed_save(_lib.ptr(time), _lib.ptr(tm[1].weight), _lib.ptr(tm[1].bias), _lib.ptr(tm[3].weight),
+                                          _lib.ptr(tm[3].bias), _lib.ptr(temb), _lib.ptr(pe), _lib.ptr(pre), B, u.dim, td, st))
+        J = u._tproj_w.shape[0]
+        dss = torch.zeros(B, J, device=dev, dtype=torch.float32)
+        tape.temb, tape.dss = temb, dss
 
-                def up_bwd(h=h, up_t=up_t, n_=n_, hh=hh, ww=ww, cc=cc):
-                    d = tape.pop(up_t)
-                    dx = torch.empty_like(h)
-                    _lib.check(lib.fd_upsample2x_bwd(_lib.ptr(d), _lib.ptr(dx), n_, hh, ww, cc, st))
-                    tape.add_grad(h, dx)
+        def time_bwd():
+            # (each ResnetBlock's mlp Linear gradient was taken inside its own block: _t_resnet.mlp_bwd)
+            dtemb = torch.empty(B, td, device=dev, dtype=torch.float32)
+            _lib.check(lib.fd_linear_bwd_x(_lib.ptr(dss), J, _lib.ptr(u._tproj_w), _lib.ptr(temb), td, _lib.ptr(dtemb), td,
+                                           B, J, td, 1, st))
+            _lib.check(lib.fd_linear_bwd_w(_lib.ptr(dtemb), td, _lib.ptr(pre), td, _lib.ptr(gb.of(tm[3].weight)),
+                                           _lib.ptr(gb.of(tm[3].bias)), B, td, td, 2, st))
+            dpre = torch.empty(B, td, device=dev, dtype=torch.float32)
+            _lib.check(lib.fd_linear_bwd_x(_lib.ptr(dtemb), td, _lib.ptr(tm[3].weight), _lib.ptr(pre), td, _lib.ptr(dpre), td,
+                                           B, td, td, 2, st))
+            _lib.check(lib.fd_linear_bwd_w(_lib.ptr(dpre), td, _lib.ptr(pe), u.dim, _lib.ptr(gb.of(tm[1].weight)),
+                                           _lib.ptr(gb.of(tm[1].bias)), B, td, u.dim, 0, st))
 
-                tape.record(up_bwd)
-                h = self._t_conv(tape, f"ups.{i}.3", up_t)
-                del up_t
-            else:
-                h = self._t_conv(tape, f"ups.{i}.3", h)
-        self._t_group_boundary(tape, "final")
-        h = self._t_resnet(tape, "final_res_block", self.final_res_block, h, r, ss, dss)
-        out = torch.empty(B, self.out_dim, H, W, device=dev, dtype=torch.float32)
-        fc = self.final_conv
-        _lib.check(lib.fd_final_conv(_lib.ptr(h), _lib.ptr(fc.weight), _lib.ptr(fc.bias), _lib.ptr(out), B, H * W, self.dim,
-                                     self.out_dim, st))
-        h_last = h
-        self._stats = None
+        tape.record(time_bwd)          # runs after every block's backward has written its d(scale, shift) into dss
+        return temb
 
-        def backward(dout: Tensor):
-            _lib.require_cuda(dout)
-            dout = dout.float()
-            if ph or pw:
-                dout = torch.nn.functional.pad(dout, pad)        # the cropped border received no gradient
-            dout = dout.contiguous()
-            dh = torch.empty_like(h_last)
-            _lib.check(lib.fd_final_conv_bwd(_lib.ptr(h_last), _lib.ptr(fc.weight), _lib.ptr(dout), _lib.ptr(dh),
-                                             _lib.ptr(gb.of(fc.weight)), _lib.ptr(gb.of(fc.bias)), B, H * W, self.dim,
-                                             self.out_dim, st))
-            tape.g[id(h_last)] = dh
-            ws = self._wgrad_workspace()
-            ws["flat"].zero_()
-            tape.run()          # the group boundaries unpack the packed weight gradients bucket by bucket (_t_group_boundary)
+    def final(self, h: Tensor, r: Tensor, ss: Optional[Tensor], frame) -> Tensor:
+        u = self.unet
+        self.h_last = u._t_resnet(self.tape, "final_res_block", u.final_res_block, h, r, ss)
+        self.frame = frame
+        return u._final_conv_crop(self.h_last, frame)
 
-        if ph or pw:
-            out = out[:, :, pad[2]:pad[2] + H0, pad[0]:pad[0] + W0].contiguous()
-        return out, backward
+    def backward(self, dout: Tensor):
+        u, tape, gb, h = self.unet, self.tape, self.gb, self.h_last
+        fc = u.final_conv
+        B, H, W, _ = h.shape
+        H0, W0, pt, pl = self.frame
+        _lib.require_cuda(dout)
+        dout = dout.float()
+        if (H0, W0) != (H, W):
+            dout = torch.nn.functional.pad(dout, (pl, W - W0 - pl, pt, H - H0 - pt))     # the cropped border received no gradient
+        dout = dout.contiguous()
+        dh = torch.empty_like(h)
+        _lib.check(tape.lib.fd_final_conv_bwd(_lib.ptr(h), _lib.ptr(fc.weight), _lib.ptr(dout), _lib.ptr(dh),
+                                              _lib.ptr(gb.of(fc.weight)), _lib.ptr(gb.of(fc.bias)), B, H * W, u.dim, u.out_dim,
+                                              tape.st))
+        tape.g[id(h)] = dh
+        u._wgrad_workspace()["flat"].zero_()
+        tape.run()          # the group boundaries unpack the packed weight gradients bucket by bucket (_t_group_boundary)
 
 
 class UnetFunction(torch.autograd.Function):

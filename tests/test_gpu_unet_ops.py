@@ -113,8 +113,8 @@ def test_time_embed_and_proj(L):
 
 
 @pytest.mark.parametrize("nan_mask", [False, True])
-def test_pack_input_and_init_conv_weights(L, nan_mask):
-    """pack_input + kind-2 weight packing + 7x1 implicit GEMM == 7x7 conv (denoising_diffusion.py:297)."""
+def test_pack_input_pad_unpadded_and_init_conv_weights(L, nan_mask):
+    """pack_input_pad with zero padding + kind-2 weight packing + 7x1 implicit GEMM == 7x7 conv (denoising_diffusion.py:297)."""
     lib = L.load()
     g = torch.Generator().manual_seed(9)
     B, Cx, Cc, H, W = 2, 5 if nan_mask else 2, 3, 16, 24
@@ -128,7 +128,8 @@ def test_pack_input_and_init_conv_weights(L, nan_mask):
     bias = torch.randn(64, generator=g)
     packed = torch.empty(B, H, W, 64, device="cuda", dtype=BF)
     xc, cc, wc, bc = x.cuda(), cond.cuda(), w.cuda(), bias.cuda()
-    L.check(lib.fd_pack_input(L.ptr(xc), L.ptr(cc), L.ptr(packed), B, Cx, Cc, H, W, int(nan_mask), L.stream()))
+    L.check(lib.fd_pack_input_pad(L.ptr(xc), L.ptr(cc), L.ptr(packed), B, Cx, Cc, H, W, 0, 0, H, W, int(nan_mask),
+                                  L.stream()))
     wp = torch.empty(64, 7 * 64, device="cuda", dtype=BF)
     L.check(lib.fd_prep_weight(L.ptr(wc), L.ptr(wp), 64, Ctot, 7, 7, 2, 0, 0.0, L.stream()))
     out = torch.empty(B, H, W, 64, device="cuda", dtype=BF)
@@ -166,14 +167,15 @@ def test_prep_weight_standardize(L, kind):
     assert torch.allclose(out.float().cpu(), ref.to(BF).float(), rtol=1e-2, atol=1e-3)
 
 
-def test_final_conv(L):
+def test_final_conv_crop_full_window(L):
+    """final_conv_crop whose window is the whole frame == the plain 1x1 conv."""
     lib = L.load()
     g = torch.Generator().manual_seed(2)
     x = torch.randn(2, 64, 6, 9, generator=g).to(BF).float().cuda()
     w, b = torch.randn(2, 64, 1, 1, generator=g).cuda(), torch.randn(2, generator=g).cuda()
     out = torch.empty(2, 2, 6, 9, device="cuda")
     xh = nhwc(x)
-    L.check(lib.fd_final_conv(L.ptr(xh), L.ptr(w), L.ptr(b), L.ptr(out), 2, 54, 64, 2, L.stream()))
+    L.check(lib.fd_final_conv_crop(L.ptr(xh), L.ptr(w), L.ptr(b), L.ptr(out), 2, 6, 9, 64, 2, 0, 0, 6, 9, L.stream()))
     assert torch.allclose(out, F.conv2d(x, w, b), rtol=1e-4, atol=1e-4)
 
 
