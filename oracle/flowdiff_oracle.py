@@ -75,18 +75,20 @@ def _resnet_block(sd, p: str, x: Tensor, temb: Optional[Tensor]) -> Tensor:
     return h + x
 
 
-def _chan_layernorm(x: Tensor, g: Tensor) -> Tensor:
-    """LayerNorm.forward, denoising_diffusion.py:121-125 (over channels, biased var, gain only)."""
-    eps = 1e-5 if x.dtype == torch.float32 else 1e-3
+def _chan_layernorm(x: Tensor, g: Tensor, eps: Optional[float] = None) -> Tensor:
+    """LayerNorm.forward, denoising_diffusion.py:121-125 (over channels, biased var, gain only).  ``eps`` defaults to the
+    reference's choice by dtype (1e-5 for fp32, 1e-3 otherwise); a float64 restatement of the fp32 model passes 1e-5."""
+    if eps is None:
+        eps = 1e-5 if x.dtype == torch.float32 else 1e-3
     var = torch.var(x, dim=1, unbiased=False, keepdim=True)
     mean = torch.mean(x, dim=1, keepdim=True)
     return (x - mean) * (var + eps).rsqrt() * g
 
 
-def _linear_attention(sd, p: str, x: Tensor, heads: int = 4, dim_head: int = 32) -> Tensor:
+def _linear_attention(sd, p: str, x: Tensor, heads: int = 4, dim_head: int = 32, eps: Optional[float] = None) -> Tensor:
     """Residual(PreNorm(LinearAttention)), denoising_diffusion.py:81-87,127-135,229-244."""
     b, c, h, w = x.shape
-    y = _chan_layernorm(x, sd[p + "norm.g"])
+    y = _chan_layernorm(x, sd[p + "norm.g"], eps)
     qkv = F.conv2d(y, sd[p + "fn.to_qkv.weight"])
     q, k, v = (t.reshape(b, heads, dim_head, h * w) for t in qkv.chunk(3, dim=1))
     q = q.softmax(dim=-2) * dim_head ** -0.5
@@ -95,7 +97,7 @@ def _linear_attention(sd, p: str, x: Tensor, heads: int = 4, dim_head: int = 32)
     ctx = torch.einsum("bhdn,bhen->bhde", k, v)
     out = torch.einsum("bhde,bhdn->bhen", ctx, q).reshape(b, heads * dim_head, h, w)
     out = F.conv2d(out, sd[p + "fn.to_out.0.weight"], sd[p + "fn.to_out.0.bias"])
-    out = _chan_layernorm(out, sd[p + "fn.to_out.1.g"])
+    out = _chan_layernorm(out, sd[p + "fn.to_out.1.g"], eps)
     return out + x
 
 
