@@ -396,6 +396,14 @@ FD_API int fd_sumsq(const float* g, long n, float* out, void* stream);
 FD_API int fd_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, long n, float lr,
                  float beta1, float beta2, float eps, float weight_decay, int step, const float* grad_sumsq,
                  float max_norm, float grad_scale, void* stream);
+/* fd_adam_step plus an exponential moving average of the weights in the same pass (param, exp_avg and exp_avg_sq are
+ * bitwise what fd_adam_step writes).  With p the updated parameter and w = ema_weight in [0, 1] (torch.lerp's form, so
+ * w = 1 copies p exactly):
+ *   ema = w >= 0.5 ? p - (p - ema) * (1 - w) : ema + w * (p - ema)
+ * 36 bytes of traffic per parameter instead of 28. */
+FD_API int fd_adam_ema_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, float* ema, long n,
+                     float lr, float beta1, float beta2, float eps, float weight_decay, int step,
+                     const float* grad_sumsq, float max_norm, float grad_scale, float ema_weight, void* stream);
 
 /* ---- training augmentation on the GPU: augmentation.py:6-76 (torchvision ColorJitter / Grayscale / GaussianBlur(3) /
  *      flips / RandomResizedCrop, applied item by item in the reference).  fp32 NCHW images in [0,1].

@@ -99,6 +99,7 @@ SIGNATURES = {
     "fd_time_embed_save": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P]),
     "fd_sumsq": (c_int, [_P, _L, _P, _P]),
     "fd_adam_step": (c_int, [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _I, _P, _F, _F, _P]),
+    "fd_adam_ema_step": (c_int, [_P, _P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _I, _P, _F, _F, _F, _P]),
     "fd_aug_photometric": (c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _P]),
     "fd_aug_blur3": (c_int, [_P, _P, _P, _P, _I, _I, _I, _P]),
     "fd_aug_geometric": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P]),

@@ -723,10 +723,14 @@ __global__ void __launch_bounds__(256) sumsq_kernel(const float4* __restrict__ g
   if (threadIdx.x == 0) atomicAdd(out, s[0]);
 }
 
+// EMA = true also folds the weight EMA into the same pass: the freshly updated parameter is still in a register, so the
+// update costs the 8 bytes of reading and writing `ema` and no launch.  torch.lerp's two-branch form, so w = 1 copies.
+template <bool EMA>
 __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
-                                                   float* __restrict__ v, long n, float lr, float b1, float b2, float eps,
-                                                   float wd, float bc1, float bc2_sqrt, const float* __restrict__ sumsq,
-                                                   float max_norm, float grad_scale) {
+                                                   float* __restrict__ v, float* __restrict__ ema, long n, float lr, float b1,
+                                                   float b2, float eps, float wd, float bc1, float bc2_sqrt,
+                                                   const float* __restrict__ sumsq, float max_norm, float grad_scale,
+                                                   float ema_w) {
   float clip = grad_scale;
   if (sumsq != nullptr && max_norm > 0.f) {
     const float norm = sqrtf(*sumsq) * grad_scale;
@@ -740,7 +744,12 @@ __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const 
     const float vi = b2 * v[i] + (1.f - b2) * gi * gi;
     m[i] = mi;
     v[i] = vi;
-    p[i] = pi - (lr / bc1) * mi / (sqrtf(vi) / bc2_sqrt + eps);
+    const float pn = pi - (lr / bc1) * mi / (sqrtf(vi) / bc2_sqrt + eps);
+    p[i] = pn;
+    if constexpr (EMA) {
+      const float e = ema[i];
+      ema[i] = ema_w >= 0.5f ? pn - (pn - e) * (1.f - ema_w) : e + ema_w * (pn - e);
+    }
   }
 }
 
@@ -918,9 +927,23 @@ int fd_adam_step(float* param, const float* grad, float* exp_avg, float* exp_avg
   FD_REQUIRE(param && grad && exp_avg && exp_avg_sq && n > 0 && step >= 1, "adam_step: bad argument");
   const float bc1 = 1.f - powf(beta1, (float)step);
   const float bc2 = 1.f - powf(beta2, (float)step);
-  adam_kernel<<<egrid(n, 256, 8), 256, 0, (cudaStream_t)stream>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps,
-                                                                 weight_decay, bc1, sqrtf(bc2), grad_sumsq, max_norm,
-                                                                 grad_scale);
+  adam_kernel<false><<<egrid(n, 256, 8), 256, 0, (cudaStream_t)stream>>>(param, grad, exp_avg, exp_avg_sq, nullptr, n, lr,
+                                                                        beta1, beta2, eps, weight_decay, bc1, sqrtf(bc2),
+                                                                        grad_sumsq, max_norm, grad_scale, 0.f);
+  FD_LAUNCH_CHECK();
+  return FD_OK;
+}
+
+int fd_adam_ema_step(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, float* ema, long n, float lr,
+                     float beta1, float beta2, float eps, float weight_decay, int step, const float* grad_sumsq,
+                     float max_norm, float grad_scale, float ema_weight, void* stream) {
+  FD_REQUIRE(param && grad && exp_avg && exp_avg_sq && ema && n > 0 && step >= 1, "adam_ema_step: bad argument");
+  FD_REQUIRE(ema_weight >= 0.f && ema_weight <= 1.f, "adam_ema_step: ema_weight %g outside [0, 1]", (double)ema_weight);
+  const float bc1 = 1.f - powf(beta1, (float)step);
+  const float bc2 = 1.f - powf(beta2, (float)step);
+  adam_kernel<true><<<egrid(n, 256, 8), 256, 0, (cudaStream_t)stream>>>(param, grad, exp_avg, exp_avg_sq, ema, n, lr, beta1,
+                                                                       beta2, eps, weight_decay, bc1, sqrtf(bc2), grad_sumsq,
+                                                                       max_norm, grad_scale, ema_weight);
   FD_LAUNCH_CHECK();
   return FD_OK;
 }

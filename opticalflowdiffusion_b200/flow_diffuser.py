@@ -8,7 +8,9 @@ experiment runner that drives the reference class (experiments/exp_base.py:120-2
 
 New optional config keys (SURVEY.md section 8b): ``sampling_timesteps`` (DDIM when < ``timesteps``),
 ``image_size`` as ``[H, W]``, ``return_all_timesteps`` (default true like the reference), ``sampler`` (null: the
-reference's DDIM / DDPM; ``dpmpp``: multistep DPM-Solver++ on the DDIM grid) with ``solver_order`` (1-3).
+reference's DDIM / DDPM; ``dpmpp``: multistep DPM-Solver++ on the DDIM grid) with ``solver_order`` (1-3), and
+``ema_decay`` (null: off) with ``ema_update_after_step`` / ``ema_update_every``: an exponential moving average of the UNet
+weights (``ema_unet``), kept by the fused optimiser step and used for sampling and validation.
 
 When ``pytorch_lightning`` is importable the class derives from ``LightningModule``; otherwise from a
 minimal stand-in with the attributes the reference touches (``log_dict``, ``log``, ``global_step``,
@@ -16,6 +18,7 @@ minimal stand-in with the attributes the reference touches (``log_dict``, ``log`
 """
 from __future__ import annotations
 
+import copy
 import os
 import random
 from typing import Optional, Sequence, Tuple
@@ -209,11 +212,25 @@ class FlowDiffuser(_Base):
         # (flow_diffuser.py:122: in latent mode the reference passes latent_dim whatever the target -- kept: it is the channel
         # count of the sampler's initial noise, so latent sampling works for target='target' exactly as far as it does there)
         channels = cfg.latent_dim if self.latent else 2 + int(self.target == "target") + 3 * int(self.target == "joint")
-        self.model = ConditionalDiffusion(
-            self._model, _cfg_get(cfg, "image_size", 128), objective="pred_x0", channels=channels, auto_normalize=False,
-            noise_space="image" if cfg.noiser == "image" else "flow", timesteps=cfg.timesteps,
-            sampling_timesteps=_cfg_get(cfg, "sampling_timesteps"), min_snr_loss_weight=True,
-            sampler=_cfg_get(cfg, "sampler"), solver_order=int(_cfg_get(cfg, "solver_order", 2)))
+
+        def diffusion(net):
+            return ConditionalDiffusion(
+                net, _cfg_get(cfg, "image_size", 128), objective="pred_x0", channels=channels, auto_normalize=False,
+                noise_space="image" if cfg.noiser == "image" else "flow", timesteps=cfg.timesteps,
+                sampling_timesteps=_cfg_get(cfg, "sampling_timesteps"), min_snr_loss_weight=True,
+                sampler=_cfg_get(cfg, "sampler"), solver_order=int(_cfg_get(cfg, "solver_order", 2)))
+
+        self.model = diffusion(self._model)
+        ema_decay = _cfg_get(cfg, "ema_decay")
+        self.ema_decay = None if ema_decay is None else float(ema_decay)
+        if self.ema_decay is not None:
+            # the averaged UNet: registered (its 276 tensors ride in state_dict as ema_unet.*) but outside self.model, so
+            # the optimiser never sees it.  Its sampler is NOT registered (no state_dict keys); ema_model points its schedule
+            # tables at self.model's, and it keeps its own CUDA-graph cache.
+            self.ema_unet = copy.deepcopy(self.unet).requires_grad_(False)
+            net = UnetWithWarp(cfg, self.ema_unet, full_output=self.target == "joint") \
+                if self.target in ("target", "joint") else self.ema_unet
+            object.__setattr__(self, "_ema_diffusion", diffusion(net))
         self.return_all_timesteps = bool(_cfg_get(cfg, "return_all_timesteps", True))
         self.use_cuda_graph = bool(_cfg_get(cfg, "use_cuda_graph", False))
 
@@ -229,18 +246,44 @@ class FlowDiffuser(_Base):
                 self._augmentor = Augmentor()
         return self._augmentor
 
+    @property
+    def ema_model(self) -> ConditionalDiffusion:
+        """The ``ConditionalDiffusion`` over the EMA network (``ema_decay`` set), sharing ``self.model``'s schedule tables
+        wherever the module has been moved."""
+        if self.ema_decay is None:
+            raise ValueError("this FlowDiffuser keeps no weight EMA (algorithm.ema_decay is null)")
+        ema = self.__dict__["_ema_diffusion"]
+        for name in ConditionalDiffusion.BUFFERS:
+            setattr(ema, name, getattr(self.model, name))
+        return ema
+
+    def _diffusion(self, use_ema: Optional[bool]) -> ConditionalDiffusion:
+        """None: the EMA network when there is one, else the online one."""
+        if use_ema is None:
+            use_ema = self.ema_decay is not None
+        return self.ema_model if use_ema else self.model
+
     def configure_optimizers(self):
         """flow_diffuser.py:129-134: Adam(lr, weight_decay) over the model's parameters -- here the fused flat-buffer
         implementation with the same update rule; ``clipping`` (experiment.training.clipping, exp_base.py:192) can be
-        folded into the step by setting ``optimizer.max_grad_norm``."""
+        folded into the step by setting ``optimizer.max_grad_norm``.  With ``ema_decay`` set the same step keeps
+        ``ema_unet`` as the weights' moving average."""
         from .optim import FusedAdam
+        ema = {}
+        if self.ema_decay is not None:
+            ema = dict(ema_params=list(self.ema_unet.parameters()), ema_decay=self.ema_decay,
+                       ema_update_after_step=int(_cfg_get(self.cfg, "ema_update_after_step", 100)),
+                       ema_update_every=int(_cfg_get(self.cfg, "ema_update_every", 10)))
 
         def invalidate():
             self.unet.weights_epoch += 1
+            if opt.ema_updated:
+                self.ema_unet.weights_epoch += 1
 
-        self.optimizers = FusedAdam(self.model.parameters(), lr=self.cfg.lr, weight_decay=self.cfg.weight_decay,
-                                    max_grad_norm=float(_cfg_get(self.cfg, "clipping", 0.0) or 0.0), on_step=invalidate)
-        return self.optimizers
+        opt = FusedAdam(self.model.parameters(), lr=self.cfg.lr, weight_decay=self.cfg.weight_decay,
+                        max_grad_norm=float(_cfg_get(self.cfg, "clipping", 0.0) or 0.0), on_step=invalidate, **ema)
+        self.optimizers = opt
+        return opt
 
     # ------------------------------------------------------------------ data
     def preprocess(self, batch, aug: bool = True):
@@ -263,25 +306,32 @@ class FlowDiffuser(_Base):
 
     # ------------------------------------------------------------------ loss / sampling
     def loss(self, tgt, cond, flow, override=None, **kw):
+        """The training loss, always of the online network."""
+        return self._loss(self.model, tgt, cond, flow, override, **kw)
+
+    def _loss(self, diffusion, tgt, cond, flow, override=None, **kw):
         if self.cfg.target == "target":
-            return self.model(tgt, external_cond=cond, additional_tgt=flow, additional_weight=self.cfg.flow_weight,
-                              model_out_override=override, **kw)
-        return self.model(tgt, external_cond=cond, model_out_override=override, **kw)
+            return diffusion(tgt, external_cond=cond, additional_tgt=flow, additional_weight=self.cfg.flow_weight,
+                             model_out_override=override, **kw)
+        return diffusion(tgt, external_cond=cond, model_out_override=override, **kw)
 
     @torch.no_grad()
-    def sample(self, cond, flow, **kw) -> Tuple[Tensor, Tensor]:
-        """flow_diffuser.py:189-215: (samples, flows); with ``return_all_timesteps`` the flows keep a time axis at dim 1."""
+    def sample(self, cond, flow, use_ema: Optional[bool] = None, **kw) -> Tuple[Tensor, Tensor]:
+        """flow_diffuser.py:189-215: (samples, flows); with ``return_all_timesteps`` the flows keep a time axis at dim 1.
+        ``use_ema``: None samples the EMA network when ``ema_decay`` is set and the online one otherwise; False always
+        the online network."""
+        model = self._diffusion(use_ema)
         bsz = flow.shape[0]
         all_t = self.return_all_timesteps
         if self.cfg.target == "target":
-            samples, flow = self.model.sample(batch_size=bsz, external_cond=cond, additional_tgt=flow,
-                                              return_all_timesteps=all_t, **kw)
+            samples, flow = model.sample(batch_size=bsz, external_cond=cond, additional_tgt=flow,
+                                         return_all_timesteps=all_t, **kw)
         elif self.cfg.target == "joint":
-            joint = self.model.sample(batch_size=bsz, external_cond=cond, return_all_timesteps=all_t, **kw)
+            joint = model.sample(batch_size=bsz, external_cond=cond, return_all_timesteps=all_t, **kw)
             samples, flow = (joint[:, :, :self.dim], joint[:, :, self.dim:]) if all_t else (joint[:, :self.dim], joint[:, self.dim:])
         else:
-            flow = self.model.sample(batch_size=bsz, external_cond=cond, return_all_timesteps=all_t,
-                                     use_cuda_graph=self.use_cuda_graph, **kw)
+            flow = model.sample(batch_size=bsz, external_cond=cond, return_all_timesteps=all_t,
+                                use_cuda_graph=self.use_cuda_graph, **kw)
             last = flow[:, -1] if all_t else flow
             samples = W.warp(cond[:, :self.dim], None, last.contiguous(), mode="forward")
         return samples, flow
@@ -300,10 +350,12 @@ class FlowDiffuser(_Base):
 
     @torch.no_grad()
     def validation_step(self, batch, batch_idx):
-        """flow_diffuser.py:237-349 (scalar metrics; image logging when a logger is attached)."""
+        """flow_diffuser.py:237-349 (scalar metrics; image logging when a logger is attached).  Every metric is of the EMA
+        network when ``ema_decay`` is set."""
         img, tgt, flow = batch
+        model = self._diffusion(None)
         tgt_, cond, flow_ = self.preprocess(batch, aug=False)
-        loss = self.loss(tgt_, cond, flow_)
+        loss = self._loss(model, tgt_, cond, flow_)
         keep = self.return_all_timesteps
         self.return_all_timesteps = True
         try:
@@ -326,8 +378,8 @@ class FlowDiffuser(_Base):
         if self.target in ("target", "joint"):
             warped = W.warp(cond[:, :self.dim], None, flow_ * self.flow_max, mode="forward")
             override = (warped, flow_) if self.target == "target" else (torch.cat((warped, flow_), dim=1), None)
-            metrics["val/ideal_loss"] = self.loss(tgt_, cond, flow_, override=override)
-            last = self.model.model(tgt_, cond, torch.zeros((img.shape[0],), device=img.device, dtype=torch.long), None,
+            metrics["val/ideal_loss"] = self._loss(model, tgt_, cond, flow_, override=override)
+            last = model.model(tgt_, cond, torch.zeros((img.shape[0],), device=img.device, dtype=torch.long), None,
                                     additional_out=True)[:, -2:]
             metrics["val/last_step"] = torch.nn.functional.mse_loss(last, flow_)
         self.log_dict(metrics, sync_dist=True)

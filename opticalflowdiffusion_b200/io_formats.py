@@ -8,6 +8,7 @@ reference:
 * Lightning-style checkpoints: ``{"state_dict": ...}`` whose keys carry the reference's triple aliasing of the UNet
   (``unet.*``, ``_model.*`` / ``_model.model.*``, ``model.model.*`` / ``model.model.model.*``, SURVEY.md section 5) plus
   the 13 schedule buffers -- ``load_checkpoint`` accepts any one alias family (or all), ``save_checkpoint`` writes all;
+  a model with a weight EMA adds ``ema_unet.*``;
 * ``SintelFlowDataset``: (frame_t, frame_t+1, flow_t) triples in the (img, tgt, flow) convention of FlowDiffuser.preprocess
   (flow_diffuser.py:136-168) from an MPI-Sintel tree at a configurable root (the reference hard-codes a private path).
 """
@@ -79,6 +80,7 @@ class InputPadder:
 # checkpoints
 # ------------------------------------------------------------------------------------------------
 _UNET_PREFIXES = ("model.model.model.", "_model.model.", "model.model.", "_model.", "unet.")
+_EMA_PREFIX = "ema_unet."
 
 
 def _split_unet_key(key: str, unet_keys) -> Optional[str]:
@@ -91,15 +93,21 @@ def _split_unet_key(key: str, unet_keys) -> Optional[str]:
 def load_checkpoint(algo, path_or_dict, strict: bool = True) -> Dict[str, List[str]]:
     """Load a Lightning ``.ckpt`` (or a bare state_dict) of the reference's FlowDiffuser into ``algo``.  The reference
     registers the same UNet under up to three names; a checkpoint that carries only one of them (e.g. after
-    ``rewrite_checkpoint_for_compatibility``) still loads.  Returns {"missing": [...], "unexpected": [...]}."""
+    ``rewrite_checkpoint_for_compatibility``) still loads.  Returns {"missing": [...], "unexpected": [...]}, plus:
+
+    * ``"ema_initialised"`` when ``algo`` keeps a weight EMA: True when the checkpoint has no ``ema_unet.*`` keys (every
+      reference checkpoint), so the EMA starts from the loaded UNet weights; False when the EMA was restored from it;
+    * ``"ignored"``: the ``ema_unet.*`` keys of a checkpoint loaded into a model without EMA (present only when any)."""
     ck = torch.load(path_or_dict, map_location="cpu", weights_only=False) if isinstance(path_or_dict, (str, os.PathLike)) \
         else path_or_dict
     sd = ck.get("state_dict", ck)
     own = algo.state_dict()
     unet_keys = set(algo.unet.state_dict().keys())
+    ema = getattr(algo, "ema_unet", None)
     unet_vals: Dict[str, torch.Tensor] = {}
     other: Dict[str, torch.Tensor] = {}
     unexpected: List[str] = []
+    ignored: List[str] = []
     for k, v in sd.items():
         sub = _split_unet_key(k, unet_keys)
         if sub is not None:
@@ -109,24 +117,36 @@ def load_checkpoint(algo, path_or_dict, strict: bool = True) -> Dict[str, List[s
             unet_vals[sub] = v
         elif k in own:
             other[k] = v
+        elif ema is None and k.startswith(_EMA_PREFIX):
+            ignored.append(k)
         else:
             unexpected.append(k)
     missing = sorted(unet_keys - set(unet_vals))
     algo.unet.load_state_dict(unet_vals, strict=False)
+    ema_init = ema is not None and not any(k.startswith(_EMA_PREFIX) for k in other)
     buf_missing = []
     with torch.no_grad():
         for k, v in other.items():
             own[k].copy_(v)
+        if ema_init:
+            for e, p in zip(ema.state_dict().values(), algo.unet.state_dict().values()):
+                e.copy_(p)
     for k in own:
-        if _split_unet_key(k, unet_keys) is None and k not in other:
+        if _split_unet_key(k, unet_keys) is None and k not in other and not (ema_init and k.startswith(_EMA_PREFIX)):
             buf_missing.append(k)
     missing += buf_missing
     if strict and (missing or unexpected):
         raise KeyError(f"checkpoint mismatch: missing {missing[:5]}{'...' if len(missing) > 5 else ''}, "
                        f"unexpected {unexpected[:5]}{'...' if len(unexpected) > 5 else ''}")
-    if getattr(algo.unet, "weights_epoch", None) is not None:
-        algo.unet.weights_epoch += 1          # packed bf16 weights must be rebuilt
-    return {"missing": missing, "unexpected": unexpected}
+    for net in (algo.unet, ema):
+        if getattr(net, "weights_epoch", None) is not None:
+            net.weights_epoch += 1            # packed bf16 weights must be rebuilt
+    out = {"missing": missing, "unexpected": unexpected}
+    if ema is not None:
+        out["ema_initialised"] = ema_init
+    if ignored:
+        out["ignored"] = ignored
+    return out
 
 
 def save_checkpoint(algo, path: str, optimizer=None, global_step: int = 0, epoch: int = 0) -> None:
