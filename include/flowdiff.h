@@ -48,21 +48,17 @@ FD_API unsigned long long fd_launch_count(void);   /* kernels launched by the li
  * (see oracle/flowdiff_oracle.py:backwarp) and is bit-exact against it. */
 FD_API int fd_backwarp_fwd(const float* image, const float* flow, float* out, float* mask,
                     int B, int C, int H, int W, void* stream);
-/* grads of sum(out * gout): gimage (B,C,H,W) is zero-filled by the call; either may be NULL */
-FD_API int fd_backwarp_bwd(const float* image, const float* flow, const float* gout,
-                    float* gimage, float* gflow, int B, int C, int H, int W, void* stream);
-
-/* Backward passes with a caller-provided workspace (fd_warp_bwd_workspace_floats(B, H, W) floats, 16-byte aligned): on
- * three-channel frames with W % 4 == 0 the gradient of the sampled frame is accumulated pixel-interleaved in the workspace
- * with ONE 128-bit reduction per bilinear tap (4 instead of 12 L2 reduction operations per pixel; the gathers read the frame
- * from TMA-staged shared-memory windows) and converted to the planar gradient by a second launch.  Same arguments and
- * results as fd_backwarp_bwd / fd_backwarp_photo_epe_bwd, which serve every other shape (and a NULL workspace). */
-FD_API size_t fd_warp_bwd_workspace_floats(int B, int H, int W);
-FD_API int fd_backwarp_bwd_ws(const float* image, const float* flow, const float* gout, float* gimage, float* gflow,
-                     float* workspace, int B, int C, int H, int W, void* stream);
-FD_API int fd_backwarp_photo_epe_bwd_ws(const float* frame1, const float* frame2, const float* flow, const float* flow_gt,
-                     const float* sums, float g_photo, float g_epe, float* gflow, float* gframe2, float* workspace,
-                     int B, int C, int H, int W, void* stream);
+/* grads of sum(out * gout): gimage (B,C,H,W) and gflow (B,2,H,W), either may be NULL.
+ * Backward passes (this one and fd_backwarp_photo_epe_bwd) take a workspace of fd_warp_bwd_workspace_floats(B, C, H, W)
+ * floats, 16-byte aligned.  The query is non-zero for three-channel frames with W % 4 == 0 and W >= 64: with 16-byte aligned
+ * planes those run on TMA-staged shared-memory windows, and the gradient of the sampled frame is accumulated
+ * pixel-interleaved in the workspace with ONE 128-bit reduction per bilinear tap (4 instead of 12 L2 reduction operations
+ * per pixel), then converted to the planar gradient by a second launch.  There the workspace is required when the frame
+ * gradient is requested (an error otherwise) and unused when it is NULL.  Every other shape runs the gather kernels, which
+ * ignore the workspace (NULL is fine). */
+FD_API size_t fd_warp_bwd_workspace_floats(int B, int C, int H, int W);
+FD_API int fd_backwarp_bwd(const float* image, const float* flow, const float* gout, float* gimage, float* gflow,
+                    float* workspace, int B, int C, int H, int W, void* stream);
 
 /* Self-test of the warp kernels' division: the normalisation `2 v / (W - 1)` of warp.py:107-108 is computed with the
  * reciprocal half of `__fdiv_rn`'s own instruction sequence hoisted out of the pixel loop (fd_warp_common.cuh:bw_div_rn);
@@ -82,14 +78,19 @@ FD_API int fd_backwarp_photo_epe_fwd(const float* frame1, const float* frame2, c
                               const float* flow_gt, float* sums, float* partials,
                               int B, int C, int H, int W, void* stream);
 /* backward of  L = g_photo * sums[0]/sums[1] + g_epe * sums[2]/sums[3]  (mask treated as constant,
- * as autograd does through the reference's thresholding): gflow (B,2,H,W), gframe2 (B,C,H,W, zero-filled) */
+ * as autograd does through the reference's thresholding): gflow (B,2,H,W), gframe2 (B,C,H,W), either may be NULL;
+ * workspace as for fd_backwarp_bwd */
 FD_API int fd_backwarp_photo_epe_bwd(const float* frame1, const float* frame2, const float* flow,
                               const float* flow_gt, const float* sums, float g_photo, float g_epe,
-                              float* gflow, float* gframe2, int B, int C, int H, int W, void* stream);
+                              float* gflow, float* gframe2, float* workspace, int B, int C, int H, int W, void* stream);
 
 /* ---- forward splat: softsplat_new.py:352-423 / 489-565 / 600-700 ----------------------
- * flow channel 0 = dx, channel 1 = dy.  out is (B,C,H/scale,W/scale) and is zero-filled by the call. */
-FD_API int fd_splat_fwd(const float* in, const float* flow, float* out,
+ * flow channel 0 = dx, channel 1 = dy.  out is (B,C,H/scale,W/scale) and is overwritten by the call.
+ * fd_splat_fwd takes a workspace of fd_splat_fwd_workspace_floats(B, C, H, W, scale) floats, 16-byte aligned.  For C = 3
+ * or 4 the query is non-zero and the workspace is required: the splat is accumulated pixel-interleaved in it with one 128-bit
+ * reduction per tap, then copied out to the planar `out`.  Other channel counts accumulate per plane and ignore it. */
+FD_API size_t fd_splat_fwd_workspace_floats(int B, int C, int H, int W, int scale);
+FD_API int fd_splat_fwd(const float* in, const float* flow, float* out, float* workspace,
                  int B, int C, int H, int W, int scale, int off_x, int off_y, void* stream);
 FD_API int fd_splat_ingrad(const float* flow, const float* gout, float* gin,
                     int B, int C, int H, int W, int scale, int off_x, int off_y, void* stream);
@@ -100,12 +101,6 @@ FD_API int fd_splat_flowgrad(const float* in, const float* flow, const float* go
 FD_API int fd_splat_prepare(const float* first, float* ten_in, int B, int C, int HW, void* stream);
 /* warp_forward_flow post-processing (warp.py:139-156): img[b,c] = splat[b,C]>0 ? splat[b,c] : NaN; splat is (B,C+1,HW) */
 FD_API int fd_splat_finish(const float* splat, float* img, int B, int C, int HW, int set_nans, void* stream);
-/* fd_splat_fwd with a caller-provided workspace (fd_splat_fwd_workspace_floats floats, 16-byte aligned): for C = 3 or 4 the
- * splat is accumulated pixel-interleaved with one 128-bit reduction per tap and copied out to the planar `out`; every other
- * channel count (or a NULL workspace) runs fd_splat_fwd.  Same results up to the order of the atomics. */
-FD_API size_t fd_splat_fwd_workspace_floats(int B, int H, int W, int scale);
-FD_API int fd_splat_fwd_ws(const float* in, const float* flow, float* out, float* workspace, int B, int C, int H, int W,
-                     int scale, int off_x, int off_y, void* stream);
 /* warp_forward_flow(warp_style='sum') for THREE-channel images in two launches (warp.py:121-156; prepare + splat + finish
  * fused): `acc` is a caller-provided workspace of 4*B*(H/scale)*(W/scale) floats, 16-byte aligned, in which the splat is
  * accumulated pixel-interleaved (r, g, b, weight) so that a tap is one 128-bit vector reduction; img (B,3,H/s,W/s) receives

@@ -25,21 +25,18 @@ SIGNATURES = {
     "fd_num_sms": (c_int, []),
     "fd_launch_count": (ctypes.c_ulonglong, []),
     "fd_backwarp_fwd": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _P]),
-    "fd_backwarp_bwd": (c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
+    "fd_backwarp_bwd": (c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "fd_photo_epe_workspace_floats": (c_size_t, [_I, _I, _I]),
     "fd_warp_div_selftest": (c_int, [_F, _P, _P]),
-    "fd_warp_bwd_workspace_floats": (c_size_t, [_I, _I, _I]),
-    "fd_backwarp_bwd_ws": (c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
-    "fd_backwarp_photo_epe_bwd_ws": (c_int, [_P, _P, _P, _P, _P, _F, _F, _P, _P, _P, _I, _I, _I, _I, _P]),
+    "fd_warp_bwd_workspace_floats": (c_size_t, [_I, _I, _I, _I]),
     "fd_backwarp_photo_epe_fwd": (c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
-    "fd_backwarp_photo_epe_bwd": (c_int, [_P, _P, _P, _P, _P, _F, _F, _P, _P, _I, _I, _I, _I, _P]),
-    "fd_splat_fwd": (c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "fd_backwarp_photo_epe_bwd": (c_int, [_P, _P, _P, _P, _P, _F, _F, _P, _P, _P, _I, _I, _I, _I, _P]),
+    "fd_splat_fwd": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "fd_splat_ingrad": (c_int, [_P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "fd_splat_flowgrad": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "fd_splat_prepare": (c_int, [_P, _P, _I, _I, _I, _P]),
     "fd_splat_finish": (c_int, [_P, _P, _I, _I, _I, _I, _P]),
-    "fd_splat_fwd_workspace_floats": (c_size_t, [_I, _I, _I, _I]),
-    "fd_splat_fwd_ws": (c_int, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "fd_splat_fwd_workspace_floats": (c_size_t, [_I, _I, _I, _I, _I]),
     "fd_forward_warp_sum3": (c_int, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _I, _P]),
     "fd_nan_mse_workspace_floats": (c_size_t, [_I, _I, _I]),
     "fd_nan_mse_fwd": (c_int, [_P, _P, _P, _P, _I, _I, _I, _L, _L, _P]),

@@ -494,7 +494,8 @@ __global__ void __launch_bounds__(256) splat_finish3_kernel(const float* __restr
 }
 
 // fd_splat_fwd for 3 or 4 input channels through the same pixel-interleaved accumulation (one 128-bit reduction per tap; a
-// fourth channel of zeros for C = 3), then a planar copy-out: fd_splat_fwd_ws.
+// fourth channel of zeros for C = 3), then a planar copy-out.  Same products as splat_fwd_kernel (which every other channel
+// count runs); the sums differ by the order of the atomics only.
 template <int C>
 __global__ void __launch_bounds__(256) splat_fwd_il_kernel(const float* __restrict__ in, const float* __restrict__ flow,
                                                            float* __restrict__ acc, int B, int H, int W, int Ho, int Wo, int scale,
@@ -565,38 +566,34 @@ int check(int B, int C, int H, int W, int scale, int off_x, int off_y) {
 
 extern "C" {
 
-int fd_splat_fwd(const float* in, const float* flow, float* out, int B, int C, int H, int W, int scale, int off_x,
-                 int off_y, void* stream) {
+size_t fd_splat_fwd_workspace_floats(int B, int C, int H, int W, int scale) {
+  return (C == 3 || C == 4) ? (size_t)4 * B * (H / scale) * (W / scale) : 0;
+}
+
+int fd_splat_fwd(const float* in, const float* flow, float* out, float* workspace, int B, int C, int H, int W, int scale,
+                 int off_x, int off_y, void* stream) {
   if (int e = check(B, C, H, W, scale, off_x, off_y)) return e;
   FD_REQUIRE(in && flow && out, "splat_fwd: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
   const int Ho = H / scale, Wo = W / scale;
-  FD_CUDA(cudaMemsetAsync(out, 0, sizeof(float) * (size_t)B * C * Ho * Wo, st));
-  if (W % 4 == 0 && al16({in, flow})) {
-    const long items = (long)B * H * (W / 4);
-    splat_fwd_kernel<4><<<sgrid(items), 256, 0, st>>>(in, flow, out, B, C, H, W, Ho, Wo, scale, off_x, off_y, items);
-  } else {
-    const long items = (long)B * H * W;
-    splat_fwd_kernel<1><<<sgrid(items), 256, 0, st>>>(in, flow, out, B, C, H, W, Ho, Wo, scale, off_x, off_y, items);
+  if (C != 3 && C != 4) {
+    FD_CUDA(cudaMemsetAsync(out, 0, sizeof(float) * (size_t)B * C * Ho * Wo, st));
+    if (W % 4 == 0 && al16({in, flow})) {
+      const long items = (long)B * H * (W / 4);
+      splat_fwd_kernel<4><<<sgrid(items), 256, 0, st>>>(in, flow, out, B, C, H, W, Ho, Wo, scale, off_x, off_y, items);
+    } else {
+      const long items = (long)B * H * W;
+      splat_fwd_kernel<1><<<sgrid(items), 256, 0, st>>>(in, flow, out, B, C, H, W, Ho, Wo, scale, off_x, off_y, items);
+    }
+    FD_LAUNCH_CHECK();
+    return FD_OK;
   }
-  FD_LAUNCH_CHECK();
-  return FD_OK;
-}
-
-size_t fd_splat_fwd_workspace_floats(int B, int H, int W, int scale) { return (size_t)4 * B * (H / scale) * (W / scale); }
-
-int fd_splat_fwd_ws(const float* in, const float* flow, float* out, float* workspace, int B, int C, int H, int W, int scale,
-                    int off_x, int off_y, void* stream) {
-  if (workspace == nullptr || (C != 3 && C != 4) || (reinterpret_cast<uintptr_t>(workspace) & 15) != 0)
-    return fd_splat_fwd(in, flow, out, B, C, H, W, scale, off_x, off_y, stream);
-  if (int e = check(B, C, H, W, scale, off_x, off_y)) return e;
-  FD_REQUIRE(in && flow && out, "splat_fwd_ws: null pointer");
-  cudaStream_t st = (cudaStream_t)stream;
-  const int Ho = H / scale, Wo = W / scale;
+  FD_REQUIRE(workspace != nullptr && (reinterpret_cast<uintptr_t>(workspace) & 15) == 0,
+             "splat_fwd: C = %d needs a 16-byte aligned workspace of fd_splat_fwd_workspace_floats floats", C);
   FD_CUDA(cudaMemsetAsync(workspace, 0, sizeof(float) * 4 * (size_t)B * Ho * Wo, st));
   const unsigned segs = (unsigned)((W + 255) / 256);
   const long jobs = (long)B * H * segs;
-  FD_REQUIRE(jobs < (1L << 31), "splat_fwd_ws: too many row segments");
+  FD_REQUIRE(jobs < (1L << 31), "splat_fwd: too many row segments");
   long grid = jobs;
   if (grid > (long)FD_NUM_SMS * 16) grid = (long)FD_NUM_SMS * 16;
   if (C == 3) {

@@ -234,7 +234,7 @@ inline int make_tmap_bf16(CUtensorMap* map, const void* base, int rank, const ui
 // fp32 tensor, up to 5 dims, NO swizzle (plain row-major box in shared memory), zero fill out of bounds (negative start
 // coordinates included): the sampled-frame windows of fd_warp_win.cu.
 inline int make_tmap_f32_plain(CUtensorMap* map, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                               const uint32_t* box, bool l2_promotion = true) {
+                               const uint32_t* box) {
   EncodeTiledFn fn = get_encode_tiled();
   if (!fn) {
     fd_set_error("cuTensorMapEncodeTiled is unavailable (driver entry point lookup failed)");
@@ -251,7 +251,7 @@ inline int make_tmap_f32_plain(CUtensorMap* map, const void* base, int rank, con
   for (int i = 0; i + 1 < rank; ++i) gs[i] = strides_bytes[i];
   CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                  l2_promotion ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     fd_set_error("cuTensorMapEncodeTiled (fp32) failed (%d): rank %d dims [%llu %llu %llu] box [%u %u %u]", (int)r, rank,

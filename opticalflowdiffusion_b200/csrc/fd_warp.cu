@@ -1,9 +1,9 @@
 // Backward bilinear warp (warp.py:95-119 of the reference) and the fused
 // warp + Charbonnier photometric + end-point-error objective (losses.py:3-6,46-47).
 //
-// Gather/scatter work on fp32 NCHW planes.  The FORWARD operations on three-channel frames with W % 4 == 0 run the
-// shared-memory window kernels of fd_warp_win.cu (TMA-staged frame, 1.5-2x faster on the config-#4 white-noise flow);
-// the kernels in this file serve every other shape and all the backward passes.  Layout choices:
+// Gather/scatter work on fp32 NCHW planes.  Three-channel frames with W % 4 == 0, W >= 64 and 16-byte aligned planes run the
+// shared-memory window kernels of fd_warp_win.cu (TMA-staged frame, 1.5-2x faster on the config-#4 white-noise flow), forward
+// and backward; the kernels in this file serve every other shape.  Layout choices:
 //   * one thread owns VEC (2 when W is even, else 1) consecutive pixels of a row, so flow / flow_gt /
 //     frame1 / out / mask move as wide coalesced accesses; a block walks (row, segment) jobs, no per-thread divisions;
 //   * the 4-tap gathers of the warped frame go through the read-only path (L1/L2 resident: a
@@ -418,23 +418,21 @@ static int check_dims(int B, int C, int H, int W) {
 
 }  // namespace
 
-// fd_warp_win.cu: forward kernels with the sampled frame staged in shared memory by TMA (three-channel frames, W % 4 == 0)
+// fd_warp_win.cu: the kernels with the sampled frame staged in shared memory by TMA (three-channel frames, W % 4 == 0)
 int fd_warp_win_grid(int B, int H, int W);
 int fd_warp_fwd_win(int mode, const float* frame1, const float* frame2, const float* flow, const float* flow_gt, float* out,
                     float* mask, float* partials, float* sums, int B, int H, int W, cudaStream_t st);
-
 int fd_warp_bwd_win(int mode, const float* frame1, const float* frame2, const float* flow, const float* flow_gt, const float* gout,
-                    const float* sums, float g_photo, float g_epe, float* gflow, float* gimage, int B, int H, int W, cudaStream_t st);
+                    const float* fsums, float g_photo, float g_epe, float* gflow, float* gimage, float* acc, int B, int H, int W,
+                    cudaStream_t st);
 
-int fd_warp_bwd_win2(int mode, const float* frame1, const float* frame2, const float* flow, const float* flow_gt, const float* gout,
-                     const float* fsums, float g_photo, float g_epe, float* gflow, float* gimage, float* acc, int B, int H, int W,
-                     cudaStream_t st);
-
-// the window kernels take three-channel frames, W % 4 == 0 and 16-byte aligned planes; the gather kernels everything else
+// the window kernels take three-channel frames, W % 4 == 0 (W >= 64) and 16-byte aligned planes; the gather kernels everything
+// else.  win_shape is the half of the decision that fd_warp_bwd_workspace_floats can see.
+static bool win_shape(int C, int W) { return C == 3 && W % 4 == 0 && W >= 64; }
 static bool use_win(int C, int W, const void* a, const void* b, const void* c, const void* d, const void* e2 = nullptr,
                     const void* f = nullptr) {
   auto al = [](const void* q) { return q == nullptr || (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
-  return C == 3 && W % 4 == 0 && W >= 64 && al(a) && al(b) && al(c) && al(d) && al(e2) && al(f);
+  return win_shape(C, W) && al(a) && al(b) && al(c) && al(d) && al(e2) && al(f);
 }
 
 extern "C" {
@@ -455,15 +453,17 @@ int fd_backwarp_fwd(const float* image, const float* flow, float* out, float* ma
   return FD_OK;
 }
 
-int fd_backwarp_bwd(const float* image, const float* flow, const float* gout, float* gimage, float* gflow, int B,
-                    int C, int H, int W, void* stream) {
+size_t fd_warp_bwd_workspace_floats(int B, int C, int H, int W) { return win_shape(C, W) ? (size_t)4 * B * H * W : 0; }
+
+int fd_backwarp_bwd(const float* image, const float* flow, const float* gout, float* gimage, float* gflow, float* workspace,
+                    int B, int C, int H, int W, void* stream) {
   if (int e = check_dims(B, C, H, W)) return e;
   FD_REQUIRE(image && flow && gout, "backwarp_bwd: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
+  if (use_win(C, W, image, flow, gout, gimage, gflow))
+    return fd_warp_bwd_win(2, nullptr, image, flow, nullptr, gout, nullptr, 0.f, 0.f, gflow, gimage, workspace, B, H, W, st);
   const BwGeom g = make_geom(H, W);
   if (gimage) FD_CUDA(cudaMemsetAsync(gimage, 0, sizeof(float) * (size_t)B * C * H * W, st));
-  if (use_win(C, W, image, flow, gout, gimage, gflow))
-    return fd_warp_bwd_win(0, nullptr, image, flow, nullptr, gout, nullptr, 0.f, 0.f, gflow, gimage, B, H, W, st);
   const int vec = vec_for(W, {image, flow, gout, gimage, gflow});
   const unsigned segs = row_segs(W, vec, 256);
   const long items = (long)B * H * segs;                       // row jobs
@@ -480,34 +480,6 @@ int fd_warp_div_selftest(float divisor, unsigned long long* mismatches, void* st
   div_selftest_kernel<<<FD_NUM_SMS * 8, 256, 0, st>>>(divisor, mismatches);
   FD_LAUNCH_CHECK();
   return FD_OK;
-}
-
-// Backward passes with a caller-provided workspace of fd_warp_bwd_workspace_floats(B, H, W) floats (16-byte aligned): on
-// three-channel frames with W % 4 == 0 the frame gradient is accumulated pixel-interleaved in it, one 128-bit reduction per
-// tap (4 instead of 12 L2 reduction operations per pixel), and converted to the planar gradient by a second launch; every
-// other shape runs the workspace-free entry points above.
-size_t fd_warp_bwd_workspace_floats(int B, int H, int W) { return (size_t)4 * B * H * W; }
-
-int fd_backwarp_bwd_ws(const float* image, const float* flow, const float* gout, float* gimage, float* gflow, float* workspace,
-                       int B, int C, int H, int W, void* stream) {
-  if (int e = check_dims(B, C, H, W)) return e;
-  FD_REQUIRE(image && flow && gout, "backwarp_bwd_ws: null pointer");
-  if (workspace != nullptr && use_win(C, W, image, flow, gout, gimage, gflow, workspace))
-    return fd_warp_bwd_win2(2, nullptr, image, flow, nullptr, gout, nullptr, 0.f, 0.f, gflow, gimage, workspace, B, H, W,
-                            (cudaStream_t)stream);
-  return fd_backwarp_bwd(image, flow, gout, gimage, gflow, B, C, H, W, stream);
-}
-
-int fd_backwarp_photo_epe_bwd_ws(const float* frame1, const float* frame2, const float* flow, const float* flow_gt,
-                                 const float* sums, float g_photo, float g_epe, float* gflow, float* gframe2, float* workspace,
-                                 int B, int C, int H, int W, void* stream) {
-  if (int e = check_dims(B, C, H, W)) return e;
-  FD_REQUIRE(frame1 && frame2 && flow && flow_gt && sums, "photo_epe_bwd_ws: null pointer");
-  if (workspace != nullptr && use_win(C, W, frame1, frame2, flow, flow_gt, gflow, gframe2) &&
-      (reinterpret_cast<uintptr_t>(workspace) & 15) == 0)
-    return fd_warp_bwd_win2(3, frame1, frame2, flow, flow_gt, nullptr, sums, g_photo, g_epe, gflow, gframe2, workspace, B, H, W,
-                            (cudaStream_t)stream);
-  return fd_backwarp_photo_epe_bwd(frame1, frame2, flow, flow_gt, sums, g_photo, g_epe, gflow, gframe2, B, C, H, W, stream);
 }
 
 size_t fd_photo_epe_workspace_floats(int B, int H, int W) {
@@ -539,15 +511,15 @@ int fd_backwarp_photo_epe_fwd(const float* frame1, const float* frame2, const fl
 }
 
 int fd_backwarp_photo_epe_bwd(const float* frame1, const float* frame2, const float* flow, const float* flow_gt,
-                              const float* sums, float g_photo, float g_epe, float* gflow, float* gframe2, int B,
-                              int C, int H, int W, void* stream) {
+                              const float* sums, float g_photo, float g_epe, float* gflow, float* gframe2, float* workspace,
+                              int B, int C, int H, int W, void* stream) {
   if (int e = check_dims(B, C, H, W)) return e;
   FD_REQUIRE(frame1 && frame2 && flow && flow_gt && sums, "photo_epe_bwd: null pointer");
   cudaStream_t st = (cudaStream_t)stream;
+  if (use_win(C, W, frame1, frame2, flow, flow_gt, gflow, gframe2))
+    return fd_warp_bwd_win(3, frame1, frame2, flow, flow_gt, nullptr, sums, g_photo, g_epe, gflow, gframe2, workspace, B, H, W, st);
   const BwGeom g = make_geom(H, W);
   if (gframe2) FD_CUDA(cudaMemsetAsync(gframe2, 0, sizeof(float) * (size_t)B * C * H * W, st));
-  if (use_win(C, W, frame1, frame2, flow, flow_gt, gflow, gframe2))
-    return fd_warp_bwd_win(1, frame1, frame2, flow, flow_gt, nullptr, sums, g_photo, g_epe, gflow, gframe2, B, H, W, st);
   const int vec = vec_for(W, {frame1, frame2, flow, flow_gt, gflow, gframe2});
   const unsigned segs = row_segs(W, vec, 256);
   const long items = (long)B * H * segs;                       // row jobs

@@ -1,5 +1,6 @@
-// Backward bilinear warp (warp.py:95-119) and the fused warp + Charbonnier photometric + end-point-error forward
-// (losses.py:3-6,46-47) with the sampled frame staged in shared memory by TMA -- the forward kernels of BASELINE config #4.
+// Backward bilinear warp (warp.py:95-119) and the fused warp + Charbonnier photometric + end-point-error objective
+// (losses.py:3-6,46-47) with the sampled frame staged in shared memory by TMA -- the forward and backward kernels of BASELINE
+// config #4 (one kernel template, MODE 0 / 1 forward, 2 / 3 backward).
 //
 // Why: the config's flow is white noise (sigma = 4 px), so the 12 bilinear taps of a pixel land in 12 different 32-byte
 // sectors and a warp-wide gather instruction touches ~24 sectors in ~5.5 L1 wavefronts (ncu, profiles/r2_prof_warp_summary.txt:
@@ -402,66 +403,26 @@ int fd_warp_win_grid(int B, int H, int W) {
   return (int)(tiles < FD_NUM_SMS ? tiles : FD_NUM_SMS);
 }
 
-// Backward passes on the forward kernel's skeleton (same TMA windows for the gathers): mode 2 = plain warp given gout, mode 3 =
-// fused photometric + EPE objective.  The gradient of the sampled frame is accumulated in `acc` (B, H, W, 4 floats, 16-byte
-// aligned workspace) with one 128-bit reduction per tap and converted to the planar `gimage` by a second launch.
-int fd_warp_bwd_win2(int mode, const float* frame1, const float* frame2, const float* flow, const float* flow_gt, const float* gout,
-                     const float* fsums, float g_photo, float g_epe, float* gflow, float* gimage, float* acc, int B, int H, int W,
-                     cudaStream_t st) {
-  FD_REQUIRE(W % 4 == 0 && (mode == 2 || mode == 3), "warp_win_bwd2: bad argument");
-  FD_REQUIRE(gimage == nullptr || (acc != nullptr && (reinterpret_cast<uintptr_t>(acc) & 15) == 0), "warp_win_bwd2: workspace");
-  WinParams p{};
-  p.frame1 = frame1; p.frame2 = frame2; p.flow = flow; p.flow_gt = flow_gt; p.gout = gout; p.fsums = fsums;
-  p.g_photo = g_photo; p.g_epe = g_epe; p.gflow = gflow; p.acc = gimage != nullptr ? acc : nullptr;
-  p.g = make_geom(H, W);
-  p.B = B;
-  p.tiles_x = (W + kTW - 1) / kTW;
-  p.tiles_y = (H + kTH - 1) / kTH;
-  const long tiles = (long)B * p.tiles_x * p.tiles_y;
-  FD_REQUIRE(tiles < (1L << 31), "warp_win_bwd2: too many tiles");
-  p.ntiles = (int)tiles;
-  CUtensorMap map;
-  {
-    const uint64_t dims[3] = {(uint64_t)W, (uint64_t)H, (uint64_t)B * kC};
-    const uint64_t str[2] = {(uint64_t)W * 4, (uint64_t)H * W * 4};
-    const uint32_t box[3] = {(uint32_t)kWW, (uint32_t)kWH, (uint32_t)kC};
-    if (int e = make_tmap_f32_plain(&map, frame2, 3, dims, str, box)) return e;
+namespace {
+
+template <int MODE>
+int launch_mode(const CUtensorMap& map, const WinParams& p, int grid, cudaStream_t st) {
+  static bool attr_done = false;
+  if (!attr_done) {
+    FD_CUDA(cudaFuncSetAttribute(warp_win_fwd_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+    attr_done = true;
   }
-  if (p.acc != nullptr) FD_CUDA(cudaMemsetAsync(acc, 0, sizeof(float) * 4 * (size_t)B * H * W, st));
-  const int grid = fd_warp_win_grid(B, H, W);
-  static bool attr_done[2] = {false, false};
-  if (mode == 2) {
-    if (!attr_done[0]) {
-      FD_CUDA(cudaFuncSetAttribute(warp_win_fwd_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-      attr_done[0] = true;
-    }
-    warp_win_fwd_kernel<2><<<grid, kThreads, kSmemBytes, st>>>(map, p);
-  } else {
-    if (!attr_done[1]) {
-      FD_CUDA(cudaFuncSetAttribute(warp_win_fwd_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-      attr_done[1] = true;
-    }
-    warp_win_fwd_kernel<3><<<grid, kThreads, kSmemBytes, st>>>(map, p);
-  }
+  warp_win_fwd_kernel<MODE><<<grid, kThreads, kSmemBytes, st>>>(map, p);
   FD_LAUNCH_CHECK();
-  if (gimage != nullptr) {
-    long blocks = ((long)B * H * W + 255) / 256;
-    if (blocks > (long)FD_NUM_SMS * 16) blocks = (long)FD_NUM_SMS * 16;
-    acc_to_planes3_kernel<<<(unsigned)blocks, 256, 0, st>>>(acc, gimage, B, (long)H * W);
-    FD_LAUNCH_CHECK();
-  }
   return FD_OK;
 }
 
-// mode 0: out / mask; mode 1: sums[4] = {photo sum, mask sum, EPE sum, pixel count}, partials = workspace of
-// fd_warp_win_grid * 3 + 1 floats.  C == 3, W % 4 == 0.
-int fd_warp_fwd_win(int mode, const float* frame1, const float* frame2, const float* flow, const float* flow_gt, float* out,
-                    float* mask, float* partials, float* sums, int B, int H, int W, cudaStream_t st) {
+// One launch of warp_win_fwd_kernel<mode> over three-channel frames with W % 4 == 0: fills in the geometry and the tile walk
+// of p (whose pointers the caller has set) and builds the tensor map of the sampled frame p.frame2.
+int launch_win(int mode, WinParams p, int B, int H, int W, cudaStream_t st) {
   FD_REQUIRE(W % 4 == 0, "warp_win: W %% 4 != 0");
-  FD_REQUIRE((reinterpret_cast<uintptr_t>(frame2) & 15) == 0 && (reinterpret_cast<uintptr_t>(flow) & 15) == 0,
+  FD_REQUIRE((reinterpret_cast<uintptr_t>(p.frame2) & 15) == 0 && (reinterpret_cast<uintptr_t>(p.flow) & 15) == 0,
              "warp_win: 16-byte aligned tensors");
-  WinParams p{};
-  p.frame1 = frame1; p.frame2 = frame2; p.flow = flow; p.flow_gt = flow_gt; p.out = out; p.mask = mask; p.partials = partials; p.sums = sums;
   p.g = make_geom(H, W);
   p.B = B;
   p.tiles_x = (W + kTW - 1) / kTW;
@@ -472,31 +433,56 @@ int fd_warp_fwd_win(int mode, const float* frame1, const float* frame2, const fl
   static const int dbg = fd_diag_bits("FD_WARP_WIN_DBG");
   p.dbg = dbg;
   CUtensorMap map;
-  {
-    const uint64_t dims[3] = {(uint64_t)W, (uint64_t)H, (uint64_t)B * kC};
-    const uint64_t str[2] = {(uint64_t)W * 4, (uint64_t)H * W * 4};
-    const uint32_t box[3] = {(uint32_t)kWW, (uint32_t)kWH, (uint32_t)kC};
-    if (int e = make_tmap_f32_plain(&map, frame2, 3, dims, str, box)) return e;
-  }
+  const uint64_t dims[3] = {(uint64_t)W, (uint64_t)H, (uint64_t)B * kC};
+  const uint64_t str[2] = {(uint64_t)W * 4, (uint64_t)H * W * 4};
+  const uint32_t box[3] = {(uint32_t)kWW, (uint32_t)kWH, (uint32_t)kC};
+  if (int e = make_tmap_f32_plain(&map, p.frame2, 3, dims, str, box)) return e;
   const int grid = fd_warp_win_grid(B, H, W);
-  static bool attr_done[2] = {false, false};
-  if (mode == 0) {
-    if (!attr_done[0]) {
-      FD_CUDA(cudaFuncSetAttribute(warp_win_fwd_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-      attr_done[0] = true;
+  switch (mode) {
+    case 0: return launch_mode<0>(map, p, grid, st);
+    case 1: {
+      static std::atomic<unsigned> next_tag{0};
+      do {
+        p.tag = ++next_tag;                      // unique per launch, never 0
+      } while (p.tag == 0);
+      return launch_mode<1>(map, p, grid, st);
     }
-    warp_win_fwd_kernel<0><<<grid, kThreads, kSmemBytes, st>>>(map, p);
-  } else {
-    if (!attr_done[1]) {
-      FD_CUDA(cudaFuncSetAttribute(warp_win_fwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-      attr_done[1] = true;
-    }
-    static std::atomic<unsigned> next_tag{0};
-    do {
-      p.tag = ++next_tag;                      // unique per launch, never 0
-    } while (p.tag == 0);
-    warp_win_fwd_kernel<1><<<grid, kThreads, kSmemBytes, st>>>(map, p);
+    case 2: return launch_mode<2>(map, p, grid, st);
+    default: return launch_mode<3>(map, p, grid, st);
   }
-  FD_LAUNCH_CHECK();
+}
+
+}  // namespace
+
+// mode 0: out / mask; mode 1: sums[4] = {photo sum, mask sum, EPE sum, pixel count}, partials = workspace of
+// fd_warp_win_grid * 3 + 1 floats.  C == 3, W % 4 == 0.
+int fd_warp_fwd_win(int mode, const float* frame1, const float* frame2, const float* flow, const float* flow_gt, float* out,
+                    float* mask, float* partials, float* sums, int B, int H, int W, cudaStream_t st) {
+  WinParams p{};
+  p.frame1 = frame1; p.frame2 = frame2; p.flow = flow; p.flow_gt = flow_gt; p.out = out; p.mask = mask; p.partials = partials; p.sums = sums;
+  return launch_win(mode, p, B, H, W, st);
+}
+
+// Backward passes on the forward kernel's skeleton (same TMA windows for the gathers): mode 2 = plain warp given gout, mode 3 =
+// fused photometric + EPE objective.  The gradient of the sampled frame, when requested, is accumulated in `acc` (B, H, W, 4
+// floats, 16-byte aligned workspace) with one 128-bit reduction per tap and converted to the planar `gimage` by a second
+// launch; without it `acc` is not touched.
+int fd_warp_bwd_win(int mode, const float* frame1, const float* frame2, const float* flow, const float* flow_gt, const float* gout,
+                    const float* fsums, float g_photo, float g_epe, float* gflow, float* gimage, float* acc, int B, int H, int W,
+                    cudaStream_t st) {
+  FD_REQUIRE(mode == 2 || mode == 3, "warp_win_bwd: bad mode %d", mode);
+  FD_REQUIRE(gimage == nullptr || (acc != nullptr && (reinterpret_cast<uintptr_t>(acc) & 15) == 0),
+             "warp_win_bwd: the frame gradient needs a 16-byte aligned workspace of fd_warp_bwd_workspace_floats floats");
+  WinParams p{};
+  p.frame1 = frame1; p.frame2 = frame2; p.flow = flow; p.flow_gt = flow_gt; p.gout = gout; p.fsums = fsums;
+  p.g_photo = g_photo; p.g_epe = g_epe; p.gflow = gflow; p.acc = gimage != nullptr ? acc : nullptr;
+  if (p.acc != nullptr) FD_CUDA(cudaMemsetAsync(acc, 0, sizeof(float) * 4 * (size_t)B * H * W, st));
+  if (int e = launch_win(mode, p, B, H, W, st)) return e;
+  if (gimage != nullptr) {
+    long blocks = ((long)B * H * W + 255) / 256;
+    if (blocks > (long)FD_NUM_SMS * 16) blocks = (long)FD_NUM_SMS * 16;
+    acc_to_planes3_kernel<<<(unsigned)blocks, 256, 0, st>>>(acc, gimage, B, (long)H * W);
+    FD_LAUNCH_CHECK();
+  }
   return FD_OK;
 }

@@ -29,13 +29,14 @@ def _f32c(t: Tensor) -> Tensor:
 # --------------------------------------------------------------------------------------
 
 
+def _workspace(floats: int, device) -> Optional[Tensor]:
+    """A kernel workspace of the size the library asked for (None -> NULL when it needs none)."""
+    return torch.empty(floats, device=device, dtype=torch.float32) if floats else None
+
+
 def _bwd_workspace(lib, image: Tensor, need_image_grad: bool) -> Optional[Tensor]:
-    """Workspace of the warp backward kernels (pixel-interleaved frame gradient, fd_warp_bwd_workspace_floats): only the
-    three-channel W % 4 == 0 path uses it."""
-    B, C, H, W = image.shape
-    if not need_image_grad or C != 3 or W % 4 != 0:
-        return None
-    return torch.empty(lib.fd_warp_bwd_workspace_floats(B, H, W), device=image.device, dtype=torch.float32)
+    """Workspace of the warp backward kernels (pixel-interleaved frame gradient): only a requested frame gradient uses it."""
+    return _workspace(lib.fd_warp_bwd_workspace_floats(*image.shape), image.device) if need_image_grad else None
 
 
 class _BackwarpFn(torch.autograd.Function):
@@ -62,8 +63,8 @@ class _BackwarpFn(torch.autograd.Function):
         gflow = torch.empty_like(flow) if ctx.needs_input_grad[1] else None
         lib = _lib.load()
         ws = _bwd_workspace(lib, image, gimage is not None)
-        _lib.check(lib.fd_backwarp_bwd_ws(_lib.ptr(image), _lib.ptr(flow), _lib.ptr(gout), _lib.ptr(gimage),
-                                          _lib.ptr(gflow), _lib.ptr(ws), B, C, H, W, _lib.stream()))
+        _lib.check(lib.fd_backwarp_bwd(_lib.ptr(image), _lib.ptr(flow), _lib.ptr(gout), _lib.ptr(gimage),
+                                       _lib.ptr(gflow), _lib.ptr(ws), B, C, H, W, _lib.stream()))
         return gimage, gflow
 
 
@@ -102,9 +103,9 @@ class _PhotoEpeFn(torch.autograd.Function):
         sg[1] = sums[1] / g_photo.detach().float()
         sg[3] = sums[3] / g_epe.detach().float()
         ws = _bwd_workspace(lib, frame2, gframe2 is not None)
-        _lib.check(lib.fd_backwarp_photo_epe_bwd_ws(_lib.ptr(frame1), _lib.ptr(frame2), _lib.ptr(flow),
-                                                    _lib.ptr(flow_gt), _lib.ptr(sg), 1.0, 1.0,
-                                                    _lib.ptr(gflow), _lib.ptr(gframe2), _lib.ptr(ws), B, C, H, W, _lib.stream()))
+        _lib.check(lib.fd_backwarp_photo_epe_bwd(_lib.ptr(frame1), _lib.ptr(frame2), _lib.ptr(flow),
+                                                 _lib.ptr(flow_gt), _lib.ptr(sg), 1.0, 1.0,
+                                                 _lib.ptr(gflow), _lib.ptr(gframe2), _lib.ptr(ws), B, C, H, W, _lib.stream()))
         return None, gframe2, gflow, None
 
 
@@ -129,11 +130,9 @@ class softsplat_func(torch.autograd.Function):
         B, C, H, W = tenIn.shape
         out = torch.empty(B, C, H // scale, W // scale, device=tenIn.device, dtype=torch.float32)
         lib = _lib.load()
-        ws = None
-        if C in (3, 4):      # pixel-interleaved accumulation: one vector reduction per tap instead of C scalar ones
-            ws = torch.empty(lib.fd_splat_fwd_workspace_floats(B, H, W, int(scale)), device=tenIn.device, dtype=torch.float32)
-        _lib.check(lib.fd_splat_fwd_ws(_lib.ptr(tenIn), _lib.ptr(tenFlow), _lib.ptr(out), _lib.ptr(ws), B, C, H, W,
-                                       int(scale), int(offset_x), int(offset_y), _lib.stream()))
+        ws = _workspace(lib.fd_splat_fwd_workspace_floats(B, C, H, W, int(scale)), tenIn.device)
+        _lib.check(lib.fd_splat_fwd(_lib.ptr(tenIn), _lib.ptr(tenFlow), _lib.ptr(out), _lib.ptr(ws), B, C, H, W,
+                                    int(scale), int(offset_x), int(offset_y), _lib.stream()))
         ctx.save_for_backward(tenIn, tenFlow)
         ctx.geom = (int(scale), int(offset_x), int(offset_y))
         return out
@@ -187,9 +186,10 @@ def softsplat(tenIn: Tensor, tenFlow: Tensor, tenMetric: Optional[Tensor], strMo
 
 
 class _ForwardWarpSumFn(torch.autograd.Function):
-    """warp_forward_flow(warp_style='sum') as three launches: prepare (NaN -> weight 0, append the
-    weight channel), splat, finish (holes -> NaN).  Gradient flows to ``flow`` only (cond has no
-    grad in training, SURVEY.md S2) and to ``first`` on request."""
+    """warp_forward_flow(warp_style='sum') as prepare (NaN -> weight 0, append the weight channel),
+    splat, finish (holes -> NaN); for three-channel images fused into the two launches of
+    fd_forward_warp_sum3.  Gradient flows to ``flow`` only (cond has no grad in training, SURVEY.md
+    S2) and to ``first`` on request."""
 
     @staticmethod
     def forward(ctx, first: Tensor, flow: Tensor, scale: int, set_nans: bool, off_x: int, off_y: int):
@@ -215,7 +215,8 @@ class _ForwardWarpSumFn(torch.autograd.Function):
         _lib.check(lib.fd_splat_prepare(_lib.ptr(first), _lib.ptr(ten_in), B, C, H * W, st))
         Ho, Wo = H // scale, W // scale
         ret = torch.empty(B, C + 1, Ho, Wo, device=first.device, dtype=torch.float32)
-        _lib.check(lib.fd_splat_fwd(_lib.ptr(ten_in), _lib.ptr(flow), _lib.ptr(ret), B, C + 1, H, W, scale,
+        ws = _workspace(lib.fd_splat_fwd_workspace_floats(B, C + 1, H, W, scale), first.device)
+        _lib.check(lib.fd_splat_fwd(_lib.ptr(ten_in), _lib.ptr(flow), _lib.ptr(ret), _lib.ptr(ws), B, C + 1, H, W, scale,
                                     off_x, off_y, st))
         img = torch.empty(B, C, Ho, Wo, device=first.device, dtype=torch.float32)
         _lib.check(lib.fd_splat_finish(_lib.ptr(ret), _lib.ptr(img), B, C, Ho * Wo, int(bool(set_nans)), st))

@@ -70,38 +70,36 @@ def measure(iters=50, warmup=10):
 
     t = timeit(lambda: _lib.check(lib.fd_backwarp_photo_epe_fwd(P(f1), P(f2), P(flow), P(gt), P(sums), P(ws), B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
     rec("photo_epe_fwd", t, 40 * px)
-    wsb = torch.empty(lib.fd_warp_bwd_workspace_floats(B, H, W), device="cuda")
-    t = timeit(lambda: _lib.check(lib.fd_backwarp_photo_epe_bwd_ws(P(f1), P(f2), P(flow), P(gt), P(sums), 1.0, 1.0, P(gflow), P(gf2), P(wsb), B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
+    wsb = torch.empty(lib.fd_warp_bwd_workspace_floats(B, C, H, W), device="cuda")
+    t = timeit(lambda: _lib.check(lib.fd_backwarp_photo_epe_bwd(P(f1), P(f2), P(flow), P(gt), P(sums), 1.0, 1.0, P(gflow), P(gf2), P(wsb), B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
     rec("photo_epe_bwd", t, 60 * px)
     t = timeit(lambda: _lib.check(lib.fd_backwarp_fwd(P(f2), P(flow), P(out), P(mask), B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
     rec("backwarp_fwd", t, (8 + 12 + 12 + 12) * px)
-    t = timeit(lambda: _lib.check(lib.fd_backwarp_bwd_ws(P(f2), P(flow), P(out), P(gf2), P(gflow), P(wsb), B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
+    t = timeit(lambda: _lib.check(lib.fd_backwarp_bwd(P(f2), P(flow), P(out), P(gf2), P(gflow), P(wsb), B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
     rec("backwarp_bwd", t, (8 + 12 + 12 + 12 + 8) * px)
-    # the workspace-free entry points (frame gradient accumulated in shared-memory windows, TMA reduce-add)
-    t = timeit(lambda: _lib.check(lib.fd_backwarp_photo_epe_bwd(P(f1), P(f2), P(flow), P(gt), P(sums), 1.0, 1.0, P(gflow), P(gf2), B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
-    rec("photo_epe_bwd_no_workspace", t, 60 * px)
-    t = timeit(lambda: _lib.check(lib.fd_backwarp_bwd(P(f2), P(flow), P(out), P(gf2), P(gflow), B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
-    rec("backwarp_bwd_no_workspace", t, (8 + 12 + 12 + 12 + 8) * px)
+    # the flow gradient alone (frames without gradient, as in a training step that learns only the flow): no scatter
+    t = timeit(lambda: _lib.check(lib.fd_backwarp_photo_epe_bwd(P(f1), P(f2), P(flow), P(gt), P(sums), 1.0, 1.0, P(gflow), None, None, B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
+    rec("photo_epe_bwd_flow_only", t, 48 * px)
+    t = timeit(lambda: _lib.check(lib.fd_backwarp_bwd(P(f2), P(flow), P(out), None, P(gflow), None, B, C, H, W, st)), flush=flush, iters=iters, warmup=warmup)
+    rec("backwarp_bwd_flow_only", t, (8 + 12 + 12 + 8) * px)
     so = torch.empty_like(f2)
-    wss = torch.empty(lib.fd_splat_fwd_workspace_floats(B, H, W, 1), device="cuda")
-    t = timeit(lambda: _lib.check(lib.fd_splat_fwd_ws(P(f2), P(flow), P(so), P(wss), B, C, H, W, 1, 0, 0, st)), flush=flush, iters=iters, warmup=warmup)
+    wss = torch.empty(lib.fd_splat_fwd_workspace_floats(B, C, H, W, 1), device="cuda")
+    t = timeit(lambda: _lib.check(lib.fd_splat_fwd(P(f2), P(flow), P(so), P(wss), B, C, H, W, 1, 0, 0, st)), flush=flush, iters=iters, warmup=warmup)
     rec("splat_fwd", t, (8 + 12 + 12) * px)
-    t = timeit(lambda: _lib.check(lib.fd_splat_fwd(P(f2), P(flow), P(so), B, C, H, W, 1, 0, 0, st)), flush=flush, iters=iters, warmup=warmup)
-    rec("splat_fwd_no_workspace", t, (8 + 12 + 12) * px)
     t = timeit(lambda: _lib.check(lib.fd_splat_flowgrad(P(f2), P(flow), P(out), P(gflow), B, C, H, W, 1, 0, 0, st)), flush=flush, iters=iters, warmup=warmup)
     rec("splat_flowgrad", t, (8 + 12 + 12 + 8) * px)
-    # warp_forward_flow on a three-channel image (what UnetWithWarp / the pyramid loss call): generic three launches vs the
-    # fused two-launch path with pixel-interleaved accumulation; bytes: image 12 + flow 8 + output 12 per pixel
+    # warp_forward_flow on a three-channel image (what UnetWithWarp / the pyramid loss call): generic prepare / splat / finish
+    # vs the fused two-launch path; bytes: image 12 + flow 8 + output 12 per pixel
     ten_in = torch.empty(B, 4, H, W, device="cuda")
     ret = torch.empty(B, 4, H, W, device="cuda")
     acc = torch.empty(B, H, W, 4, device="cuda")
 
     def generic():
         _lib.check(lib.fd_splat_prepare(P(f2), P(ten_in), B, C, H * W, st))
-        _lib.check(lib.fd_splat_fwd(P(ten_in), P(flow), P(ret), B, C + 1, H, W, 1, 0, 0, st))
+        _lib.check(lib.fd_splat_fwd(P(ten_in), P(flow), P(ret), P(acc), B, C + 1, H, W, 1, 0, 0, st))
         _lib.check(lib.fd_splat_finish(P(ret), P(so), B, C, H * W, 1, st))
     t = timeit(generic, flush=flush, iters=iters, warmup=warmup)
-    rec("forward_warp_sum_3launch", t, (12 + 8 + 12) * px)
+    rec("forward_warp_sum_generic", t, (12 + 8 + 12) * px)
     t = timeit(lambda: _lib.check(lib.fd_forward_warp_sum3(P(f2), P(flow), None, P(acc), P(so), None, B, H, W, 1, 0, 0, 1, st)),
                flush=flush, iters=iters, warmup=warmup)
     rec("forward_warp_sum_fused", t, (12 + 8 + 12) * px)

@@ -146,7 +146,7 @@ int main() {
     run<0, 0>("3 x f32 planar, displacement 0", buf, bytes, bps);
     run<1, 0>("3 x f32 planar, white-noise +-12 px", buf, bytes, bps);
   }
-  // the two bandwidth-bound passes that surround the scatter in fd_splat_fwd_ws / fd_warp_bwd_win2
+  // the two bandwidth-bound passes that surround the scatter in fd_splat_fwd / fd_warp_bwd_win
   cudaEvent_t s, e;
   cudaEventCreate(&s);
   cudaEventCreate(&e);

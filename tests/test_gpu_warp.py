@@ -244,47 +244,46 @@ def test_hoisted_reciprocal_division_is_exact(divisor):
 
 @pytest.mark.parametrize("C", [3, 4])
 @pytest.mark.parametrize("geom", [(1, 0, 0), (2, 1, 0), (4, 1, 3)])
-def test_splat_forward_interleaved_accumulation(C, geom):
-    """fd_splat_fwd_ws (pixel-interleaved accumulation, one 128-bit reduction per tap, planar copy-out) == fd_splat_fwd
-    (softsplat_new.py:352-423, golden-pinned by the tests above) up to the order of the atomics, NaN / Inf / far flows
-    included; and fd_forward_warp_sum3 == prepare + splat + finish."""
+def test_splat_forward_interleaved_vs_oracle(C, geom):
+    """fd_splat_fwd at C = 3 / 4 (pixel-interleaved accumulation, one 128-bit reduction per tap, planar copy-out) == the
+    oracle's splat (softsplat_new.py:352-423) up to the order of the atomics, NaN / Inf / far flows included; and
+    fd_forward_warp_sum3 == the oracle's warp_forward_flow (prepare + splat + finish)."""
     from opticalflowdiffusion_b200 import _lib
     lib = _lib.load()
     scale, ox, oy = geom
     B, H, W = 2, 24, 40
     g = torch.Generator().manual_seed(C * 10 + scale)
-    x = torch.randn(B, C, H, W, generator=g).cuda()
-    flow = (torch.randn(B, 2, H, W, generator=g) * 3).cuda()
+    x = torch.randn(B, C, H, W, generator=g)
+    flow = torch.randn(B, 2, H, W, generator=g) * 3
     flow[0, 0, 3, 4] = float("nan")
     flow[1, 1, 5, 6] = float("inf")
     flow[0, :, 0, 0] = -50.0
     Ho, Wo = H // scale, W // scale
     P, st = _lib.ptr, _lib.stream()
-    ref = torch.empty(B, C, Ho, Wo, device="cuda")
-    got = torch.full_like(ref, float("nan"))
-    ws = torch.empty(lib.fd_splat_fwd_workspace_floats(B, H, W, scale), device="cuda")
-    _lib.check(lib.fd_splat_fwd(P(x), P(flow), P(ref), B, C, H, W, scale, ox, oy, st))
-    _lib.check(lib.fd_splat_fwd_ws(P(x), P(flow), P(got), P(ws), B, C, H, W, scale, ox, oy, st))
-    torch.cuda.synchronize()
+    ref = O.splat_forward(x, flow, scale, ox, oy)
+    xc, fc = x.cuda(), flow.cuda()
+    got = torch.full((B, C, Ho, Wo), float("nan"), device="cuda")
+    ws = torch.empty(lib.fd_splat_fwd_workspace_floats(B, C, H, W, scale), device="cuda")
+    _lib.check(lib.fd_splat_fwd(P(xc), P(fc), P(got), P(ws), B, C, H, W, scale, ox, oy, st))
+    got = got.cpu()
     assert torch.isfinite(got).all()
     assert (got - ref).abs().max().item() <= 1e-5 * max(1.0, ref.abs().max().item())
     if C == 3:
         first = x.clone()
         first[0, 1, 7, 8] = float("nan")                      # NaN source pixel: weight 0
+        img_ref = O.warp_forward_flow(first, flow, scale, True, (ox, oy))
+        wsum_ref = O.splat_forward((~torch.isnan(first).any(1, keepdim=True)).float(), flow, scale, ox, oy)
+        first = first.cuda()
         ten_in = torch.empty(B, 4, H, W, device="cuda")
-        ret = torch.empty(B, 4, Ho, Wo, device="cuda")
-        img_ref = torch.empty(B, 3, Ho, Wo, device="cuda")
         _lib.check(lib.fd_splat_prepare(P(first), P(ten_in), B, 3, H * W, st))
-        _lib.check(lib.fd_splat_fwd(P(ten_in), P(flow), P(ret), B, 4, H, W, scale, ox, oy, st))
-        _lib.check(lib.fd_splat_finish(P(ret), P(img_ref), B, 3, Ho * Wo, 1, st))
         ten2, acc = torch.empty_like(ten_in), torch.empty(B, Ho, Wo, 4, device="cuda")
-        img, wsum = torch.empty_like(img_ref), torch.empty(B, 1, Ho, Wo, device="cuda")
-        _lib.check(lib.fd_forward_warp_sum3(P(first), P(flow), P(ten2), P(acc), P(img), P(wsum), B, H, W, scale, ox, oy, 1, st))
-        torch.cuda.synchronize()
+        img, wsum = torch.empty(B, 3, Ho, Wo, device="cuda"), torch.empty(B, 1, Ho, Wo, device="cuda")
+        _lib.check(lib.fd_forward_warp_sum3(P(first), P(fc), P(ten2), P(acc), P(img), P(wsum), B, H, W, scale, ox, oy, 1, st))
+        img, wsum = img.cpu(), wsum.cpu()
         assert torch.equal(ten2, ten_in)
         assert torch.equal(torch.isnan(img), torch.isnan(img_ref))
         assert (img.nan_to_num() - img_ref.nan_to_num()).abs().max().item() <= 1e-5 * max(1.0, ref.abs().max().item())
-        assert (wsum[:, 0] - ret[:, 3]).abs().max().item() <= 1e-5
+        assert (wsum - wsum_ref).abs().max().item() <= 1e-5
 
 
 def _misaligned(t):
@@ -298,10 +297,11 @@ def _misaligned(t):
 
 
 @pytest.mark.parametrize("shape", [(1, 50, 68), (2, 17, 132), (3, 16, 128), (1, 97, 260), (1, 1024, 2048)])
-def test_window_kernels_equal_gather_kernels(shape):
-    """The shared-memory-window kernels (fd_warp_win*.cu: tiles of 16 x 128, 16-pixel halo, TMA zero fill, border tiles,
+def test_window_kernels_equal_gather_kernels_and_flow_only(shape):
+    """The shared-memory-window kernels (fd_warp_win.cu: tiles of 16 x 128, 16-pixel halo, TMA zero fill, border tiles,
     out-of-window fallback) against the one-thread-per-pixel gather kernels on ragged / small / large shapes with flows that
-    leave the window and the image: forward output and mask bit-identical, sums and gradients to the order of the atomics."""
+    leave the window and the image: forward output and mask bit-identical, sums and gradients to the order of the atomics,
+    the flow gradient of the window backward bit-identical with and without the frame gradient."""
     from opticalflowdiffusion_b200 import _lib
     lib = _lib.load()
     B, H, Wd = shape
@@ -333,29 +333,56 @@ def test_window_kernels_equal_gather_kernels(shape):
 
     def close(a, b):
         return (a - b).abs().max().item() <= 2e-5 * max(b.abs().max().item(), 1e-12)
-    wsb = torch.empty(lib.fd_warp_bwd_workspace_floats(B, H, Wd), device="cuda")
+    wsb = torch.empty(lib.fd_warp_bwd_workspace_floats(B, 3, H, Wd), device="cuda")
+    assert wsb.numel() == 4 * B * H * Wd
+    # window kernels with and without the frame gradient (flow only: no accumulation buffer), gather kernels on the views
     res = []
-    for (a1, a2, fl_, gt_, use_ws) in ((f1, f2, flow, gt, True), (f1, f2, flow, gt, False), (m1, m2, mf, mg, False)):
-        gfl, gf2 = torch.empty_like(flow), torch.full_like(f2, float("nan"))
-        if use_ws:
-            _lib.check(lib.fd_backwarp_photo_epe_bwd_ws(P(a1), P(a2), P(fl_), P(gt_), P(s_g), 1.0, 0.5, P(gfl), P(gf2), P(wsb),
-                                                        B, 3, H, Wd, st))
-        else:
-            _lib.check(lib.fd_backwarp_photo_epe_bwd(P(a1), P(a2), P(fl_), P(gt_), P(s_g), 1.0, 0.5, P(gfl), P(gf2), B, 3, H, Wd, st))
+    for (a1, a2, fl_, gt_, frame_grad) in ((f1, f2, flow, gt, True), (f1, f2, flow, gt, False), (m1, m2, mf, mg, True)):
+        gfl = torch.empty_like(flow)
+        gf2 = torch.full_like(f2, float("nan")) if frame_grad else None
+        _lib.check(lib.fd_backwarp_photo_epe_bwd(P(a1), P(a2), P(fl_), P(gt_), P(s_g), 1.0, 0.5, P(gfl), P(gf2),
+                                                 P(wsb if frame_grad else None), B, 3, H, Wd, st))
         res.append((gfl, gf2))
-    for gfl, gf2 in res[:2]:
-        assert close(gfl, res[2][0]) and close(gf2, res[2][1])
+    (gfl_w, gf2_w), (gfl_fo, _), (gfl_g, gf2_g) = res
+    assert close(gfl_w, gfl_g) and close(gf2_w, gf2_g) and close(gfl_fo, gfl_g)
+    assert torch.equal(gfl_fo, gfl_w)          # the flow gradient is written per pixel without atomics
     res = []
-    for (a2, fl_, go_, use_ws) in ((f2, flow, gout, True), (f2, flow, gout, False), (m2, mf, mo, False)):
-        gim, gfl = torch.full_like(f2, float("nan")), torch.empty_like(flow)
-        if use_ws:
-            _lib.check(lib.fd_backwarp_bwd_ws(P(a2), P(fl_), P(go_), P(gim), P(gfl), P(wsb), B, 3, H, Wd, st))
-        else:
-            _lib.check(lib.fd_backwarp_bwd(P(a2), P(fl_), P(go_), P(gim), P(gfl), B, 3, H, Wd, st))
+    for (a2, fl_, go_, frame_grad) in ((f2, flow, gout, True), (f2, flow, gout, False), (m2, mf, mo, True)):
+        gfl = torch.empty_like(flow)
+        gim = torch.full_like(f2, float("nan")) if frame_grad else None
+        _lib.check(lib.fd_backwarp_bwd(P(a2), P(fl_), P(go_), P(gim), P(gfl), P(wsb if frame_grad else None), B, 3, H, Wd, st))
         res.append((gim, gfl))
     torch.cuda.synchronize()
-    for gim, gfl in res[:2]:
-        assert close(gim, res[2][0]) and close(gfl, res[2][1])
+    (gim_w, gfl_w), (_, gfl_fo), (gim_g, gfl_g) = res
+    assert close(gim_w, gim_g) and close(gfl_w, gfl_g) and close(gfl_fo, gfl_g)
+    assert torch.equal(gfl_fo, gfl_w)
+
+
+def test_frame_gradient_without_workspace_is_an_error():
+    """Shapes whose query returns a workspace need it for the frame gradient (the window backward kernels, the interleaved
+    splat): a NULL workspace is refused by the argument checks, before anything is launched, and the outputs stay untouched."""
+    from opticalflowdiffusion_b200 import _lib
+    lib = _lib.load()
+    B, C, H, Wd = 1, 3, 32, 128
+    P, st = _lib.ptr, _lib.stream()
+    f1, f2, gout = (torch.rand(B, C, H, Wd, device="cuda") for _ in range(3))
+    flow, gt = torch.randn(B, 2, H, Wd, device="cuda"), torch.randn(B, 2, H, Wd, device="cuda")
+    sums = torch.ones(4, device="cuda")
+    assert lib.fd_warp_bwd_workspace_floats(B, C, H, Wd) > 0
+    gfl, gim = torch.full_like(flow, float("nan")), torch.full_like(f2, float("nan"))
+    assert lib.fd_backwarp_bwd(P(f2), P(flow), P(gout), P(gim), P(gfl), None, B, C, H, Wd, st) != 0
+    assert "workspace" in lib.fd_last_error().decode()
+    assert lib.fd_backwarp_photo_epe_bwd(P(f1), P(f2), P(flow), P(gt), P(sums), 1.0, 1.0, P(gfl), P(gim), None,
+                                         B, C, H, Wd, st) != 0
+    assert "workspace" in lib.fd_last_error().decode()
+    for c in (3, 4):
+        assert lib.fd_splat_fwd_workspace_floats(B, c, H, Wd, 1) > 0
+        x, out = torch.rand(B, c, H, Wd, device="cuda"), torch.full((B, c, H, Wd), float("nan"), device="cuda")
+        assert lib.fd_splat_fwd(P(x), P(flow), P(out), None, B, c, H, Wd, 1, 0, 0, st) != 0
+        assert "workspace" in lib.fd_last_error().decode()
+        assert torch.isnan(out).all()
+    torch.cuda.synchronize()
+    assert torch.isnan(gfl).all() and torch.isnan(gim).all()
 
 
 def test_photo_epe_ticket_needs_no_clean_workspace():
