@@ -450,6 +450,22 @@ FD_API int fd_edge_smooth_fwd(const float* img, const float* flow, float* out, f
 FD_API int fd_edge_smooth_bwd(const float* img, const float* flow, const float* upstream, float* gflow, int B, int Ci,
                        int Cf, int H, int W, void* stream);
 
+/* ---- scoring of K sampled flows per image against the ground truth (evaluation.score_flows) ----
+ * samples fp32 (B, K, 2, H, W) contiguous, in the sampler's normalised units: flow k in px is scale * samples[b, k].
+ * gt fp32 (B, 2, H, W) px or NULL; mean_out (B, 2, H, W) px or NULL; spread_out (B, H, W) px or NULL.
+ * Per pixel: mean flow m = scale * (1/K) sum_k f_k (summed in order k = 0 .. K-1); spread = sqrt((1/K) sum_k |scale f_k - m|^2)
+ * (exactly 0 when K = 1).  A pixel is valid when both gt components are finite and |gt| < 1e9 (the .flo "unknown" marker);
+ * with gt == NULL every pixel is valid.  EPE = |f - gt|_2 in px.
+ * per_image fp64 (B, 8 + K): 0 valid pixels, 1 sum EPE(mean), 2/3/4 count EPE(mean) < 1/3/5 px, 5 Fl outliers (EPE(mean) > 3 px
+ * and > 0.05 |gt|), 6 sum spread, 7 valid pixels with max(|gt_u|, |gt_v|) > gt_limit, 8 + k sum EPE(sample k); sums over
+ * valid pixels only; with gt == NULL only columns 0 and 6 are non-zero.  A non-finite sample at a valid pixel makes the sums
+ * NaN.  workspace: fd_flow_eval_workspace_floats(B, K, H, W) floats, any contents on entry.  No allocation, no atomics, no
+ * synchronisation: the same inputs give the same bits.  16-byte path when W % 4 == 0 and every tensor pointer is 16-byte
+ * aligned, scalar otherwise.  B <= 65535. */
+FD_API size_t fd_flow_eval_workspace_floats(int B, int K, int H, int W);
+FD_API int fd_flow_eval(const float* samples, float scale, const float* gt, float gt_limit, float* mean_out, float* spread_out,
+                 double* per_image, float* workspace, int B, int K, int H, int W, void* stream);
+
 /* debug / test helpers: fp32 NCHW <-> bf16 NHWC */
 FD_API int fd_nchw_to_nhwc_bf16(const float* x, void* out, int N, int C, int HW, void* stream);
 FD_API int fd_nhwc_bf16_to_nchw(const void* x, float* out, int N, int C, int HW, void* stream);

@@ -114,6 +114,8 @@ SIGNATURES = {
     "fd_soft_charb_multi_fwd": (c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "fd_soft_charb_multi_bwd": (c_int, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "fd_conv_wgrad": (c_int, [_P, _I, _P, _I, _P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P]),
+    "fd_flow_eval_workspace_floats": (c_size_t, [_I, _I, _I, _I]),
+    "fd_flow_eval": (c_int, [_P, _F, _P, _F, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
 }
 
 

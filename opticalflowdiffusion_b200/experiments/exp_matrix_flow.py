@@ -3,7 +3,8 @@ experiments/exp_base.py:47-59,120-238 + exp_99.py:18-45 that drives the hot path
 
 The reference builds a ``pl.Trainer`` (DDP when more than one GPU is visible, exp_base.py:198).
 Lightning is not part of this path's contract, so the loop here is explicit: one process per GPU
-(torchrun), batch-sharded data, ``validation`` / ``sample`` tasks run the CUDA sampling path; ``train`` is
+(torchrun), batch-sharded data, ``validation`` / ``sample`` tasks run the CUDA sampling path, ``evaluate`` scores K sampled
+flows per image against the ground truth over a whole split (``evaluation.FlowScores``); ``train`` is
 ``training_step`` -> ``loss.backward()`` (the UnetFunction backward kernels) -> one NCCL all-reduce of the flat
 gradient (DDPStrategy's exchange, exp_base.py:198) -> fused clip + Adam."""
 from __future__ import annotations
@@ -18,7 +19,7 @@ from ..datasets import SyntheticSintelDataset
 from ..io_formats import SintelFlowDataset, load_checkpoint
 from ..flow_diffuser import FlowDiffuser
 from ..flow_learner import FlowLearner
-from ..parallel import init_distributed, reduce_metrics, sync_module_from_rank0
+from ..parallel import init_distributed, reduce_metrics, shard_range, sync_module_from_rank0
 
 
 class MatrixFlowExperiment:
@@ -67,6 +68,8 @@ class MatrixFlowExperiment:
             return self.train()
         if task in ("validation", "validate", "test"):
             return self.validate()
+        if task == "evaluate":
+            return self.evaluate()
         raise ValueError(f"Specified task '{task}' not implemented for class {self.__class__.__name__}.")
 
     def train(self, max_steps: Optional[int] = None):
@@ -154,3 +157,38 @@ class MatrixFlowExperiment:
             self.algo.validation_step(tuple(t.to(dev) for t in batch), i)
             out = {k: float(v) for k, v in self.algo.logged.items()} if hasattr(self.algo, "logged") else {}
         return reduce_metrics(out, device=dev)     # sync_dist=True semantics for the scalars
+
+    @torch.no_grad()
+    def evaluate(self, max_batches: Optional[int] = None):
+        """End-point error of ``experiment.evaluation.num_samples`` sampled flows per image against the ground truth over
+        ``experiment.evaluation.split``: each rank scores the contiguous ``shard_range`` of the split's indices, unshuffled
+        (no DistributedSampler: it pads by repeating images), and one fp64 SUM all-reduce gives every rank the same
+        dataset-level metrics (``evaluation.FlowScores``).  ``limit_batch`` / ``max_batches`` cap the batches per rank."""
+        from ..evaluation import FlowScores
+        if not hasattr(self.algo, "evaluate_step"):
+            raise NotImplementedError(f"algorithm '{self.cfg.algorithm.name}' has no evaluate_step")
+        dev = torch.device("cuda", self.local_rank)
+        torch.cuda.set_device(dev)
+        distributed = init_distributed(dev)
+        self.algo.to(dev)
+        if distributed and not getattr(self, "_synced", False):
+            sync_module_from_rank0(self.algo)
+            self._synced = True
+        ev = self.cfg.experiment.evaluation
+        K, seed = int(ev.num_samples), int(ev.seed)
+        limit = max_batches or ev.get("limit_batch")
+        ds = self._build_dataset(str(ev.split))
+        mine = shard_range(len(ds), self.rank, self.world)
+        loader = torch.utils.data.DataLoader(torch.utils.data.Subset(ds, list(mine)), batch_size=int(ev.data.batch_size),
+                                             shuffle=False, num_workers=0)
+        scores = FlowScores(K, device=dev)
+        start = mine.start
+        for i, batch in enumerate(loader):
+            if limit is not None and i >= int(limit):
+                break
+            n = batch[0].shape[0]
+            rows = self.algo.evaluate_step(tuple(t.to(dev) for t in batch), range(start, start + n), K, seed,
+                                           max_batch=ev.get("max_sample_batch"))
+            scores.update(rows)
+            start += n
+        return scores.metrics()

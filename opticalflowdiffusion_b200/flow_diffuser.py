@@ -336,6 +336,62 @@ class FlowDiffuser(_Base):
             samples = W.warp(cond[:, :self.dim], None, last.contiguous(), mode="forward")
         return samples, flow
 
+    @torch.no_grad()
+    def sample_flows(self, cond: Tensor, ids: Sequence[int], num_samples: int, seed: int, max_batch: Optional[int] = None,
+                     use_ema: Optional[bool] = None) -> Tensor:
+        """``num_samples`` (K) final flows per image, normalised (pixels / ``flow_max``), as (B, K, 2, H, W).
+
+        ``cond`` (B, C, H, W) is the conditioning ``preprocess`` returns, ``ids`` the images' dataset indices.  x_T of
+        sample k of image i is drawn on the device from a generator seeded with ``evaluation.sample_seed(seed, i, k)``; the
+        B*K samples go through ``sample`` (the CUDA-graph path where it takes one) in chunks of at most ``max_batch``
+        (default B).  With the deterministic samplers (DDIM with eta = 0, DPM-Solver++) an image's samples therefore do
+        not depend on its batch, the chunking or the number of ranks, up to the batch invariance of the UNet kernels (and,
+        for target='joint' / 'target', the float-atomic forward splat of the UNet input, which varies run to run).
+        DDPM and DDIM with eta > 0 also draw per-step noise from the global generator: those samples depend on the order of
+        the calls.  The flow taken is the one ``validation_step`` treats as final for each ``target``."""
+        from .evaluation import MAX_SAMPLES, sample_seed
+        B, K = cond.shape[0], int(num_samples)
+        if len(ids) != B:
+            raise ValueError(f"{len(ids)} dataset indices for a batch of {B}")
+        if not 1 <= K <= MAX_SAMPLES:
+            raise ValueError(f"num_samples must be in [1, {MAX_SAMPLES}], got {K}")
+        chunk = int(max_batch or B)
+        if chunk < 1:
+            raise ValueError(f"max_batch must be positive, got {max_batch}")
+        dev = cond.device
+        H, Wd = cond.shape[-2:]
+        shape = (self._diffusion(use_ema).channels, H, Wd)
+        x_T = torch.empty((B * K,) + shape, device=dev, dtype=torch.float32)
+        gen = torch.Generator(device=dev)
+        for b, i in enumerate(ids):
+            for k in range(K):
+                gen.manual_seed(sample_seed(seed, int(i), k))
+                torch.randn(shape, generator=gen, device=dev, out=x_T[b * K + k])
+        cond_k = cond.repeat_interleave(K, dim=0)
+        flows = torch.empty((B * K, 2, H, Wd), device=dev, dtype=torch.float32)
+        keep = self.return_all_timesteps
+        self.return_all_timesteps = False
+        try:
+            for s in range(0, B * K, chunk):
+                e = min(s + chunk, B * K)
+                # the flow argument only gives sample() the batch size and, for target='target', the 2 flow channels
+                _, flow = self.sample(cond_k[s:e], cond_k.new_empty((e - s, 2, 1, 1)), use_ema=use_ema, x_T=x_T[s:e])
+                flows[s:e] = flow[-1] if self.target == "target" else flow     # target: the last step's flow output
+        finally:
+            self.return_all_timesteps = keep
+        return flows.view(B, K, 2, H, Wd)
+
+    @torch.no_grad()
+    def evaluate_step(self, batch, ids: Sequence[int], num_samples: int, seed: int,
+                      max_batch: Optional[int] = None) -> Tensor:
+        """Scores ``num_samples`` sampled flows per image of ``batch`` = (img, tgt, flow px) against its raw flow:
+        the per-image rows of ``evaluation.score_flows`` (B, 8 + K), fp64 on the device.  ``cond`` comes from
+        ``preprocess(batch, aug=False)``; the EMA network samples when there is one.  Logs nothing."""
+        from .evaluation import score_flows
+        _, cond, _ = self.preprocess(batch, aug=False)
+        flows = self.sample_flows(cond, ids, num_samples, seed, max_batch=max_batch)
+        return score_flows(flows, self.flow_max, gt=batch[2].float())[2]
+
     # ------------------------------------------------------------------ steps
     @staticmethod
     def _stats(prefix: str, name: str, x: Tensor):
