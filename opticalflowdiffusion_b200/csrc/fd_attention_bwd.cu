@@ -248,22 +248,34 @@ __global__ void __launch_bounds__(128, 6) linattn_bwd_apply_kernel(const __nv_bf
                                                                 __nv_bfloat16* __restrict__ dqkv, int HW) {
   __shared__ __align__(16) __nv_bfloat16 s_ctx[kHeads * kD * kMatStride];
   __shared__ __align__(16) __nv_bfloat16 s_dctx[kHeads * kD * kMatStride];
-  __shared__ float s_m[kHidden], s_iz[kHidden], s_r[kHidden];
+  __shared__ float s_m[kHidden], s_iz[kHidden], s_r[kHidden], s_cmean[kHidden];
   const int n = blockIdx.y;
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const int g = lane >> 2, tq = lane & 3;
   const float* st = stats + (long)n * kStatsFloats;
   const float* dc = dctx + (long)n * kHeads * kD * kD;
   const float inv_hw = 1.f / (float)HW;
+  // ctx[d,e] is the k-softmax average of v_e (/ HW): when v carries an offset common to the pixels, every row d holds about
+  // the same value and dq = scale sm (dqs - <sm, dqs>) keeps only the small d-dependent part of dqs = dout ctx^T.  dq is
+  // unchanged by a shift of ctx that depends on e only (sum_d sm = 1), so ctx is centred over d before its bf16 rounding:
+  // the rounding then scales with that d-dependent part instead of with the offset.
+  {
+    const float* col = st + 2 * kHidden + (t >> 5) * kD * kD + (t & 31);
+    float s = 0.f;
+#pragma unroll
+    for (int d = 0; d < kD; ++d) s += col[d * kD];
+    s_cmean[t] = s * (1.f / kD);
+  }
+  __syncthreads();
   for (int i = t; i < kHeads * kD * kD; i += 128) {
     const int row = i >> 5, e = i & 31;
-    s_ctx[row * kMatStride + e] = __float2bfloat16(st[2 * kHidden + i]);
+    s_ctx[row * kMatStride + e] = __float2bfloat16(st[2 * kHidden + i] - s_cmean[(row >> 5) * kD + e]);
     s_dctx[row * kMatStride + e] = __float2bfloat16(dc[i]);
   }
   s_m[t] = st[t];
   s_iz[t] = 1.f / st[kHidden + t];
   {
-    float r = 0.f;      // r[d] = sum_e dctx[d,e] ctx[d,e]   (fp32 sources)
+    float r = 0.f;      // r[d] = sum_e dctx[d,e] ctx[d,e]   (fp32 sources, ctx not centred)
 #pragma unroll
     for (int e = 0; e < kD; ++e) r += dc[t * kD + e] * st[2 * kHidden + t * kD + e];
     s_r[t] = r;

@@ -3,7 +3,7 @@ checks (tests/test_gpu_bench_launches.py) hold each launch to.
 
 ``record(B, H, W)`` runs ``Unet(64, 5, 2)`` under ``torch.no_grad()`` on the CPU with the library replaced by the
 recording fake of tests/test_unet_host.py and returns every distinct ``(name, scalars, nulls)`` with its count.  Weight
-preparation and workspace-size queries are left out: the checkers call them as set-up.  ``DEFAULT`` and ``MATRIX`` are
+preparation and size queries (``*_floats``) are left out: the checkers call them as set-up.  ``DEFAULT`` and ``MATRIX`` are
 that record, committed, for the two bench.py workloads; tests/test_bench_launch_table.py re-records them on the CPU.
 
 The bound functions take float64 tensors on any device; tests/test_bench_launch_table.py shows on the CPU that exact fp32
@@ -18,9 +18,10 @@ from opticalflowdiffusion_b200 import _lib
 SETUP = ("fd_prep_weight_batch", "fd_prep_weight_upconv", "fd_linattn_tc_prep")
 
 
-def record(B, H, W):
+def record(B, H, W, train=False):
     """{(name, scalars, nulls): count} of one inference forward of Unet(64, 5, 2) on a B x H x W batch, in launch order.
-    ``nulls`` has one character per pointer argument: "P" for a pointer, "0" for NULL (the stream is always "0")."""
+    ``nulls`` has one character per pointer argument: "P" for a pointer, "0" for NULL (the stream is always "0").
+    ``train``: the training forward (autograd on) and its backward from ``out.backward(ones)`` instead."""
     from test_unet_host import _Event, _FakeLib
     from opticalflowdiffusion_b200.unet import Unet
 
@@ -31,13 +32,18 @@ def record(B, H, W):
     try:
         torch.manual_seed(0)
         net = Unet(64, 5, 2)
-        with torch.no_grad():
-            net(torch.zeros(B, 2, H, W), torch.zeros(B, 3, H, W), torch.full((B,), 17))
+        args = torch.zeros(B, 2, H, W), torch.zeros(B, 3, H, W), torch.full((B,), 17)
+        if train:
+            out = net(*args)
+            out.backward(torch.ones_like(out))
+        else:
+            with torch.no_grad():
+                net(*args)
     finally:
         _lib.load, _lib.stream, _lib.require_cuda, torch.cuda.Event = saved
     seen = collections.OrderedDict()
     for c in lib.calls:
-        if c.name in SETUP or c.name.endswith("_workspace_floats"):
+        if c.name in SETUP or c.name.endswith("_floats"):
             continue
         key = (c.name, c.scalars, "".join("0" if z else "P" for z in c.nulls))
         seen[key] = seen.get(key, 0) + 1

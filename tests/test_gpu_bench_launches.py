@@ -209,6 +209,12 @@ def _gn_silu_sample(x, st, gamma, beta, eps, sc=None, sh=None):
 
 def check_gn_silu_fast(L, scalars, nulls, seed):
     """fd_gn_silu_fast: GroupNorm apply + (scale + 1, shift) + tanh-form SiLU (+ residual); grid-stride at large HW."""
+    check_gn_silu_form(L, "fd_gn_silu_fast", BL.silu_tanh, scalars, nulls, seed)
+
+
+def check_gn_silu_form(L, name, silu, scalars, nulls, seed):
+    """GroupNorm apply + (scale + 1, shift) + SiLU (+ residual) of the kernel ``name`` against ``silu(z, dz)``, which gives
+    silu(z) and the bound of the kernel's SiLU form."""
     lib = L.load()
     stride, N, HW, C, eps = scalars
     use_ss, use_res = nulls[4] == "P", nulls[5] == "P"
@@ -220,8 +226,8 @@ def check_gn_silu_fast(L, scalars, nulls, seed):
 
     def launch(fill):
         buf, out = guarded((N, HW, C), BF, fill)
-        L.check(lib.fd_gn_silu_fast(L.ptr(x), L.ptr(st), L.ptr(gamma), L.ptr(beta), rows.data_ptr() + 4 * off if use_ss else None,
-                                    stride, L.ptr(res), L.ptr(out), N, HW, C, eps, L.stream()))
+        L.check(getattr(lib, name)(L.ptr(x), L.ptr(st), L.ptr(gamma), L.ptr(beta), rows.data_ptr() + 4 * off if use_ss else None,
+                                   stride, L.ptr(res), L.ptr(out), N, HW, C, eps, L.stream()))
         torch.cuda.synchronize()
         guard_intact(buf, out)
         return out
@@ -229,12 +235,14 @@ def check_gn_silu_fast(L, scalars, nulls, seed):
     out = launch(NAN)
     worst = 0.0
     for n in range(N):
-        s, ds = _gn_silu_sample(x[n], st[n], gamma, beta, eps, sc[n] if use_ss else None, sh[n] if use_ss else None)
+        z, dz = BL.gn_affine(x[n].double(), st[n], gamma.double(), beta.double(), eps, sc[n] if use_ss else None,
+                             sh[n] if use_ss else None)
+        s, ds = silu(z, dz)
         ref = s + res[n].double() if use_res else s
         bound = BL.OUT_ROUND * ref.abs() + (1 + BL.OUT_ROUND) * ds
         worst = max(worst, BL.ratio((out[n].double() - ref).abs(), bound))
-        del s, ds, ref, bound
-    report("fd_gn_silu_fast", scalars, nulls, err_over_bound=worst)
+        del z, dz, s, ds, ref, bound
+    report(name, scalars, nulls, err_over_bound=worst)
     assert worst <= 1
     assert torch.equal(out, launch(0.0))
 
@@ -542,6 +550,15 @@ def check_time_embed(L, scalars, nulls, seed):
         return out
 
     out = launch(NAN)
+    ref, bound = time_embed_ref(sd, t, dim, tdim)[4:]
+    worst = BL.ratio((out.double() - ref).abs(), bound)
+    report("fd_time_embed", scalars, nulls, err_over_bound=worst)
+    assert worst <= 1
+    assert torch.equal(out, launch(0.0))
+
+
+def time_embed_ref(sd, t, dim, tdim):
+    """(pe, its bound, the pre-GELU activations, their bound, temb, its bound) of the time MLP in float64."""
     sd64 = {k: v.double() for k, v in sd.items()}
     ref = O.time_embedding(sd64, t.double(), dim)
     half = dim // 2
@@ -554,10 +571,7 @@ def check_time_embed(L, scalars, nulls, seed):
     gel = F.gelu(h)
     dg = 1.13 * dh + 2.0 ** -21 * h.abs()
     bound = dg @ w2.abs().t() + (tdim + 1) * 2.0 ** -23 * (gel.abs() @ w2.abs().t() + b2.abs())
-    worst = BL.ratio((out.double() - ref).abs(), bound)
-    report("fd_time_embed", scalars, nulls, err_over_bound=worst)
-    assert worst <= 1
-    assert torch.equal(out, launch(0.0))
+    return pe, dpe, h, dh, ref, bound
 
 
 def check_time_proj(L, scalars, nulls, seed):
